@@ -359,6 +359,8 @@ def run_b200(args):
     ms_max = float(t.item())
     value = world * N * T * K / (ms_max * 1e-3)
     rmse = float(s[4])
+    if args.dump_outputs and rank == 0:  # before the e2e leg replays other epochs on the same batch
+        dump_outputs(args.dump_outputs, batch, s, stream)
 
     # ---- end to end through the C ABI with HOST (pinned) buffers
     e2e = None
@@ -502,12 +504,41 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
-def config5_leg(local, dev, world, rank, comm, total_filters, n_macro, K, W, full=True, chunk=None):
+def dump_outputs(out_dir, batch, stats, stream, n_sample=1 << 16):
+    """What the last timed step hands its caller, as float64 .npy files under `out_dir`: the state `x` [n][S],
+    covariance `P` [n*n][S] and status words `status` [S] of a fixed sample of S <= n_sample filters (their
+    indices in `filter_index`; every filter when N <= n_sample) and the reduced statistics `error_stats` [6].
+    The sample depends on N alone, so two builds run with the same arguments can be compared file by file.
+    It is gathered on the device, so the host holds the dump alone: 8 (n*n + n + 2) bytes per sampled filter,
+    23 MB for T6 (n = 6), 39 MB for K8 (n = 8).  A directory created here ignores itself in git."""
+    import torch
+    from roskfpos_b200 import synth
+    N, n = batch.N, batch.n
+    dev = torch.device("cuda", torch.cuda.current_device())
+    idx = np.arange(N) if N <= n_sample else np.sort(np.random.default_rng(synth.SEED).choice(N, n_sample, replace=False))
+    sel = torch.as_tensor(idx, device=dev)
+    out = {"filter_index": idx, "error_stats": stats}
+    for name, shape, dtype in (("x", (n, N), torch.float64), ("P", (n * n, N), torch.float64),
+                               ("status", (N,), torch.int32)):
+        full = torch.empty(shape, device=dev, dtype=dtype)
+        batch.get_state_into(**{name: full}, stream=stream)
+        out[name] = full.index_select(-1, sel).cpu().numpy()
+        del full
+    if not os.path.isdir(out_dir):
+        os.makedirs(out_dir)
+        with open(os.path.join(out_dir, ".gitignore"), "w") as f:
+            f.write("*\n")
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def config5_leg(local, dev, world, rank, comm, total_filters, n_macro, K, W, full=True, chunk=None, dump=None):
     """BASELINE config 5 (full=False: config 3) as a STRONG-scaling leg: `total_filters` K8 filters in total,
     sharded by index over the ranks, inputs generated on the device chunk by chunk inside the timed region
     (never resident), statistics fused into the replay, ONE collective at the end (kfpos_stats_allreduce).
     Generator and summation tree depend on the global filter index only, so the reduced statistics are
-    bit-identical for any number of GPUs: the hex strings of the returned dict are there to be compared."""
+    bit-identical for any number of GPUs: the hex strings of the returned dict are there to be compared.
+    dump: a directory for dump_outputs of this rank's batch after the timed steps."""
     import torch
     import torch.distributed as dist
     from roskfpos_b200 import lib as L, synth
@@ -555,6 +586,8 @@ def config5_leg(local, dev, world, rank, comm, total_filters, n_macro, K, W, ful
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     cnt = batch.counters(reset=True)
+    if dump:
+        dump_outputs(dump, batch, s, stream)
     batch.close()
     del bufs, x0
     torch.cuda.empty_cache()
@@ -592,7 +625,8 @@ def run_config5(args):
     if world > 1:
         from roskfpos_b200.shard import nccl_comm
         comm = nccl_comm(rank, world, local)
-    r = config5_leg(local, dev, world, rank, comm, args.mc_filters, args.mc_macro_steps, args.steps, args.warmup, full=full)
+    r = config5_leg(local, dev, world, rank, comm, args.mc_filters, args.mc_macro_steps, args.steps, args.warmup, full=full,
+                    dump=args.dump_outputs if rank == 0 else None)
     if rank == 0:
         print(json.dumps({"metric": "k8_multisensor_events_per_sec", "value": r["events_per_s"],
                           "unit": "events/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -819,7 +853,15 @@ def main():
     ap.add_argument("--mc-filters", type=int, default=0, help="config3/5: total filters (default 1 Mi / 64 Mi)")
     ap.add_argument("--mc-macro-steps", type=int, default=0,
                     help="config3/5: 0.1 s macro-steps per bench step (default 1000 / 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl b200: after the timed steps, write what the last one computed (state, covariance, "
+                         "status of a fixed sample of rank 0's filters, reduced error statistics) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        # the reference leg times a sample whose size follows the measured CPU speed: nothing fixed to compare
+        ap.error("--dump-outputs applies to --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
     if args.impl == "reference":
