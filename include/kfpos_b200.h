@@ -436,6 +436,35 @@ int kfpos_batch_set_truth(kfpos_batch *b, const double *truth, void *stream);
 struct ncclComm;
 int kfpos_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, const double *truth, double out[6], void *stream);
 
+/* Time-resolved Monte Carlo statistics (no reference equivalent; SURVEY.md G5 extended to every epoch).
+ * Registers a truth trajectory SoA [n_rows][3][N] (x, y, z per output row; K8: z = the tag height, as for
+ * kfpos_batch_set_truth).  A device pointer is borrowed; a host array is copied.  NULL unregisters.
+ * Registering, and every kfpos_batch_set_state, sets the row cursor to 0.  While a trajectory is
+ * registered, every replay launch (replay_toa / step_toa, replay_epochs, replay_events, _ragged) leaves,
+ * for each of its output rows (the rows of its `traj`: a T6 epoch, a K8 / T9 TOA event), the partial
+ * sums of row `cursor + r`, and advances the cursor.  A launch that would pass n_rows fails with
+ * KFPOS_ERR_INVALID and runs nothing.  ML batches: KFPOS_ERR_INVALID.  Device scratch: 48 B per 32
+ * filters per row, allocated here (KFPOS_ERR_NOMEM when it cannot be).                                  */
+int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const double *truth, void *stream);
+
+/* out [n_rows][6] (host or device; n_rows must equal the registered count), per row:
+ *   [0] sum |p - truth|^2   [1] same over x, y   [2] filters counted (finite error)
+ *   [3] filters whose status word of THIS epoch is != 0
+ *   [4] sum NEES = e^T S^-1 e over the position block S of the covariance after the epoch
+ *       (T6 / T9: 3x3, K8: the x-y 2x2 block, e = the x-y error)   [5] filters in [4] (finite NEES, S positive
+ *       definite by its LDL^T pivots)
+ * A filter without an epoch in that row (per-filter dt < 0) adds nothing.  Rows the cursor has not
+ * reached are zero.  Summation order: a fixed 32-leaf tree per 32-filter chunk, then a pairwise tree
+ * over the chunk index.  It depends on the filter index only.  Device `out`: asynchronous on `stream`.
+ * Nothing registered: KFPOS_ERR_NOT_READY.                                                             */
+int kfpos_batch_epoch_stats(kfpos_batch *b, int64_t n_rows, double *out, void *stream);
+
+/* The same summed over the ranks of `comm`: one ncclAllGather of n_rows * 6 doubles per rank, then the
+ * pairwise rank tree on every rank.  With aligned power-of-two shards (a multiple of 32 filters) the
+ * result is bit-identical to the single-GPU result.  NCCL is bound as for kfpos_stats_allreduce
+ * (comm == NULL: this batch alone).                                                                    */
+int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, double *out, void *stream);
+
 /* Roofline denominator for this FP64 CUDA-core path (no reference equivalent):
  * times a DFMA-only kernel on `device` and returns the sustained FLOP/s.        */
 int kfpos_measure_fp64_peak(int device, double *flops_per_s);
@@ -464,6 +493,13 @@ int kfpos_synth_k8(int device, int64_t n_filters, int64_t first_filter, uint64_t
                    const double *anchors_xyz, double tag_z, double sigma_r, int n_events,
                    const kfpos_synth_event *events, double t_end, int64_t range_rows, int64_t sensor_rows,
                    int32_t *ranges, double *sensors, double *x0, double *truth_end, void *stream);
+
+/* Truth of the kfpos_synth_k8 workload at host times t[0..n_times): SoA [n_times][3][N] = (x, y, tag_z).
+ * The same per-filter Philox constants and kinematics as kfpos_synth_k8, so that a chunked run can
+ * register the truth of each chunk's TOA events.  Asynchronous on `stream` when `t` and `truth` are
+ * device pointers, else it synchronises `stream` before returning.                                  */
+int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first_filter, uint64_t seed, int n_times,
+                         const double *t, double tag_z, double *truth, void *stream);
 
 /* Accuracy self-test of the kernels' elementary functions (no reference equivalent): evaluates the
  * MUFU-seeded reciprocal and reciprocal square root and the reduced-range sincos on x[0..n) so that

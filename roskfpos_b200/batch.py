@@ -74,6 +74,7 @@ class Batch:
         self.cfg = config if config is not None else make_config(**cfg_kw)
         self.model = model
         self.N = int(n_filters)
+        self.device = int(device)
         L.check(L.lib().kfpos_batch_create(C.byref(self._h), int(device), int(model),
                                            C.c_int64(self.N), C.byref(self.cfg)), "kfpos_batch_create")
         self.n = L.lib().kfpos_batch_state_dim(self._h)
@@ -303,6 +304,56 @@ class Batch:
         c = C.c_void_p(int(comm)) if comm else None
         L.check(L.lib().kfpos_stats_allreduce(self._h, c, p, C.byref(buf), _stream_ptr(stream)), "kfpos_stats_allreduce")
         return np.array(list(buf))
+
+    # ------------------------------------------------- per-epoch statistics
+    def set_truth_traj(self, truth, stream=None):
+        """Registers the truth trajectory SoA [rows][3][N] (K8: z = the tag height) for the per-epoch statistics:
+        every replay launch then leaves the partial sums of its output rows and advances the row cursor
+        (kfpos_batch_set_truth_traj; set_state resets the cursor).  A device tensor is borrowed -- keep it alive.
+        None unregisters."""
+        rows = 0 if truth is None else int(truth.shape[0])
+        p, k = _ptr(truth, np.float64)
+        self._etruth_keep = k
+        self._es_rows = rows
+        L.check(L.lib().kfpos_batch_set_truth_traj(self._h, C.c_int64(rows), p, _stream_ptr(stream)),
+                "kfpos_batch_set_truth_traj")
+
+    def epoch_stats(self, readback=True, out=None, stream=None):
+        """[rows][6] per output row: sum |e|^2, sum |e_xy|^2, n, n with status != 0 in that epoch, sum NEES,
+        n in the NEES (kfpos_batch_epoch_stats).  out: a device tensor [rows][6] to fill asynchronously
+        (returned as given); readback False without `out`: a new device tensor, filled asynchronously."""
+        rows = getattr(self, "_es_rows", 0)
+        if out is None and readback:
+            out = np.zeros((rows, 6))
+        if out is None:
+            import torch
+            out = torch.empty((rows, 6), dtype=torch.float64, device="cuda:%d" % self.device)
+        L.check(L.lib().kfpos_batch_epoch_stats(self._h, C.c_int64(rows), _ptr(out)[0], _stream_ptr(stream)),
+                "kfpos_batch_epoch_stats")
+        return out
+
+    def epoch_stats_allreduce(self, comm=None, stream=None):
+        """kfpos_epoch_stats_allreduce: epoch_stats summed over the ranks of the NCCL communicator `comm` (a raw
+        ncclComm_t as an int / c_void_p, see shard.nccl_comm; None = this batch alone).  Returns [rows][6]."""
+        rows = getattr(self, "_es_rows", 0)
+        out = np.zeros((rows, 6))
+        c = C.c_void_p(int(comm)) if comm else None
+        L.check(L.lib().kfpos_epoch_stats_allreduce(self._h, c, C.c_int64(rows), C.c_void_p(out.ctypes.data),
+                                                    _stream_ptr(stream)), "kfpos_epoch_stats_allreduce")
+        return out
+
+
+def epoch_summary(stats):
+    """Per-row summary of epoch_stats / epoch_stats_allreduce output [rows][6]: dict of arrays rmse, rmse_xy
+    (over the filters with a finite error), anees (average NEES over the filters it counts), n, n_bad.
+    Rows without filters give NaN."""
+    s = np.asarray(stats, dtype=np.float64).reshape(-1, 6)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        n = s[:, 2]
+        ne = s[:, 5]
+        return dict(rmse=np.where(n > 0, np.sqrt(s[:, 0] / n), np.nan),
+                    rmse_xy=np.where(n > 0, np.sqrt(s[:, 1] / n), np.nan),
+                    anees=np.where(ne > 0, s[:, 4] / ne, np.nan), n=n.copy(), n_bad=s[:, 3].copy())
 
 
 def assemble_epochs(anchor, seq, range_mm, t, n_anchors, max_epochs, err=None, fix_row_clear=False, first_dt=0.1,

@@ -75,6 +75,12 @@ struct kfpos_batch {
     bool partials_fresh = false;
     bool out4_valid = false; // d_out4 holds the statistics of the current state
     double *d_gather = nullptr; // [n_ranks][4] of kfpos_stats_allreduce
+    // per-epoch statistics (kfpos_batch_set_truth_traj): truth rows SoA [es_rows][3][N], per-warp sums
+    // [es_rows][n_warps][6] left by the replay kernels, the next output row, and the fold buffers
+    const double *d_etruth = nullptr;
+    double *d_etruth_own = nullptr, *d_escratch = nullptr, *d_efold = nullptr, *d_eout = nullptr;
+    int64_t es_rows = 0, es_cursor = 0, es_fold_rows = 0;
+    DevBuf es_gather;
     // K8 / T9 latched sensor samples, SoA rows (see kfpos_k8.cuh)
     double *d_latch = nullptr;
     double *d_latch_u = nullptr; // batch-wide latched IMU covariances
@@ -164,6 +170,23 @@ RangeStream make_rs(const kfpos_batch *b, const void *ranges, int fmt, double er
     rs.fmt = fmt;
     rs.m_slots = b->anchors.n;
     return rs;
+}
+
+int64_t es_warps(const kfpos_batch *b) { return (b->N + 31) / 32; }
+// a launch with `rows` output rows: fits the registered truth trajectory (or none is registered)?
+int es_check(const kfpos_batch *b, int64_t rows) {
+    return (b->d_escratch && b->es_cursor + rows > b->es_rows) ? KFPOS_ERR_INVALID : KFPOS_OK;
+}
+// the per-epoch statistics pointers of the next launch, then the cursor moves past its `rows` output rows
+template <class Params>
+void es_bind(kfpos_batch *b, Params &p, int64_t rows) {
+    p.n_warps = es_warps(b);
+    p.etruth = nullptr;
+    p.escratch = nullptr;
+    if (!b->d_escratch) return;
+    p.etruth = b->d_etruth + b->es_cursor * 3 * b->N;
+    p.escratch = b->d_escratch + b->es_cursor * p.n_warps * ES_W;
+    b->es_cursor += rows;
 }
 
 } // namespace
@@ -264,6 +287,11 @@ extern "C" void kfpos_batch_destroy(kfpos_batch *b) {
     cudaFree(b->d_out4);
     cudaFree(b->d_truth_own);
     cudaFree(b->d_gather);
+    cudaFree(b->d_etruth_own);
+    cudaFree(b->d_escratch);
+    cudaFree(b->d_efold);
+    cudaFree(b->d_eout);
+    b->es_gather.release();
     cudaFree(b->d_latch);
     cudaFree(b->d_has);
     cudaFree(b->d_latch_u);
@@ -333,6 +361,7 @@ extern "C" int kfpos_batch_set_state(kfpos_batch *b, const double *x, const doub
     b->imu_seen = false; // the latches are cleared above
     b->partials_fresh = false;
     b->out4_valid = false;
+    b->es_cursor = 0;
     b->stepped = P != nullptr; // a restored checkpoint is a running filter; P0 = 0 is a fresh one
     if (!xd || (P && !on_device(P))) CK(cudaStreamSynchronize(s));
     return KFPOS_OK;
@@ -435,6 +464,7 @@ extern "C" int kfpos_batch_replay_toa(kfpos_batch *b, int n_steps, const double 
     if (fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     if (n_steps == 0) return KFPOS_OK;
+    if (es_check(b, n_steps)) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n;
@@ -534,6 +564,7 @@ extern "C" int kfpos_batch_replay_epochs(kfpos_batch *b, int n_steps, const doub
     if (fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     if (n_steps == 0) return KFPOS_OK;
+    if (es_check(b, n_steps)) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n, T = (size_t)n_steps;
@@ -600,6 +631,7 @@ int launch_replay(kfpos_batch *b, int T, const double *d_dt, const void *d_range
         p.counters = b->d_counters;
         p.truth = b->d_truth;
         p.partials = b->d_partials;
+        es_bind(b, p, T);
         CK(launch_t6_replay(p, s));
         b->partials_fresh = b->d_truth != nullptr;
         b->out4_valid = false;
@@ -673,6 +705,8 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
     const RangeStream rs = make_rs(b, d_ranges, fmt, err_scalar, d_err);
     poll_uninit(b);
     const bool track_uninit = b->uninit_possible;
+    int64_t n_toa = 0;
+    for (int i = 0; i < n; ++i) n_toa += events[i].kind == KFPOS_EV_TOA;
     if (track_uninit) {
         int rc = arm_uninit(b, s);
         if (rc) return rc;
@@ -699,6 +733,7 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
         p.counters = b->d_counters;
         p.truth = b->d_truth;
         p.partials = b->d_partials;
+        es_bind(b, p, n_toa);
         CK(launch_k8_replay(p, s));
         CK(cudaMemcpyAsync(b->d_latch_u, b->d_latch_u + 16, sizeof(double) * 16, cudaMemcpyDeviceToDevice, s));
         b->partials_fresh = b->d_truth != nullptr;
@@ -733,6 +768,7 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
         p.counters = b->d_counters;
         p.truth = b->d_truth;
         p.partials = b->d_partials;
+        es_bind(b, p, n_toa);
         CK(launch_t9_replay(p, s));
         CK(cudaMemcpyAsync(b->d_latch_u, b->d_latch_u + 16, sizeof(double) * 16, cudaMemcpyDeviceToDevice, s));
         b->partials_fresh = b->d_truth != nullptr;
@@ -777,6 +813,7 @@ static int replay_events_impl(kfpos_batch *b, int n_events, const kfpos_event *e
             if (!sensors || ev.offset + rows > sensor_rows) return KFPOS_ERR_INVALID;
         }
     }
+    if (es_check(b, n_toa)) return KFPOS_ERR_INVALID;
     const void *d_r = nullptr, *d_e = nullptr, *d_s = nullptr;
     int rc = stage_in(b, 4, ranges, (size_t)range_rows * N * fmt_size(fmt), s, &d_r);
     if (rc) return rc;
@@ -1338,6 +1375,111 @@ extern "C" int kfpos_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, cons
     return KFPOS_OK;
 }
 
+// ------------------------------------------------------- per-epoch statistics
+extern "C" int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const double *truth, void *stream) {
+    if (!b || b->model == KFPOS_MODEL_ML || (truth && n_rows <= 0)) return KFPOS_ERR_INVALID;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    // (cudaFree waits for the device: no launch still reads the buffers of the previous registration)
+    cudaFree(b->d_etruth_own);
+    cudaFree(b->d_escratch);
+    cudaFree(b->d_efold);
+    cudaFree(b->d_eout);
+    b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
+    b->d_etruth = nullptr;
+    b->es_rows = b->es_cursor = b->es_fold_rows = 0;
+    if (!truth) return KFPOS_OK;
+    const int64_t W = es_warps(b);
+    const size_t row_bytes = sizeof(double) * ES_W * (size_t)W;
+    // the fold of kfpos_batch_epoch_stats works on batches of rows in a buffer of at most 256 MB
+    int64_t fold_rows = (int64_t)(((size_t)256 << 20) / row_bytes);
+    if (fold_rows < 1) fold_rows = 1;
+    if (fold_rows > n_rows) fold_rows = n_rows;
+    const bool dev = on_device(truth);
+    cudaError_t e = cudaMalloc((void **)&b->d_escratch, row_bytes * (size_t)n_rows);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_efold, row_bytes * (size_t)fold_rows);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_eout, sizeof(double) * ES_W * (size_t)n_rows);
+    const size_t tbytes = sizeof(double) * 3 * (size_t)b->N * (size_t)n_rows;
+    if (e == cudaSuccess && !dev) e = cudaMalloc((void **)&b->d_etruth_own, tbytes);
+    if (e == cudaSuccess && !dev) e = cudaMemcpyAsync(b->d_etruth_own, truth, tbytes, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && !dev) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) {
+        cudaFree(b->d_etruth_own);
+        cudaFree(b->d_escratch);
+        cudaFree(b->d_efold);
+        cudaFree(b->d_eout);
+        b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
+        cudaGetLastError();
+        return map_cuda_err(e);
+    }
+    b->d_etruth = dev ? truth : b->d_etruth_own; // a device array is borrowed: the caller keeps it alive
+    b->es_rows = n_rows;
+    b->es_fold_rows = fold_rows;
+    return KFPOS_OK;
+}
+
+namespace {
+// [n_rows][6] of this batch into the device array `d_out`: rows [0, cursor) folded over the warp index (batches
+// of es_fold_rows rows through d_efold, the per-warp sums stay as they are), the rest zero
+int enqueue_epoch_stats(kfpos_batch *b, double *d_out, cudaStream_t s) {
+    const int64_t W = es_warps(b), done = b->es_cursor < b->es_rows ? b->es_cursor : b->es_rows;
+    for (int64_t r0 = 0; r0 < done; r0 += b->es_fold_rows) {
+        const int64_t rb = done - r0 < b->es_fold_rows ? done - r0 : b->es_fold_rows;
+        CK(launch_stats_tree(ES_W, rb, W, b->d_escratch + r0 * W * ES_W, b->d_efold, W * ES_W, ES_W, d_out + r0 * ES_W, s));
+    }
+    if (done < b->es_rows)
+        CK(cudaMemsetAsync(d_out + done * ES_W, 0, sizeof(double) * ES_W * (size_t)(b->es_rows - done), s));
+    return KFPOS_OK;
+}
+int es_ready(const kfpos_batch *b, int64_t n_rows, const double *out) {
+    if (!b || b->model == KFPOS_MODEL_ML || !out) return KFPOS_ERR_INVALID;
+    if (!b->d_escratch) return KFPOS_ERR_NOT_READY;
+    return n_rows == b->es_rows ? KFPOS_OK : KFPOS_ERR_INVALID;
+}
+} // namespace
+
+extern "C" int kfpos_batch_epoch_stats(kfpos_batch *b, int64_t n_rows, double *out, void *stream) {
+    int rc = es_ready(b, n_rows, out);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool dev = on_device(out);
+    if ((rc = enqueue_epoch_stats(b, dev ? out : b->d_eout, s))) return rc;
+    if (!dev) {
+        CK(cudaMemcpyAsync(out, b->d_eout, sizeof(double) * ES_W * (size_t)n_rows, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return KFPOS_OK;
+}
+
+extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, double *out,
+                                           void *stream) {
+    int rc = es_ready(b, n_rows, out);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = enqueue_epoch_stats(b, b->d_eout, s))) return rc;
+    const double *d_res = b->d_eout;
+    const size_t bytes = sizeof(double) * ES_W * (size_t)n_rows;
+    if (comm) {
+        NcclApi &api = nccl_api();
+        if (!api.all_gather || !api.count) return KFPOS_ERR_UNSUPPORTED;
+        int n_ranks = 0;
+        if (api.count(comm, &n_ranks) != 0 || n_ranks < 1 || n_ranks > 1024) return KFPOS_ERR_INVALID;
+        CK(b->es_gather.reserve(bytes * (size_t)n_ranks));
+        double *gat = (double *)b->es_gather.p;
+        // ONE collective: every rank's [n_rows][6] to every rank ([rank][row][6]), then per row the pairwise tree
+        // over the rank index -- the top levels of the global tree; row r's result lands on its rank-0 entry
+        if (api.all_gather(b->d_eout, gat, (size_t)n_rows * ES_W, 8, comm, s) != 0) return KFPOS_ERR_CUDA;
+        CK(launch_stats_tree(ES_W, n_rows, n_ranks, gat, gat, ES_W, n_rows * ES_W, gat, s));
+        d_res = gat;
+    }
+    const bool dev = on_device(out);
+    CK(cudaMemcpyAsync(out, d_res, bytes, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
+    if (!dev) CK(cudaStreamSynchronize(s));
+    return KFPOS_OK;
+}
+
 extern "C" int kfpos_measure_fp64_peak(int device, double *flops_per_s) {
     if (!flops_per_s) return KFPOS_ERR_INVALID;
     int count = 0;
@@ -1418,6 +1560,33 @@ extern "C" int kfpos_synth_k8(int device, int64_t n_filters, int64_t first_filte
     if (e != cudaSuccess) return map_cuda_err(e);
     // host staging is freed on return: finish the work first; device outputs: asynchronous on `stream`
     if (o_r.own || o_s.own || o_x.own || o_t.own) CK(cudaStreamSynchronize(s));
+    return KFPOS_OK;
+}
+
+extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first_filter, uint64_t seed, int n_times,
+                                    const double *t, double tag_z, double *truth, void *stream) {
+    if (n_filters <= 0 || n_times < 0 || (n_times > 0 && (!t || !truth))) return KFPOS_ERR_INVALID;
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
+        cudaGetLastError();
+        return KFPOS_ERR_CUDA;
+    }
+    if (n_times == 0) return KFPOS_OK;
+    DeviceGuard g(device);
+    if (!g.ok) return KFPOS_ERR_CUDA;
+    cudaStream_t s = (cudaStream_t)stream;
+    TmpIn i_t;
+    TmpOut o_t;
+    CK(i_t.set(t, sizeof(double) * (size_t)n_times, s));
+    CK(o_t.set(truth, sizeof(double) * 3 * (size_t)n_filters * (size_t)n_times));
+    SynthTruthParams p;
+    p.N = n_filters; p.filter0 = first_filter; p.seed = seed; p.n_times = n_times; p.tag_z = tag_z;
+    p.t = (const double *)i_t.d;
+    p.truth = (double *)o_t.d;
+    CK(launch_synth_k8_truth(p, s));
+    CK(o_t.back(s));
+    // staging is freed on return: finish the work first; device arrays only: asynchronous on `stream`
+    if (i_t.own || o_t.own) CK(cudaStreamSynchronize(s));
     return KFPOS_OK;
 }
 

@@ -52,7 +52,10 @@ KF_DEV void prefetch_event(const RawColPriv &raw, const Col &land, const EventDe
 // variant 1 drops the N with the largest residual, variant 2 keeps the best THREE anchors -- and the
 // update runs on the survivors.
 // MLI: the ML-initialisation branch and the per-filter tag height (kfpos_config.ml_initial_position) are compiled in.
-template <bool PME, int MT, bool SEL = false, bool MLI = SEL>
+// ES: per-epoch statistics at every TOA event (see kfpos_t6.cu): the terms go to a private shared-memory column, and
+// the warp sums them at the top of the next event or after the last one, behind a __syncwarp -- lanes of a ragged
+// replay (SEL && dt_f) reach that point on different paths.  The NEES is that of the x-y block, z = the tag height.
+template <bool PME, int MT, bool SEL = false, bool MLI = SEL, bool ES = false>
 __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __grid_constant__ K8Params p) {
     extern __shared__ double smem[];
     const int64_t f = (int64_t)blockIdx.x * K8_BLOCK + threadIdx.x;
@@ -105,9 +108,13 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
         // the tag height is per filter only after a 3-D ML initialisation (KF.cpp:256-257)
         const bool z_per_filter = MLI && p.cfg.ml_init && !p.cfg.use_fixed_height;
         double tag_z = z_per_filter ? p.latch[9 * N + f] : p.cfg.tag_z;
+        const Col es = {col + (size_t)(ES ? k8_smem_rows(m, p.rs.fmt, PME, MT > 0) : 0) * K8_BLOCK, K8_BLOCK};
+        double *const es_out = ES ? p.escratch + (f >> 5) * ES_W : nullptr;
+        bool es_pending = false; // the row n_toa - 1 still has to be summed (common to the warp)
 
         if (p.n_events > 0) prefetch_event(raw, land, p.events[0], m, p.rs, p.sensors, N, f);
         for (int e = 0; e < p.n_events; ++e) {
+            if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
             const EventDesc ev = p.events[e];
             cp_async_wait_all();
             double dt_ev = ev.dt;
@@ -120,6 +127,10 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
                             p.traj[((int64_t)n_toa * 3 + 0) * N + f] = px;
                             p.traj[((int64_t)n_toa * 3 + 1) * N + f] = py;
                             p.traj[((int64_t)n_toa * 3 + 2) * N + f] = th;
+                        }
+                        if (ES) {
+                            epoch_terms_zero(es);
+                            es_pending = true;
                         }
                         ++n_toa;
                     }
@@ -217,6 +228,12 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
                         p.traj[((int64_t)n_toa * 3 + 1) * N + f] = py;
                         p.traj[((int64_t)n_toa * 3 + 2) * N + f] = th;
                     }
+                    if (ES) {
+                        const double *tr = p.etruth + (int64_t)n_toa * 3 * N + f;
+                        epoch_terms<2>(px - tr[0], py - tr[N], tag_z - tr[2 * N], Pr.a[0], Pr.a[1], Pr.a[2], 0.0, 0.0, 0.0,
+                                       st.status != 0u, es);
+                        es_pending = true;
+                    }
                     ++n_toa;
                 }
             } else {
@@ -296,12 +313,19 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
                         p.traj[((int64_t)n_toa * 3 + 1) * N + f] = py;
                         p.traj[((int64_t)n_toa * 3 + 2) * N + f] = th;
                     }
+                    if (ES) {
+                        const double *tr = p.etruth + (int64_t)n_toa * 3 * N + f;
+                        epoch_terms<2>(px - tr[0], py - tr[N], tag_z - tr[2 * N], Pr.a[0], Pr.a[1], Pr.a[2], 0.0, 0.0, 0.0,
+                                       st.status != 0u, es);
+                        es_pending = true;
+                    }
                     ++n_toa;
                 }
 
             }
             if (!(SEL && p.dt_f)) __syncwarp(wmask); // the IEKF trip count differs per lane
         }
+        if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
         p.x[0 * N + f] = px; p.x[1 * N + f] = py; p.x[2 * N + f] = vx; p.x[3 * N + f] = vy;
         p.x[4 * N + f] = 0.0; p.x[5 * N + f] = 0.0; p.x[6 * N + f] = th; p.x[7 * N + f] = om;
 #pragma unroll
@@ -333,29 +357,34 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, int MT, bool SEL, bool MLI>
+template <bool PME, int MT, bool SEL, bool MLI, bool ES>
 static cudaError_t launch_k(const K8Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + K8_BLOCK - 1) / K8_BLOCK);
-    const size_t smem = (size_t)k8_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) * K8_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(k8_replay_kernel<PME, MT, SEL, MLI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
+    const size_t smem = (size_t)(k8_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * K8_BLOCK * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(k8_replay_kernel<PME, MT, SEL, MLI, ES>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    k8_replay_kernel<PME, MT, SEL, MLI><<<grid, K8_BLOCK, smem, s>>>(p);
+    k8_replay_kernel<PME, MT, SEL, MLI, ES><<<grid, K8_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool PME, int MT>
+template <bool PME, int MT, bool ES>
 static cudaError_t launch_tuned(const K8Params &p, cudaStream_t s) {
-    return p.cfg.ml_init ? launch_k<PME, MT, false, true>(p, s) : launch_k<PME, MT, false, false>(p, s);
+    return p.cfg.ml_init ? launch_k<PME, MT, false, true, ES>(p, s) : launch_k<PME, MT, false, false, ES>(p, s);
+}
+
+template <bool ES>
+static cudaError_t launch_replay_es(const K8Params &p, cudaStream_t s) {
+    if (p.cfg.variant == 1 || p.cfg.variant == 2 || p.dt_f != nullptr) // the general instantiation
+        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES>(p, s) : launch_k<false, 0, true, true, ES>(p, s);
+    if (p.rs.err != nullptr) return launch_tuned<true, 0, ES>(p, s);
+    if (p.rs.m_slots == 8 && !p.cfg.zero_tz) return launch_tuned<false, 8, ES>(p, s);
+    return launch_tuned<false, 0, ES>(p, s);
 }
 
 cudaError_t launch_k8_replay(const K8Params &p, cudaStream_t s) {
     if (p.N <= 0 || p.n_events <= 0) return cudaSuccess;
-    if (p.cfg.variant == 1 || p.cfg.variant == 2 || p.dt_f != nullptr) // the general instantiation
-        return p.rs.err != nullptr ? launch_k<true, 0, true, true>(p, s) : launch_k<false, 0, true, true>(p, s);
-    if (p.rs.err != nullptr) return launch_tuned<true, 0>(p, s);
-    if (p.rs.m_slots == 8 && !p.cfg.zero_tz) return launch_tuned<false, 8>(p, s);
-    return launch_tuned<false, 0>(p, s);
+    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
 }
 
 // getPose (KF.cpp:709-747): predict-only, state untouched

@@ -57,6 +57,76 @@ KF_DEV void filter_error_terms(double px, double py, double pz, const double *tr
     v[3] = bad ? 1.0 : 0.0;
 }
 
+// ---- per-epoch statistics (kfpos_batch_set_truth_traj): at every output row a replay kernel compiled with
+// ES = true leaves, per 32-filter warp, the 6 values of kfpos_batch_epoch_stats summed by a fixed 32-leaf tree
+// (level s = 16, 8, 4, 2, 1: lane i += lane i + s; lanes without a filter count as zeros) at
+// escratch[(row * n_warps + f / 32) * 6].  The folds over the warp index and over ranks are stats_tree's.
+constexpr int ES_W = 6;
+// The 6 terms of one filter: e = position - truth (3 components; K8: z = tag height); S = the packed position
+// block of the covariance the filter holds now (s00, s10, s11, s20, s21, s22; nd = 2: the x-y block, s2x unused).
+// NEES = e^T S^-1 e by LDL^T in a fixed order; a non-positive or non-finite pivot excludes the filter from [4], [5].
+template <int nd>
+KF_DEV void epoch_terms(double ex, double ey, double ez, double s00, double s10, double s11, double s20, double s21,
+                        double s22, bool bad, const Col &out) {
+    // (no contraction into FMAs: a host can reproduce [0] and [1] bit for bit from the trajectory)
+    const double exy = __dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey));
+    const double e2 = __dadd_rn(exy, __dmul_rn(ez, ez));
+    const bool fin = isfinite(e2);
+    out[0] = fin ? e2 : 0.0;
+    out[1] = fin ? exy : 0.0;
+    out[2] = fin ? 1.0 : 0.0;
+    out[3] = bad ? 1.0 : 0.0;
+    const double d0 = s00;
+    const double l10 = s10 / d0;
+    const double d1 = s11 - l10 * s10;
+    const double y1 = ey - l10 * ex;
+    double nees = ex * ex / d0 + y1 * y1 / d1;
+    bool pd = d0 > 0.0 && d0 < INFINITY && d1 > 0.0 && d1 < INFINITY;
+    if (nd == 3) {
+        const double l20 = s20 / d0;
+        const double c = s21 - l20 * s10;
+        const double l21 = c / d1;
+        const double d2 = s22 - l20 * s20 - l21 * c;
+        const double y2 = ez - l20 * ex - l21 * y1;
+        nees += y2 * y2 / d2;
+        pd = pd && d2 > 0.0 && d2 < INFINITY;
+    }
+    const bool ok = pd && isfinite(nees);
+    out[4] = ok ? nees : 0.0;
+    out[5] = ok ? 1.0 : 0.0;
+}
+KF_DEV void epoch_terms_zero(const Col &out) {
+#pragma unroll
+    for (int q = 0; q < ES_W; ++q) out[q] = 0.0;
+}
+// the warp's sum of the 6 terms in `v` (every lane of wmask calls it; wmask = the lanes with a filter, a prefix)
+KF_DEV void epoch_stats_flush(const Col &v, unsigned wmask, double *out) {
+    const int lane = threadIdx.x & 31;
+    double a[ES_W];
+#pragma unroll
+    for (int q = 0; q < ES_W; ++q) a[q] = v[q];
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const bool has = lane + s < 32 && ((wmask >> (lane + s)) & 1u);
+#pragma unroll
+        for (int q = 0; q < ES_W; ++q) {
+            const double o = __shfl_down_sync(wmask, a[q], s);
+            a[q] += has ? o : 0.0;
+        }
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int q = 0; q < ES_W; ++q) out[q] = a[q];
+    }
+}
+
+// row `row` of the event kernels: the lanes of a warp may arrive on different paths -- reconverge, then sum
+KF_DEV bool epoch_stats_row(const Col &v, unsigned wmask, double *es_out, int64_t row, int64_t n_warps) {
+    __syncwarp(wmask);
+    epoch_stats_flush(v, wmask, es_out + row * n_warps * ES_W);
+    return false;
+}
+
 struct T6Params {
     AnchorTable anchors;
     RangeStream rs;
@@ -76,6 +146,11 @@ struct T6Params {
     unsigned long long *counters;
     const double *truth; // SoA [3][N] or null: leave the error partials of the final state in `partials`
     double *partials;    // [ceil(N / 128)][4]
+    // per-epoch statistics (launchers pick the ES = true kernels when non-null): truth rows SoA [rows][3][N] and
+    // the per-warp sums [rows][n_warps][6] of this launch's first output row
+    const double *etruth;
+    double *escratch;
+    int64_t n_warps;
 };
 
 struct MlParams {
@@ -173,6 +248,9 @@ struct K8Params {
     unsigned long long *counters;
     const double *truth; // see T6Params
     double *partials;
+    const double *etruth; // see T6Params (output rows = TOA events)
+    double *escratch;
+    int64_t n_warps;
 };
 
 cudaError_t launch_t6_replay(const T6Params &p, cudaStream_t s);
@@ -210,6 +288,9 @@ struct T9Params {
     unsigned long long *counters;
     const double *truth; // see T6Params
     double *partials;
+    const double *etruth; // see T6Params (output rows = TOA events)
+    double *escratch;
+    int64_t n_warps;
 };
 cudaError_t launch_t9_replay(const T9Params &p, cudaStream_t s);
 cudaError_t launch_t9_get_pose(int64_t N, double dt, double jolt, const double *x, const double *P, double *x_pred,
@@ -231,6 +312,11 @@ cudaError_t launch_error_stats(int64_t N, const double *x, int zrow, double zcon
                                const double *truth, double *partials, double *out4, cudaStream_t s);
 // pairwise tree over n vectors of 4 doubles (IN PLACE on `part`): level by level part[i] += part[i + stride]
 cudaError_t launch_error_stats_tree(int64_t n, double *part, double *out4, cudaStream_t s);
+// the same tree over n vectors of `width` (4 or 6) doubles, for `rows` rows at once: vector i of row r is at
+// [r * row_stride + i * elem_stride]; the first level reads `src` and writes `part` (src == part: in place), the
+// others work in `part`; out[r * width + q]
+cudaError_t launch_stats_tree(int width, int64_t rows, int64_t n, const double *src, double *part, int64_t row_stride,
+                              int64_t elem_stride, double *out, cudaStream_t s);
 
 // getPose report in the publisher's layout (kfpos_misc.cu); model 1 = T6, 2 = K8, 3 = T9
 // tagz: null, or the per-filter tag height replacing tag_z (K8 after a 3-D ML initialisation)
@@ -298,6 +384,16 @@ struct SynthK8Params {
     double *truth_end;        // SoA [3][N] or null: (x, y, tag z) at t_end
 };
 cudaError_t launch_synth_k8(const SynthK8Params &p, cudaStream_t s);
+// truth of the same workload at host times t[0..n_times): SoA [n_times][3][N] = (x, y, tag_z)
+struct SynthTruthParams {
+    int64_t N, filter0;
+    uint64_t seed;
+    int n_times;
+    double tag_z;
+    const double *t; // device [n_times]
+    double *truth;
+};
+cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s);
 
 // DFMA-only microbenchmark on the current device (the FP64 roofline denominator)
 cudaError_t measure_fp64_peak(double *flops_per_s);

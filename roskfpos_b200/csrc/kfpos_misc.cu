@@ -51,16 +51,27 @@ error_stats_chunks(int64_t N, const double *x, int zrow, double zconst, const in
     block_stats_partial(v, sh, partials + (int64_t)blockIdx.x * 4);
 }
 
-// pairwise tree over the partial index, one block: the same shape whatever produced the partials
-__global__ void __launch_bounds__(1024) error_stats_tree(int64_t n, double *part, double *out4) {
+// pairwise tree over the partial index, one block per row: the same shape whatever produced the partials.
+// The first level reads `src` (src == part: in place); an element left without a partner there is copied.
+template <int W>
+__global__ void __launch_bounds__(1024) error_stats_tree(int64_t n, const double *src, double *part, int64_t row_stride,
+                                                         int64_t es, double *out) {
+    src += (int64_t)blockIdx.x * row_stride;
+    part += (int64_t)blockIdx.x * row_stride;
+    out += (int64_t)blockIdx.x * W;
+    if (src != part && (n & 1) && threadIdx.x == 0) {
+#pragma unroll
+        for (int q = 0; q < W; ++q) part[(n - 1) * es + q] = src[(n - 1) * es + q];
+    }
     for (int64_t stride = 1; stride < n; stride <<= 1) {
+        const double *in = stride == 1 ? src : part;
         for (int64_t i = (int64_t)threadIdx.x * 2 * stride; i + stride < n; i += (int64_t)blockDim.x * 2 * stride) {
 #pragma unroll
-            for (int q = 0; q < 4; ++q) part[i * 4 + q] += part[(i + stride) * 4 + q];
+            for (int q = 0; q < W; ++q) part[i * es + q] = in[i * es + q] + in[(i + stride) * es + q];
         }
         __syncthreads();
     }
-    if (threadIdx.x < 4) out4[threadIdx.x] = n > 0 ? part[threadIdx.x] : 0.0;
+    if (threadIdx.x < W) out[threadIdx.x] = n > 0 ? (n > 1 ? part : src)[threadIdx.x] : 0.0;
 }
 
 __global__ void i32_to_f64_kernel(int64_t N, const int32_t *in, double *out) {
@@ -83,7 +94,16 @@ cudaError_t launch_error_stats(int64_t N, const double *x, int zrow, double zcon
 }
 
 cudaError_t launch_error_stats_tree(int64_t n, double *part, double *out4, cudaStream_t s) {
-    error_stats_tree<<<1, 1024, 0, s>>>(n, part, out4);
+    return launch_stats_tree(4, 1, n, part, part, 0, 4, out4, s);
+}
+
+cudaError_t launch_stats_tree(int width, int64_t rows, int64_t n, const double *src, double *part, int64_t row_stride,
+                              int64_t elem_stride, double *out, cudaStream_t s) {
+    if (rows <= 0) return cudaSuccess;
+    if (rows > 0x7fffffffLL) return cudaErrorInvalidValue;
+    if (width == 4) error_stats_tree<4><<<(unsigned)rows, 1024, 0, s>>>(n, src, part, row_stride, elem_stride, out);
+    else if (width == ES_W) error_stats_tree<ES_W><<<(unsigned)rows, 1024, 0, s>>>(n, src, part, row_stride, elem_stride, out);
+    else return cudaErrorInvalidValue;
     return cudaGetLastError();
 }
 

@@ -61,23 +61,30 @@ KF_DEV Kin kin_at(double t, double pa, double pb, double th0) {
     return k;
 }
 
+constexpr double TWO_PI = 6.283185307179586476925286766559;
+
+// per-filter constants of the truth trajectory (event index 0xFFFFFFFF is reserved for them): phases and heading
+KF_DEV void filter_constants(uint64_t seed, uint64_t gf, double &pa, double &pb, double &th0) {
+    double ua, ub, uc, ud;
+    const Philox q = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 0u, (uint32_t)seed,
+                                   (uint32_t)(seed >> 32));
+    uniform2(q, ua, ub);
+    const Philox q2 = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 1u, (uint32_t)seed,
+                                    (uint32_t)(seed >> 32));
+    uniform2(q2, uc, ud);
+    pa = ua * TWO_PI;
+    pb = ub * TWO_PI;
+    th0 = 0.3 + 0.2 * uc;
+}
+
 __global__ void __launch_bounds__(128) synth_k8_kernel(const SynthK8Params p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
     if (f >= p.N) return;
     const int64_t N = p.N;
     const uint64_t gf = (uint64_t)(p.filter0 + f);
-    // per-filter constants of the truth trajectory (event index 0xFFFFFFFF is reserved for them)
-    double ua, ub, uc, ud;
-    {
-        const Philox q = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 0u, (uint32_t)p.seed,
-                                       (uint32_t)(p.seed >> 32));
-        uniform2(q, ua, ub);
-        const Philox q2 = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 1u, (uint32_t)p.seed,
-                                        (uint32_t)(p.seed >> 32));
-        uniform2(q2, uc, ud);
-    }
-    const double TWO_PI = 6.283185307179586476925286766559;
-    const double pa = ua * TWO_PI, pb = ub * TWO_PI, th0 = 0.3 + 0.2 * uc, om = 0.05;
+    double pa, pb, th0;
+    filter_constants(p.seed, gf, pa, pb, th0);
+    const double om = 0.05;
     if (p.x0) { // state at t = 0
         const Kin k = kin_at(0.0, pa, pb, th0);
         p.x0[0 * N + f] = k.px; p.x0[1 * N + f] = k.py; p.x0[2 * N + f] = k.vx; p.x0[3 * N + f] = k.vy;
@@ -138,6 +145,26 @@ __global__ void __launch_bounds__(128) synth_k8_kernel(const SynthK8Params p) {
 cudaError_t launch_synth_k8(const SynthK8Params &p, cudaStream_t s) {
     if (p.N <= 0) return cudaSuccess;
     synth_k8_kernel<<<(unsigned)((p.N + 127) / 128), 128, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+// the truth of synth_k8_kernel's filters at the given times (the per-epoch statistics of a chunked run)
+__global__ void __launch_bounds__(128) synth_k8_truth_kernel(const SynthTruthParams p) {
+    const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (f >= p.N) return;
+    const int64_t N = p.N;
+    double pa, pb, th0;
+    filter_constants(p.seed, (uint64_t)(p.filter0 + f), pa, pb, th0);
+    for (int i = 0; i < p.n_times; ++i) {
+        const Kin k = kin_at(p.t[i], pa, pb, th0);
+        double *o = p.truth + (int64_t)i * 3 * N + f;
+        o[0] = k.px; o[N] = k.py; o[2 * N] = p.tag_z;
+    }
+}
+
+cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s) {
+    if (p.N <= 0 || p.n_times <= 0) return cudaSuccess;
+    synth_k8_truth_kernel<<<(unsigned)((p.N + 127) / 128), 128, 0, s>>>(p);
     return cudaGetLastError();
 }
 

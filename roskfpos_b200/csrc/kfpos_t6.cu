@@ -32,7 +32,10 @@ __host__ __device__ inline int t6_smem_rows(int m, int fmt, bool pme, bool in_re
 // FMT: the wire format as a compile-time constant (the tuned instantiation: the per-epoch prefetch / conversion code of
 // the other two formats -- a third of the replay loop's 2300 instructions, against a 32 KB instruction cache -- is
 // not generated); -1 = read from the parameters.
-template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1>
+// ES: per-epoch statistics (kfpos_batch_set_truth_traj): after every epoch the filter's error terms go to a private
+// shared-memory column (6 rows behind the others), and at the top of the next epoch -- the one point every lane of
+// the warp passes, stepping or not -- the warp sums them (epoch_stats_flush).  The ES = false code is unchanged.
+template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false>
 __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __grid_constant__ T6Params p) {
     extern __shared__ double smem[];
     const int fmt = FMT >= 0 ? FMT : p.rs.fmt;
@@ -65,6 +68,8 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
         ep.m_slots = m;
         // landing zone of the cp.async prefetch of the next epoch
         const RawCol raw = make_raw(smem + (size_t)row * T6_BLOCK, fmt, threadIdx.x, T6_BLOCK);
+        const Col es = {col + (size_t)(ES ? t6_smem_rows(m, fmt, PME, MT > 0) : 0) * T6_BLOCK, T6_BLOCK};
+        double *const es_out = ES ? p.escratch + (f >> 5) * ES_W : nullptr;
 
         double pos[3];
 #pragma unroll
@@ -76,6 +81,7 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
         prefetch_epoch(raw, m, p.rs.ranges, fmt, f, N);
         double dt_next = dt_f ? __ldg(dt_f + f) : 0.0;
         for (int t = 0; t < p.T; ++t) {
+            if (ES && t > 0) epoch_stats_flush(es, wmask, es_out + (int64_t)(t - 1) * p.n_warps * ES_W);
             // per-filter time steps (assembled logs): a negative dt = this filter has no epoch t.
             // The lanes that do step are the ones that re-converge below.
             const double dt = dt_f ? dt_next : __ldg(p.dt + t);
@@ -90,6 +96,7 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
                     for (int k = 0; k < 3; ++k) p.traj[((int64_t)t * 3 + k) * N + f] = pos[k];
                 }
                 if (p.sel) p.sel[(int64_t)t * N + f] = -1;
+                if (ES) epoch_terms_zero(es);
                 continue;
             }
 
@@ -184,7 +191,13 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
                 for (int k = 0; k < 3; ++k) p.traj[((int64_t)t * 3 + k) * N + f] = pos[k];
             }
             if (p.sel) p.sel[(int64_t)t * N + f] = ignored;
+            if (ES) {
+                const double *tr = p.etruth + (int64_t)t * 3 * N + f;
+                epoch_terms<3>(pos[0] - tr[0], pos[1] - tr[N], pos[2] - tr[2 * N], Pm[0], Pm[1], Pm[2], Pm[3], Pm[4], Pm[5],
+                               st.status != 0u, es);
+            }
         }
+        if (ES) epoch_stats_flush(es, wmask, es_out + (int64_t)(p.T - 1) * p.n_warps * ES_W);
 
 #pragma unroll
         for (int k = 0; k < 3; ++k) p.x[(int64_t)k * N + f] = pos[k];
@@ -208,46 +221,51 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1>
+template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false>
 static cudaError_t launch_k(const T6Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + T6_BLOCK - 1) / T6_BLOCK);
-    const size_t smem = (size_t)t6_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) * T6_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(t6_replay_kernel<PME, LOO, MT, SEL, FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
+    const size_t smem = (size_t)(t6_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * T6_BLOCK * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    t6_replay_kernel<PME, LOO, MT, SEL, FMT><<<grid, T6_BLOCK, smem, s>>>(p);
+    t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES><<<grid, T6_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
 }
 // the plain replay with a compile-time anchor count: one instantiation per wire format
-template <int MT>
+template <int MT, bool ES>
 static cudaError_t launch_tuned(const T6Params &p, cudaStream_t s) {
-    if (p.dt_f != nullptr) return launch_k<false, false, MT>(p, s); // per-filter time steps
+    if (p.dt_f != nullptr) return launch_k<false, false, MT, false, -1, ES>(p, s); // per-filter time steps
     switch (p.rs.fmt) {
-    case 1: return launch_k<false, false, MT, false, 1>(p, s);
-    case 2: return launch_k<false, false, MT, false, 2>(p, s);
-    default: return launch_k<false, false, MT, false, 0>(p, s);
+    case 1: return launch_k<false, false, MT, false, 1, ES>(p, s);
+    case 2: return launch_k<false, false, MT, false, 2, ES>(p, s);
+    default: return launch_k<false, false, MT, false, 0, ES>(p, s);
     }
 }
 
-cudaError_t launch_t6_replay(const T6Params &p, cudaStream_t s) {
-    if (p.N <= 0 || p.T <= 0) return cudaSuccess;
+template <bool ES>
+static cudaError_t launch_replay_es(const T6Params &p, cudaStream_t s) {
     const bool pme = p.rs.err != nullptr;
     const int m = p.rs.m_slots;
     if (p.variant == 1 || p.variant == 2) {
         if (p.ignore_worst) return cudaErrorInvalidValue; // the two heuristics are alternatives
-        return pme ? launch_k<true, false, 0, true>(p, s) : launch_k<false, false, 0, true>(p, s);
+        return pme ? launch_k<true, false, 0, true, -1, ES>(p, s) : launch_k<false, false, 0, true, -1, ES>(p, s);
     }
     if (p.ignore_worst) {
-        if (pme) return launch_k<true, true, 0>(p, s);
-        if (m == 8) return launch_k<false, true, 8>(p, s);
-        if (m == 16) return launch_k<false, true, 16>(p, s);
-        return launch_k<false, true, 0>(p, s);
+        if (pme) return launch_k<true, true, 0, false, -1, ES>(p, s);
+        if (m == 8) return launch_k<false, true, 8, false, -1, ES>(p, s);
+        if (m == 16) return launch_k<false, true, 16, false, -1, ES>(p, s);
+        return launch_k<false, true, 0, false, -1, ES>(p, s);
     }
-    if (pme) return launch_k<true, false, 0>(p, s);
-    if (m == 4) return launch_k<false, false, 4>(p, s);
-    if (m == 8) return launch_tuned<8>(p, s);
-    if (m == 16) return launch_tuned<16>(p, s);
-    return launch_k<false, false, 0>(p, s);
+    if (pme) return launch_k<true, false, 0, false, -1, ES>(p, s);
+    if (m == 4) return launch_k<false, false, 4, false, -1, ES>(p, s);
+    if (m == 8) return launch_tuned<8, ES>(p, s);
+    if (m == 16) return launch_tuned<16, ES>(p, s);
+    return launch_k<false, false, 0, false, -1, ES>(p, s);
+}
+
+cudaError_t launch_t6_replay(const T6Params &p, cudaStream_t s) {
+    if (p.N <= 0 || p.T <= 0) return cudaSuccess;
+    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
 }
 
 // getPose (TOA.cpp:438-473): predict-only, state untouched

@@ -192,7 +192,8 @@ KF_DEV int t9_update(const AnchorTable &A, const EpochT<PME, MT> &ep, bool has_r
 // IMU = false: the lean variant for schedules without accelerometer samples (nothing latched, no
 // IMU event): no register copy of the 9x9 covariance anywhere, 4 blocks per SM like T6.
 // SEL: the EKF-side NLOS variants (see kfpos_t6.cu), 3-D selection from the predicted position.
-template <bool PME, int MT, bool IMU, bool SEL = false>
+// ES: per-epoch statistics at every TOA event (see kfpos_t6.cu / kfpos_k8.cu), NEES of the 3x3 position block.
+template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false>
 __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_kernel(const __grid_constant__ T9Params p) {
     extern __shared__ double smem[];
     const int64_t f = (int64_t)blockIdx.x * T9_BLOCK + threadIdx.x;
@@ -241,6 +242,9 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
             Ra[3] = 0.5 * (c[2] + c[6]); Ra[4] = 0.5 * (c[5] + c[7]); Ra[5] = c[8];
         }
         int n_toa = 0;
+        const Col es = {col + (size_t)(ES ? t9_smem_rows(m, p.rs.fmt, PME, MT > 0) : 0) * T9_BLOCK, T9_BLOCK};
+        double *const es_out = ES ? p.escratch + (f >> 5) * ES_W : nullptr;
+        bool es_pending = false; // the row n_toa - 1 still has to be summed (common to the warp)
         auto prefetch = [&](const EventDesc &ev) {
             if (ev.kind == EV_TOA) {
                 prefetch_epoch(raw, m, p.rs.ranges, p.rs.fmt, ev.offset * N + f, N);
@@ -251,6 +255,7 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
         };
         if (p.n_events > 0) prefetch(p.events[0]);
         for (int e = 0; e < p.n_events; ++e) {
+            if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
             const EventDesc ev = p.events[e];
             double dt = ev.dt;
             if (SEL && p.dt_f) { // ragged replay: every filter has its own time steps
@@ -262,6 +267,10 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
                         if (p.traj) {
 #pragma unroll
                             for (int k = 0; k < 3; ++k) p.traj[((int64_t)n_toa * 3 + k) * N + f] = pos[k];
+                        }
+                        if (ES) {
+                            epoch_terms_zero(es);
+                            es_pending = true;
                         }
                         ++n_toa;
                     }
@@ -289,6 +298,12 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
                     if (p.traj) {
 #pragma unroll
                         for (int k = 0; k < 3; ++k) p.traj[((int64_t)n_toa * 3 + k) * N + f] = pos[k];
+                    }
+                    if (ES) {
+                        const double *tr = p.etruth + (int64_t)n_toa * 3 * N + f;
+                        epoch_terms<3>(pos[0] - tr[0], pos[1] - tr[N], pos[2] - tr[2 * N], Pm[0], Pm[1], Pm[2], Pm[3], Pm[4], Pm[5],
+                                       st.status != 0u, es);
+                        es_pending = true;
                     }
                     ++n_toa;
                 } else {
@@ -379,9 +394,16 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
 #pragma unroll
                     for (int k = 0; k < 3; ++k) p.traj[((int64_t)n_toa * 3 + k) * N + f] = pos[k];
                 }
+                if (ES) {
+                    const double *tr = p.etruth + (int64_t)n_toa * 3 * N + f;
+                    epoch_terms<3>(pos[0] - tr[0], pos[1] - tr[N], pos[2] - tr[2 * N], Pm[0], Pm[1], Pm[2], Pm[3], Pm[4], Pm[5],
+                                   st.status != 0u, es);
+                    es_pending = true;
+                }
                 ++n_toa;
             }
         }
+        if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             p.x[(int64_t)k * N + f] = pos[k];
@@ -417,28 +439,34 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, int MT, bool IMU, bool SEL = false>
+template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false>
 static cudaError_t launch_k(const T9Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + T9_BLOCK - 1) / T9_BLOCK);
-    const size_t smem = (size_t)t9_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) * T9_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(t9_replay_kernel<PME, MT, IMU, SEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = (size_t)(t9_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * T9_BLOCK * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(t9_replay_kernel<PME, MT, IMU, SEL, ES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
     if (e != cudaSuccess) return e;
-    t9_replay_kernel<PME, MT, IMU, SEL><<<grid, T9_BLOCK, smem, s>>>(p);
+    t9_replay_kernel<PME, MT, IMU, SEL, ES><<<grid, T9_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
+}
+
+template <bool ES>
+static cudaError_t launch_replay_es(const T9Params &p, cudaStream_t s) {
+    if (p.variant == 1 || p.variant == 2 || p.dt_f != nullptr || p.ml_init) // the general instantiation
+        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES>(p, s) : launch_k<false, 0, true, true, ES>(p, s);
+    if (p.no_imu) {
+        if (p.rs.err != nullptr) return launch_k<true, 0, false, false, ES>(p, s);
+        if (p.rs.m_slots == 8) return launch_k<false, 8, false, false, ES>(p, s);
+        return launch_k<false, 0, false, false, ES>(p, s);
+    }
+    if (p.rs.err != nullptr) return launch_k<true, 0, true, false, ES>(p, s);
+    if (p.rs.m_slots == 8) return launch_k<false, 8, true, false, ES>(p, s);
+    return launch_k<false, 0, true, false, ES>(p, s);
 }
 
 cudaError_t launch_t9_replay(const T9Params &p, cudaStream_t s) {
     if (p.N <= 0 || p.n_events <= 0) return cudaSuccess;
-    if (p.variant == 1 || p.variant == 2 || p.dt_f != nullptr || p.ml_init) // the general instantiation
-        return p.rs.err != nullptr ? launch_k<true, 0, true, true>(p, s) : launch_k<false, 0, true, true>(p, s);
-    if (p.no_imu) {
-        if (p.rs.err != nullptr) return launch_k<true, 0, false>(p, s);
-        if (p.rs.m_slots == 8) return launch_k<false, 8, false>(p, s);
-        return launch_k<false, 0, false>(p, s);
-    }
-    if (p.rs.err != nullptr) return launch_k<true, 0, true>(p, s);
-    if (p.rs.m_slots == 8) return launch_k<false, 8, true>(p, s);
-    return launch_k<false, 0, true>(p, s);
+    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
 }
 
 // getPose (TOAIMU.cpp:476-510): predict-only, state untouched

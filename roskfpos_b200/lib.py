@@ -96,6 +96,10 @@ SIGNATURES = {
     "kfpos_merge_streams": (_I, [_I, _I64, _I, _I64, _VP, _VP, _VP, _VP, _VP, _VP, _I, _VP, _D, _VP, _VP, _VP, _VP, _VP,
                                  _VP, _VP, _VP]),
     "kfpos_batch_replay_events_ragged": (_I, [_VP, _I, _VP, _VP, _VP, _I, _D, _VP, _VP, _I64, _VP, _VP]),
+    "kfpos_batch_set_truth_traj": (_I, [_VP, _I64, _VP, _VP]),
+    "kfpos_batch_epoch_stats": (_I, [_VP, _I64, _VP, _VP]),
+    "kfpos_epoch_stats_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
+    "kfpos_synth_k8_truth": (_I, [_I, _I64, _I64, C.c_uint64, _I, _VP, _D, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

@@ -204,13 +204,33 @@ def device_ranges_mm(n_filters: int, n_steps: int, anchors: np.ndarray, dt: floa
     return out, x0.contiguous(), p.contiguous()
 
 
+def device_truth_traj(n_filters: int, n_steps: int, dt: float, device, seed: int = SEED, step0: int = 0):
+    """The per-step truth of device_ranges_mm with the same arguments (same generator, same first draw, so the
+    same phases): SoA [T][3][N] float64 on `device`, row k = the position at step step0 + k + 1 -- the truth
+    of the replay's output row k, for Batch.set_truth_traj."""
+    import torch
+
+    g = torch.Generator(device=device)
+    g.manual_seed(seed)
+    ph = torch.rand((2, n_filters), generator=g, device=device, dtype=torch.float64) * (2 * np.pi)
+    out = torch.empty((n_steps, 3, n_filters), device=device, dtype=torch.float64)
+    for k in range(n_steps):
+        t = (step0 + k + 1) * dt
+        out[k, 0] = 5 + 3 * torch.sin(0.20 * t + ph[0])
+        out[k, 1] = 5 + 3 * torch.sin(0.31 * t + ph[1])
+        out[k, 2] = 1.0
+    return out
+
+
 def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, full=False, sigma_r=0.10,
-                        first_filter=0, want_x0=False, out=None, stream=None):
+                        first_filter=0, want_x0=False, out=None, stream=None, want_truth_toa=False):
     """Macro-steps [macro0, macro0 + n_macro) of the K8 Monte Carlo workload, generated ON THE DEVICE by
     kfpos_synth_k8 (Philox4x32-10; the stream of a filter depends only on seed, its global index and the
     global event index).  Returns the dict k8_workload returns (events for replay_events, ranges int32
     [T][M][N], sensors f64 [R][N], truth_end [3][N], x0 [8][N] if want_x0) with torch tensors on `device`;
-    `out` may hold the tensors of a previous chunk of the same shape to be reused."""
+    `out` may hold the tensors of a previous chunk of the same shape to be reused.  want_truth_toa: also
+    truth_toa [n_toa][3][N], the truth (x, y, tag z) at the chunk's TOA events made on the device by
+    kfpos_synth_k8_truth -- what Batch.set_truth_traj takes for the per-epoch statistics of the chunk."""
     import ctypes as C
     import torch
     from . import lib as L
@@ -257,5 +277,13 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
                                    C.c_void_p(ranges.data_ptr()), C.c_void_p(sensors.data_ptr()),
                                    None if x0 is None else C.c_void_p(x0.data_ptr()),
                                    C.c_void_p(truth_end.data_ptr()), sp), "kfpos_synth_k8")
-    return dict(events=events, ranges=ranges, sensors=sensors, x0=x0, truth_end=truth_end, tag_z=1.049,
-                n_toa=n_rng, n_events=len(events))
+    res = dict(events=events, ranges=ranges, sensors=sensors, x0=x0, truth_end=truth_end, tag_z=1.049,
+               n_toa=n_rng, n_events=len(events))
+    if want_truth_toa:
+        t_toa = np.ascontiguousarray([tt for kind, _, tt, _ in sev if kind == EV_TOA], dtype=np.float64)
+        truth_toa = buf("truth_toa", (n_rng, 3, N), torch.float64)
+        L.check(L.lib().kfpos_synth_k8_truth(dev.index or 0, N, int(first_filter), C.c_uint64(seed), n_rng,
+                                             C.c_void_p(t_toa.ctypes.data), 1.049, C.c_void_p(truth_toa.data_ptr()), sp),
+                "kfpos_synth_k8_truth")
+        res["truth_toa"] = truth_toa
+    return res
