@@ -494,12 +494,50 @@ int kfpos_synth_k8(int device, int64_t n_filters, int64_t first_filter, uint64_t
                    const kfpos_synth_event *events, double t_end, int64_t range_rows, int64_t sensor_rows,
                    int32_t *ranges, double *sensors, double *x0, double *truth_end, void *stream);
 
-/* Truth of the kfpos_synth_k8 workload at host times t[0..n_times): SoA [n_times][3][N] = (x, y, tag_z).
- * The same per-filter Philox constants and kinematics as kfpos_synth_k8, so that a chunked run can
- * register the truth of each chunk's TOA events.  Asynchronous on `stream` when `t` and `truth` are
- * device pointers, else it synchronises `stream` before returning.                                  */
+/* Truth of the kfpos_synth_k8 AND kfpos_synth_toa_ranges workloads at host times t[0..n_times): SoA
+ * [n_times][3][N] = (x, y, tag_z).  Both generators draw the same per-filter Philox constants and use the
+ * same kinematics, so that a chunked run can register the truth of each chunk's TOA events / epochs.
+ * Asynchronous on `stream` when `t` and `truth` are device pointers, else it synchronises `stream`
+ * before returning.                                                                                  */
 int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first_filter, uint64_t seed, int n_times,
                          const double *t, double tag_z, double *truth, void *stream);
+
+/* Monte Carlo ranging epochs, generated on the device (no reference equivalent): the [T][M][N] millimetre
+ * range log every ranging consumer takes (kfpos_batch_replay_toa, the K8 / T9 ranging replays,
+ * kfpos_batch_ml_solve), with optional missing rangings and NLOS biases.  For filter gf = first_filter + f,
+ * epoch g = first_epoch + k at time t[k] and anchor a (Philox4x32-10 counter (gf lo, gf hi, event, sample),
+ * key (seed lo, seed hi), as kfpos_synth_k8):
+ *   truth     (x, y, z) = the Lissajous of kfpos_synth_k8 (kfpos_synth_k8_truth gives it), z = tag_z;
+ *   distance  d_a = |(x, y, z) - anchor_a|;
+ *   noise     n_a = Box-Muller normal number a & 1 of the counter (gf, g, a >> 1);
+ *   impaired  only when p_missing > 0 or p_nlos > 0: (u, v) = two uniforms of the counter
+ *             (gf, g, 0x80000000 | a); missing when u < p_missing; NLOS bias b = -nlos_mean log(v / p_nlos)
+ *             when v < p_nlos (an exponential of mean nlos_mean), else 0;
+ *   output    mm = floor((d_a + sigma_r n_a + b) * 1000); 0 ("no ranging") when missing or mm <= 0;
+ *             KFPOS_FMT_U16_MM clamps to 65535.
+ * Each value is a pure function of (seed, gf, g, a): a run gives the same numbers however it is sharded
+ * (first_filter) or cut into chunks (first_epoch).  Epoch index 0xFFFFFFFF is reserved for the per-filter
+ * constants: first_epoch + n_epochs must not exceed it.                                                 */
+typedef struct kfpos_synth_toa {
+    uint64_t seed;
+    int64_t first_filter;  /* global index of output filter 0 (sharding)                 */
+    int64_t first_epoch;   /* global index of epoch 0 of this call (chunking)            */
+    double tag_z;          /* m                                                          */
+    double sigma_r;        /* ranging noise sd, m (>= 0)                                 */
+    double p_missing;      /* probability that a ranging is absent, [0, 1]               */
+    double p_nlos;         /* probability of a positive NLOS bias, [0, 1]                */
+    double nlos_mean;      /* mean of the exponential bias, m (> 0 when p_nlos > 0)      */
+} kfpos_synth_toa;
+
+/* t: HOST array [n_epochs] of epoch times, s.  ranges: SoA [n_epochs][n_anchors][N] in fmt
+ * (KFPOS_FMT_I32_MM or KFPOS_FMT_U16_MM).  A device `ranges` makes the call asynchronous on `stream`; a
+ * host one is staged and `stream` is synchronised before returning.  KFPOS_ERR_INVALID: a bad count,
+ * n_anchors outside [1, KFPOS_MAX_ANCHORS], a probability outside [0, 1], sigma_r < 0, nlos_mean <= 0 with
+ * p_nlos > 0, first_filter < 0, an epoch range that reaches the reserved index, another fmt.
+ * KFPOS_ERR_CUDA without a device (there is no CPU path).                                              */
+int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                           int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
+                           void *ranges, void *stream);
 
 /* Accuracy self-test of the kernels' elementary functions (no reference equivalent): evaluates the
  * MUFU-seeded reciprocal and reciprocal square root and the reduced-range sincos on x[0..n) so that

@@ -1590,6 +1590,52 @@ extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first
     return KFPOS_OK;
 }
 
+extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                      int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
+                                      void *ranges, void *stream) {
+    const auto prob = [](double q) { return q >= 0.0 && q <= 1.0; }; // false for NaN
+    if (n_filters <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || !anchors_xyz || n_epochs < 0 ||
+        (n_epochs > 0 && (!t || !ranges)) || !gen || (fmt != KFPOS_FMT_I32_MM && fmt != KFPOS_FMT_U16_MM))
+        return KFPOS_ERR_INVALID;
+    if (!prob(gen->p_missing) || !prob(gen->p_nlos) || !(gen->sigma_r >= 0.0) ||
+        (gen->p_nlos > 0.0 && !(gen->nlos_mean > 0.0)) || gen->first_filter < 0 || gen->first_epoch < 0 ||
+        gen->first_epoch + n_epochs > (int64_t)0xFFFFFFFF) // epoch index 0xFFFFFFFF: the per-filter constants
+        return KFPOS_ERR_INVALID;
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
+        cudaGetLastError();
+        return KFPOS_ERR_CUDA;
+    }
+    if (n_epochs == 0) return KFPOS_OK;
+    DeviceGuard g(device);
+    if (!g.ok) return KFPOS_ERR_CUDA;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t row = fmt_size(fmt) * (size_t)n_anchors * (size_t)n_filters; // bytes of one epoch
+    TmpOut o_r;
+    CK(o_r.set(ranges, row * (size_t)n_epochs));
+    // the epoch times travel in the parameter block, SYNTH_TOA_T per launch: nothing to stage, so a device
+    // `ranges` leaves the call asynchronous (the next chunk can be generated while this one is replayed)
+    SynthToaParams p{};
+    p.anchors.n = n_anchors;
+    for (int i = 0; i < n_anchors; ++i) {
+        p.anchors.x[i] = anchors_xyz[3 * i]; p.anchors.y[i] = anchors_xyz[3 * i + 1]; p.anchors.z[i] = anchors_xyz[3 * i + 2];
+    }
+    p.N = n_filters; p.filter0 = gen->first_filter; p.seed = gen->seed; p.M = n_anchors;
+    p.tag_z = gen->tag_z; p.sigma_r = gen->sigma_r; p.p_missing = gen->p_missing; p.p_nlos = gen->p_nlos;
+    p.nlos_mean = gen->nlos_mean;
+    for (int k0 = 0; k0 < n_epochs; k0 += SYNTH_TOA_T) {
+        p.n_epochs = n_epochs - k0 < SYNTH_TOA_T ? n_epochs - k0 : SYNTH_TOA_T;
+        p.epoch0 = (uint32_t)(gen->first_epoch + k0);
+        memcpy(p.t, t + k0, sizeof(double) * (size_t)p.n_epochs);
+        p.ranges = (char *)o_r.d + row * (size_t)k0;
+        CK(launch_synth_toa(p, fmt == KFPOS_FMT_U16_MM, s));
+    }
+    CK(o_r.back(s));
+    // host staging is freed on return: finish the work first; device output: asynchronous on `stream`
+    if (o_r.own) CK(cudaStreamSynchronize(s));
+    return KFPOS_OK;
+}
+
 extern "C" int kfpos_selftest_math(int device, int64_t n, const double *x, double *rcp, double *rsqrt, double *sn,
                                    double *cs) {
     if (n <= 0 || !x) return KFPOS_ERR_INVALID;

@@ -394,6 +394,20 @@ struct SynthTruthParams {
     double *truth;
 };
 cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s);
+// ranging epochs of the same truth for [T][M][N] range logs (kfpos_synth_toa_ranges); a launch covers at most
+// SYNTH_TOA_T epochs, whose times travel in the parameter block (8 KB of the 32 KB it may hold)
+constexpr int SYNTH_TOA_T = 1024;
+struct SynthToaParams {
+    AnchorTable anchors;
+    int64_t N, filter0;
+    uint64_t seed;
+    int M, n_epochs;
+    uint32_t epoch0; // global index of epoch 0 of this launch (RNG counter)
+    double tag_z, sigma_r, p_missing, p_nlos, nlos_mean;
+    void *ranges; // SoA [n_epochs][M][N], int32 or uint16 mm
+    double t[SYNTH_TOA_T];
+};
+cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s); // u16: uint16 mm, else int32 mm
 
 // DFMA-only microbenchmark on the current device (the FP64 roofline denominator)
 cudaError_t measure_fp64_peak(double *flops_per_s);

@@ -1,81 +1,24 @@
-// kfpos_synth.cu -- Monte Carlo input generator for KalmanFilter (K8) batches (BASELINE configs 3 and
-// 5, SURVEY.md §8d): the multi-sensor event stream of N independent tags is synthesised on the device,
-// chunk by chunk, straight into the SoA tensors the replay kernel streams -- a 64 M-filter x 1000-step
-// run never has its inputs resident (they would be 280 GB), only the chunk in flight.
+// kfpos_synth.cu -- Monte Carlo input generators, on the device.
+//
+// synth_k8_kernel: KalmanFilter (K8) batches (BASELINE configs 3 and 5, SURVEY.md §8d): the multi-sensor
+// event stream of N independent tags is synthesised on the device, chunk by chunk, straight into the SoA
+// tensors the replay kernel streams -- a 64 M-filter x 1000-step run never has its inputs resident (they
+// would be 280 GB), only the chunk in flight.
+// synth_toa_kernel: ranging epochs for every consumer of a [T][M][N] millimetre range log (T6 / K8 / T9
+// ranging replays, the ML batch), with optional missing rangings and exponential NLOS biases (DESIGN §4.5c).
 //
 // Every value is a pure function of (seed, global filter index, event index, sample index) through
-// the counter-based Philox4x32-10 generator (Salmon et al., SC'11), so a filter's stream does not
-// depend on how the batch is sharded over GPUs or cut into chunks.
+// the counter-based Philox4x32-10 generator (Salmon et al., SC'11; kfpos_synth.cuh), so a filter's stream
+// does not depend on how the batch is sharded over GPUs or cut into chunks.
 //
 // Truth: the planar Lissajous of roskfpos_b200/synth.py  x = 5 + 3 sin(0.20 t + a), y = 5 + 3 sin(0.31 t + b),
-// heading th0 + 0.05 t;  a, b, th0 drawn per filter.  Samples per 0.1 s macro-step (same schedule as
+// heading th0 + 0.05 t;  a, b, th0 drawn per filter.  K8 samples per 0.1 s macro-step (same schedule as
 // synth.MACRO_IMU_MAG / MACRO_FULL): body-frame accelerometer + gyro (IMU), compass, PX4Flow integrals
 // (full only), and one epoch of rangings quantised to millimetres.
 #include "kfpos_kernels.cuh"
+#include "kfpos_synth.cuh"
 
 namespace kfpos {
-
-struct Philox {
-    uint32_t c[4];
-};
-KF_DEV Philox philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-        c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    return Philox{{c0, c1, c2, c3}};
-}
-// two uniforms in (0, 1) from 4 x 32 bits (53-bit mantissas, never 0)
-KF_DEV void uniform2(const Philox &p, double &u0, double &u1) {
-    const unsigned long long a = ((unsigned long long)p.c[0] << 32) | p.c[1], b = ((unsigned long long)p.c[2] << 32) | p.c[3];
-    u0 = ((double)(a >> 11) + 0.5) * (1.0 / 9007199254740992.0);
-    u1 = ((double)(b >> 11) + 0.5) * (1.0 / 9007199254740992.0);
-}
-// two standard normals (Box-Muller)
-KF_DEV void normal2(uint64_t seed, uint64_t filter, uint32_t event, uint32_t sample, double &n0, double &n1) {
-    const Philox p = philox4x32_10((uint32_t)filter, (uint32_t)(filter >> 32), event, sample, (uint32_t)seed,
-                                   (uint32_t)(seed >> 32));
-    double u0, u1, s, c;
-    uniform2(p, u0, u1);
-    const double rad = sqrt(-2.0 * log(u0));
-    sincospi(2.0 * u1, &s, &c);
-    n0 = rad * c;
-    n1 = rad * s;
-}
-
-struct Kin {
-    double px, py, vx, vy, ax, ay, th;
-};
-KF_DEV Kin kin_at(double t, double pa, double pb, double th0) {
-    Kin k;
-    double s, c;
-    sincos(0.20 * t + pa, &s, &c);
-    k.px = 5 + 3 * s; k.vx = 0.6 * c; k.ax = -0.12 * s;
-    sincos(0.31 * t + pb, &s, &c);
-    k.py = 5 + 3 * s; k.vy = 0.93 * c; k.ay = -0.2883 * s;
-    k.th = th0 + 0.05 * t;
-    return k;
-}
-
-constexpr double TWO_PI = 6.283185307179586476925286766559;
-
-// per-filter constants of the truth trajectory (event index 0xFFFFFFFF is reserved for them): phases and heading
-KF_DEV void filter_constants(uint64_t seed, uint64_t gf, double &pa, double &pb, double &th0) {
-    double ua, ub, uc, ud;
-    const Philox q = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 0u, (uint32_t)seed,
-                                   (uint32_t)(seed >> 32));
-    uniform2(q, ua, ub);
-    const Philox q2 = philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 1u, (uint32_t)seed,
-                                    (uint32_t)(seed >> 32));
-    uniform2(q2, uc, ud);
-    pa = ua * TWO_PI;
-    pb = ub * TWO_PI;
-    th0 = 0.3 + 0.2 * uc;
-}
 
 __global__ void __launch_bounds__(128) synth_k8_kernel(const SynthK8Params p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
@@ -148,7 +91,8 @@ cudaError_t launch_synth_k8(const SynthK8Params &p, cudaStream_t s) {
     return cudaGetLastError();
 }
 
-// the truth of synth_k8_kernel's filters at the given times (the per-epoch statistics of a chunked run)
+// the truth of the filters of BOTH generators, synth_k8_kernel and synth_toa_kernel, at the given times (the
+// per-epoch statistics of a chunked run): they share filter_constants and kin_at
 __global__ void __launch_bounds__(128) synth_k8_truth_kernel(const SynthTruthParams p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
     if (f >= p.N) return;
@@ -165,6 +109,63 @@ __global__ void __launch_bounds__(128) synth_k8_truth_kernel(const SynthTruthPar
 cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s) {
     if (p.N <= 0 || p.n_times <= 0) return cudaSuccess;
     synth_k8_truth_kernel<<<(unsigned)((p.N + 127) / 128), 128, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+// Ranging epochs k = 0..n_epochs of global epoch index g = epoch0 + k at time t[k], one thread per filter:
+//   d_a = |(x, y, tag_z) - anchor_a| on the truth of filter_constants / kin_at;
+//   n_a = component a & 1 of normal2(seed, gf, g, a >> 1);
+//   IMPAIR: (u, v) = uniform2(Philox(gf, g, 0x80000000 | a)): missing when u < p_missing, NLOS bias
+//           -nlos_mean log(v / p_nlos) when v < p_nlos (v / p_nlos is uniform then: one draw gives both);
+//   mm = floor((d_a + sigma_r n_a + bias) * 1000), 0 ("no ranging", TOA.cpp:50) when missing or <= 0.
+// The epoch times and the anchors are read from the parameter block: every lane reads the same one at the
+// same time (constant-bank broadcast).  Stores: SoA [k][a][N], filter index fastest -- coalesced.
+template <typename Out, bool IMPAIR>
+__global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) {
+    const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (f >= p.N) return;
+    const int64_t N = p.N;
+    const uint64_t gf = (uint64_t)(p.filter0 + f);
+    double pa, pb, th0;
+    filter_constants(p.seed, gf, pa, pb, th0);
+    Out *out = (Out *)p.ranges + f;
+    const double lim = sizeof(Out) == 2 ? 65535.0 : 2147483647.0;
+    for (int k = 0; k < p.n_epochs; ++k) {
+        const Kin kn = kin_at(p.t[k], pa, pb, th0);
+        const uint32_t g = p.epoch0 + (uint32_t)k;
+        for (int a = 0; a < p.M; a += 2) {
+            double n0, n1;
+            normal2(p.seed, gf, g, (uint32_t)(a >> 1), n0, n1);
+            for (int q = 0; q < 2 && a + q < p.M; ++q) {
+                const int i = a + q;
+                const double ex = kn.px - p.anchors.x[i], ey = kn.py - p.anchors.y[i], ez = p.tag_z - p.anchors.z[i];
+                double r = sqrt(ex * ex + ey * ey + ez * ez) + p.sigma_r * (q ? n1 : n0);
+                bool missing = false;
+                if (IMPAIR) {
+                    double u, v;
+                    uniform2(philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), g, 0x80000000u | (uint32_t)i,
+                                           (uint32_t)p.seed, (uint32_t)(p.seed >> 32)), u, v);
+                    missing = u < p.p_missing;
+                    if (v < p.p_nlos) r += -p.nlos_mean * log(v / p.p_nlos);
+                }
+                const double mm = floor(r * 1000.0);
+                out[((int64_t)k * p.M + i) * N] = (missing || !(mm > 0)) ? (Out)0 : (Out)fmin(mm, lim);
+            }
+        }
+    }
+}
+
+cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) {
+    if (p.N <= 0 || p.n_epochs <= 0) return cudaSuccess;
+    const bool imp = p.p_missing > 0 || p.p_nlos > 0;
+    const unsigned grid = (unsigned)((p.N + 127) / 128);
+    if (u16) {
+        if (imp) synth_toa_kernel<uint16_t, true><<<grid, 128, 0, s>>>(p);
+        else synth_toa_kernel<uint16_t, false><<<grid, 128, 0, s>>>(p);
+    } else {
+        if (imp) synth_toa_kernel<int32_t, true><<<grid, 128, 0, s>>>(p);
+        else synth_toa_kernel<int32_t, false><<<grid, 128, 0, s>>>(p);
+    }
     return cudaGetLastError();
 }
 

@@ -54,6 +54,13 @@ class KfposSynthEvent(C.Structure):
     _fields_ = [("kind", C.c_int32), ("global_index", C.c_int32), ("t", C.c_double), ("offset", C.c_int64)]
 
 
+class KfposSynthToa(C.Structure):
+    """kfpos_synth_toa: the ranging generator of kfpos_synth_toa_ranges."""
+    _fields_ = [("seed", C.c_uint64), ("first_filter", C.c_int64), ("first_epoch", C.c_int64),
+                ("tag_z", C.c_double), ("sigma_r", C.c_double), ("p_missing", C.c_double), ("p_nlos", C.c_double),
+                ("nlos_mean", C.c_double)]
+
+
 _LIB = None
 
 # name -> (restype, argtypes); every symbol include/kfpos_b200.h declares
@@ -100,6 +107,7 @@ SIGNATURES = {
     "kfpos_batch_epoch_stats": (_I, [_VP, _I64, _VP, _VP]),
     "kfpos_epoch_stats_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
     "kfpos_synth_k8_truth": (_I, [_I, _I64, _I64, C.c_uint64, _I, _VP, _D, _VP, _VP]),
+    "kfpos_synth_toa_ranges": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

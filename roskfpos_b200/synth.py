@@ -287,3 +287,98 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
                 "kfpos_synth_k8_truth")
         res["truth_toa"] = truth_toa
     return res
+
+
+def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED, period=0.1, sigma_r=0.10,
+                         p_missing=0.0, p_nlos=0.0, nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None,
+                         want_x0=False, want_truth=False, out=None, stream=None):
+    """Ranging epochs [epoch0, epoch0 + n_epochs) of the T6 Monte Carlo workload, generated ON THE DEVICE by
+    kfpos_synth_toa_ranges (Philox4x32-10; a ranging depends only on seed, the global filter index
+    first_filter + f, the global epoch index and the anchor, so sharding and chunking change nothing).  Epoch k
+    is at t[k] = (epoch0 + k + 1) * period; the truth is the Lissajous of kfpos_synth_k8 at height tag_z.
+    p_missing: probability that a ranging is absent (written as 0); p_nlos: probability of a positive NLOS
+    bias, exponential with mean nlos_mean (m).  fmt: lib.FMT_I32_MM (default) or lib.FMT_U16_MM.
+
+    Returns dict(ranges [n][M][N] on `device`, dt = period, t (host [n]), truth_end [3][N] = the truth at
+    t[-1], x0 [6][N] (the truth at t = 0 with zero velocity, a T6 state) if want_x0, truth [n][3][N] (from
+    kfpos_synth_k8_truth, what Batch.set_truth_traj takes for the chunk) if want_truth).  `out` may hold the
+    tensors of a previous chunk of the same shape to be reused.  ML batches take `ranges` row by row."""
+    import ctypes as C
+    import torch
+    from . import lib as L
+    fmt = L.FMT_I32_MM if fmt is None else int(fmt)
+    if fmt not in (L.FMT_I32_MM, L.FMT_U16_MM):
+        raise ValueError("toa_montecarlo_chunk: fmt must be FMT_I32_MM or FMT_U16_MM")
+    anc = np.ascontiguousarray(anchors, dtype=np.float64).reshape(-1, 3)
+    M, N, n = len(anc), int(n_filters), int(n_epochs)
+    # times from the global epoch index, so that they do not depend on where a chunk starts
+    t = np.ascontiguousarray(np.arange(epoch0 + 1, epoch0 + n + 1, dtype=np.float64) * period)
+    dev = torch.device(device)
+    out = {} if out is None else out
+
+    def buf(name, shape, dtype):
+        tns = out.get(name)
+        if tns is None or tuple(tns.shape) != tuple(shape) or tns.dtype != dtype:
+            tns = out[name] = torch.empty(shape, device=dev, dtype=dtype)
+        return tns
+    ranges = buf("ranges", (n, M, N), torch.uint16 if fmt == L.FMT_U16_MM else torch.int32)
+    gen = L.KfposSynthToa(seed=int(seed), first_filter=int(first_filter), first_epoch=int(epoch0), tag_z=float(tag_z),
+                          sigma_r=float(sigma_r), p_missing=float(p_missing), p_nlos=float(p_nlos),
+                          nlos_mean=float(nlos_mean))
+    sp = None if stream is None else C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
+    L.check(L.lib().kfpos_synth_toa_ranges(dev.index or 0, N, M, C.c_void_p(anc.ctypes.data), n,
+                                           C.c_void_p(t.ctypes.data), C.byref(gen), fmt,
+                                           C.c_void_p(ranges.data_ptr()), sp), "kfpos_synth_toa_ranges")
+
+    def truth_at(name, times):
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        tr = buf(name, (len(times), 3, N), torch.float64)
+        L.check(L.lib().kfpos_synth_k8_truth(dev.index or 0, N, int(first_filter), C.c_uint64(seed), len(times),
+                                             C.c_void_p(times.ctypes.data), float(tag_z), C.c_void_p(tr.data_ptr()),
+                                             sp), "kfpos_synth_k8_truth")
+        return tr
+    res = dict(ranges=ranges, dt=float(period), t=t)
+    if want_truth:
+        res["truth"] = truth_at("truth", t)
+        res["truth_end"] = res["truth"][-1]
+    else:
+        res["truth_end"] = truth_at("truth_end", t[-1:])[0]
+    if want_x0:
+        x0 = buf("x0", (6, N), torch.float64)
+        x0.zero_()
+        x0[:3] = truth_at("truth0", [0.0])[0]
+        res["x0"] = x0
+    return res
+
+
+def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
+                   nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
+                   stream=None):
+    """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
+    for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
+    truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
+    Batch.epoch_stats reads its rows.  init_state: start from the truth at t = 0 with zero velocity (and the
+    batch's initial covariance); False continues from the batch's state at epoch epoch0.  The batch's filter f
+    is global filter first_filter + f.  Returns the [n_epochs][6] rows of kfpos_batch_epoch_stats for
+    batch.epoch_summary (RMSE(t), ANEES(t)); the truth is unregistered on return."""
+    from . import lib as L
+    if batch.model != L.MODEL_T6:
+        raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
+    if int(chunk) <= 0 or int(n_epochs) <= 0:
+        raise ValueError("toa_montecarlo: n_epochs and chunk must be positive")
+    kw = dict(seed=seed, period=period, sigma_r=sigma_r, p_missing=p_missing, p_nlos=p_nlos, nlos_mean=nlos_mean,
+              tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream)
+    rows, bufs = [], {}
+    try:
+        for k0 in range(0, int(n_epochs), int(chunk)):
+            n = min(int(chunk), int(n_epochs) - k0)
+            w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
+                                     want_x0=init_state and k0 == 0, out=bufs, **kw)
+            if init_state and k0 == 0:
+                batch.set_state(w["x0"], None, stream=stream)
+            batch.set_truth_traj(w["truth"], stream=stream)
+            batch.replay_toa(w["dt"], w["ranges"], err=err, stream=stream)
+            rows.append(batch.epoch_stats(stream=stream))
+    finally:
+        batch.set_truth_traj(None, stream=stream)
+    return np.concatenate(rows, axis=0)
