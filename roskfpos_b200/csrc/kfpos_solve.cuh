@@ -54,6 +54,11 @@ static __device__ __noinline__ double rel_change_quotient(double q, double cost)
 static __device__ __noinline__ void count_rare_event(unsigned long long *c) { atomicAdd(c, 1ull); }
 // (and the jump over whole periods when Brent's cycle detection fires: an integer modulo)
 static __device__ __noinline__ unsigned skip_whole_periods(unsigned iter, unsigned per) { return 10000u - (10000u - iter) % per; }
+// (the same with its rare-event counter, for the EKFs' inner solver: one call site in the Newton loop instead of two)
+static __device__ __noinline__ unsigned skip_whole_periods_counted(unsigned iter, unsigned per, unsigned long long *cnt) {
+    if (cnt) atomicAdd(cnt + CNT_ML_CYCLES, 1ull);
+    return 10000u - (10000u - iter) % per;
+}
 KF_DEV bool rel_change_gt(double cost, double newCost) {
     const double q = fabs(cost - newCost);
     if (cost > 0.0) {
@@ -365,8 +370,7 @@ KF_DEV int ml_solve3_ekf(const AnchorTable &A, const EpochT<false, MT> &ep, unsi
             cyc_ref[0] = p[0]; cyc_ref[1] = p[1]; cyc_ref[2] = p[2];
         } else if (p[0] == cyc_ref[0] && p[1] == cyc_ref[1] && p[2] == cyc_ref[2]) {
             const unsigned per = iter - (1u << (31 - __clz(iter)));
-            iter = skip_whole_periods(iter, per);
-            if (cnt) count_rare_event(cnt + CNT_ML_CYCLES);
+            iter = skip_whole_periods_counted(iter, per, cnt);
         }
     }
     if (cnt && iter >= 10000u) count_rare_event(cnt + CNT_ML_CAPPED);
@@ -865,27 +869,34 @@ KF_DEV void prefetch_epoch(const RAW &raw, int m, const void *ranges, int fmt, i
 }
 
 // landing zone -> metres + valid mask: keep rangings[i] > 0 (TOA.cpp:48-57, ML.cpp:478)
-template <bool PME, int MT, class RAW>
+// WIRE_MASK: the mask of the millimetre formats from the integer (mm > 0 exactly when mm / 1000 > 0), an integer compare
+// instead of an FP64 one per ranging (the T6 replay)
+template <bool PME, int MT, class RAW, bool WIRE_MASK = false>
 KF_DEV void convert_epoch(EpochT<PME, MT> &ep, const RAW &raw, const void *ranges, int fmt, const double *err,
                           int64_t base, int64_t N) {
     unsigned valid = 0u;
 #pragma unroll(MT > 0 ? MT : 1)
     for (int i = 0; i < ep.m(); ++i) {
         double r;
+        bool on;
         if (fmt == 0) {
             r = *raw.d(i);
+            on = r > 0;
         } else {
             const unsigned w = *raw.w(i);
             if (fmt == 1) {
                 r = mm_to_m((double)(int)w);
+                on = (int)w > 0;
             } else {
                 const uintptr_t a = reinterpret_cast<uintptr_t>(reinterpret_cast<const uint16_t *>(ranges) + base + (int64_t)i * N);
-                r = mm_to_m((double)((a & 2) ? (w >> 16) : (w & 0xffffu)));
+                const unsigned v = (a & 2) ? (w >> 16) : (w & 0xffffu);
+                r = mm_to_m((double)v);
+                on = v != 0u;
             }
         }
         if (MT > 0) ep.zr[i] = r;
         else ep.z[i] = r;
-        if (r > 0) valid |= 1u << i;
+        if (WIRE_MASK ? on : r > 0) valid |= 1u << i;
         if (PME) ep.e[i] = __ldg(err + base + (int64_t)i * N);
     }
     ep.valid = valid;

@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
             }
             // ---- this epoch's rangings (landed during the previous epoch); start the next fetch
             cp_async_wait_all();
-            convert_epoch<PME, MT>(ep, raw, p.rs.ranges, fmt, p.rs.err, (int64_t)t * m * N + f, N);
+            convert_epoch<PME, MT, RawCol, true>(ep, raw, p.rs.ranges, fmt, p.rs.err, (int64_t)t * m * N + f, N);
             if (t + 1 < p.T) prefetch_epoch(raw, m, p.rs.ranges, fmt, (int64_t)(t + 1) * m * N + f, N);
 
             st.status = 0u;

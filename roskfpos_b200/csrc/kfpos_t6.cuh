@@ -96,17 +96,13 @@ KF_DEV int t6_update(const AnchorTable &A, const EpochT<PME, MT> &ep, unsigned m
     double cost = 1e20;
     double prior = 0.0; // delta^T pinv(P^-) delta
     bool broke = false;
+    // the sums of the first iteration (scalar errorEstimation: those of the Newton solver's first pass) as the initial
+    // values of the loop-carried ones, not copied in the loop (~40 moves inside the replay loop)
+    double c = sse_xp, b[3] = {-g_xp[0], -g_xp[1], -g_xp[2]}, G[6] = {Gu_xp[0], Gu_xp[1], Gu_xp[2], Gu_xp[3], Gu_xp[4], Gu_xp[5]};
     for (int iter = 0; iter < 10; ++iter) {
         // ---- one pass: cost at the current iterate (TOA.cpp:297-305) and the
         //      information-form accumulators of the rows linearised there (TOA.cpp:313-320)
-        double c, b[3], G[6];
-        if (!PME && iter == 0) {
-            c = sse_xp;
-#pragma unroll
-            for (int k = 0; k < 3; ++k) b[k] = -g_xp[k];
-#pragma unroll
-            for (int k = 0; k < 6; ++k) G[k] = Gu_xp[k];
-        } else {
+        if (PME || iter > 0) {
             if constexpr (COSTFIRST && !PME && MT > 0) {
                 if (iter >= 2) { // the evaluation that usually ends the loop: the cost alone first (iekf_cost_only)
                     const double c2 = iekf_cost_only<MT>(A, ep, mask, xp[0] + dx[0], xp[1] + dx[1], xp[2] + dx[2]);
