@@ -23,6 +23,7 @@
  *  - `stream` is a cudaStream_t passed as void* (NULL = the legacy default
  *    stream); work is enqueued on it, calls taking host pointers synchronise it
  *    before returning;
+ *    the small arrays declared as HOST arrays (dt, event schedules, ...) do not count;
  *  - calls on one handle must be serialised by the caller (the reference is
  *    single-threaded: publishers/node_pos.cpp:176-181); handles are independent;
  *  - there is NO CPU fallback: without a usable CUDA device every call fails

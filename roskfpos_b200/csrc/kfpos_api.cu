@@ -74,7 +74,7 @@ struct kfpos_batch {
     double *d_truth_own = nullptr;
     bool partials_fresh = false;
     bool out4_valid = false; // d_out4 holds the statistics of the current state
-    double *d_gather = nullptr; // [n_ranks][4] of kfpos_stats_allreduce
+    DevBuf gather; // [n_ranks][4] of kfpos_stats_allreduce
     // per-epoch statistics (kfpos_batch_set_truth_traj): truth rows SoA [es_rows][3][N], per-warp sums
     // [es_rows][n_warps][6] left by the replay kernels, the next output row, and the fold buffers
     const double *d_etruth = nullptr;
@@ -128,28 +128,158 @@ bool on_device(const void *p) {
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
-size_t fmt_size(int fmt) { return fmt == KFPOS_FMT_F64_M ? 8 : (fmt == KFPOS_FMT_I32_MM ? 4 : 2); }
+// Argument staging of one call.  Device pointers pass through; a host data array goes through a device buffer,
+// and then the call synchronises its stream before returning (include/kfpos_b200.h, Conventions).  The buffers of
+// a call on a batch are the slots of its scratch pool, taken one after the other in the order the call asks for
+// them, so two buffers of one call never alias; a call without a handle allocates its own and frees them on return.
+// Errors are sticky: after a failed step every later one is skipped and `rc` holds the first error, which the
+// caller checks before it launches anything that reads the buffers.
+class Staging {
+  public:
+    int rc = KFPOS_OK;
+    bool sync = false; // finish() synchronises: a host data array was read or written, or a buffer is freed on return
 
-// input staging: device pointers pass through, host pointers are copied into
-// scratch slot `slot`
-int stage_in(kfpos_batch *b, int slot, const void *src, size_t bytes, cudaStream_t s, const void **out) {
-    if (!src) { *out = nullptr; return KFPOS_OK; }
-    if (on_device(src)) { *out = src; return KFPOS_OK; }
-    CK(b->scratch[slot].reserve(bytes));
-    CK(cudaMemcpyAsync(b->scratch[slot].p, src, bytes, cudaMemcpyHostToDevice, s));
-    *out = b->scratch[slot].p;
+    Staging(kfpos_batch *b, cudaStream_t s) : pool_(b->scratch), s_(s) {}
+    explicit Staging(cudaStream_t s) : s_(s) {}
+    Staging(const Staging &) = delete;
+    Staging &operator=(const Staging &) = delete;
+    ~Staging() {
+        for (void *p : own_) cudaFree(p);
+    }
+
+    // a device array for the call's own intermediates
+    template <class T = void> T *buf(size_t bytes) { return static_cast<T *>(alloc(bytes)); }
+    // a data array the call reads
+    template <class T> const T *in(const T *p, size_t bytes) {
+        if (!p || on_device(p)) return p;
+        T *d = buf<T>(bytes);
+        copy(d, p, bytes, cudaMemcpyHostToDevice);
+        sync = true;
+        return d;
+    }
+    // a data array the call writes: a host array gets a device buffer that finish() copies back
+    template <class T> T *out(T *p, size_t bytes) {
+        if (!p || on_device(p)) return p;
+        T *d = buf<T>(bytes);
+        if (d) back_.push_back({p, d, bytes});
+        sync = true;
+        return d;
+    }
+    // a small control array (the ones the header declares as HOST arrays: time steps, event schedules, slot
+    // tables), always copied.  It does not make the call synchronise: a copy from pageable memory has left the
+    // caller's array when cudaMemcpyAsync returns.
+    template <class T> const T *ctl(const T *p, size_t bytes) {
+        T *d = buf<T>(bytes);
+        copy(d, p, bytes, on_device(p) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice);
+        return d;
+    }
+    // direct copies between a caller's data array and batch memory; a null array is skipped
+    void copy_in(void *dst_dev, const void *src, size_t bytes) {
+        if (!src) return;
+        const bool host = !on_device(src);
+        copy(dst_dev, src, bytes, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice);
+        sync = sync || host;
+    }
+    void copy_out(void *dst, const void *src_dev, size_t bytes) {
+        if (!dst) return;
+        const bool host = !on_device(dst);
+        copy(dst, src_dev, bytes, host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice);
+        sync = sync || host;
+    }
+    // enqueues the copy-backs of out(), synchronises if `sync`, and returns the status of the call
+    int finish() {
+        for (const Back &c : back_) copy(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost);
+        if (sync && rc == KFPOS_OK) fail(cudaStreamSynchronize(s_));
+        return rc;
+    }
+
+  private:
+    struct Back {
+        void *host;
+        const void *dev;
+        size_t bytes;
+    };
+    DevBuf *pool_ = nullptr;
+    int next_ = 0;
+    cudaStream_t s_;
+    std::vector<void *> own_;
+    std::vector<Back> back_;
+
+    void fail(cudaError_t e) {
+        if (e != cudaSuccess && rc == KFPOS_OK) rc = map_cuda_err(e);
+    }
+    void copy(void *dst, const void *src, size_t bytes, cudaMemcpyKind kind) {
+        if (rc == KFPOS_OK) fail(cudaMemcpyAsync(dst, src, bytes, kind, s_));
+    }
+    void *alloc(size_t bytes) {
+        if (rc != KFPOS_OK) return nullptr;
+        if (!pool_) {
+            void *p = nullptr;
+            fail(cudaMalloc(&p, bytes));
+            if (p) own_.push_back(p);
+            sync = true; // freed on return: the work that uses it has to be done by then
+            return p;
+        }
+        if (next_ == N_SCRATCH) { // N_SCRATCH covers the call with the most buffers, kfpos_batch_ml_solve
+            rc = KFPOS_ERR_NOMEM;
+            return nullptr;
+        }
+        DevBuf &d = pool_[next_++];
+        fail(d.reserve(bytes));
+        return rc == KFPOS_OK ? d.p : nullptr;
+    }
+};
+
+// KFPOS_ERR_CUDA unless `device` is a CUDA device of this process
+int check_device(int device) {
+    int count = 0;
+    if (cudaGetDeviceCount(&count) == cudaSuccess && device >= 0 && device < count) return KFPOS_OK;
+    cudaGetLastError();
+    return KFPOS_ERR_CUDA;
+}
+
+// reads `bytes` of a host or device array on the host
+int to_host(void *dst, const void *src, size_t bytes) {
+    if (on_device(src)) CK(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost));
+    else memcpy(dst, src, bytes);
     return KFPOS_OK;
 }
 
-// output staging: returns the device pointer the kernel should write
-int stage_out(kfpos_batch *b, int slot, void *dst, size_t bytes, void **dev, bool *needs_copy) {
-    *needs_copy = false;
-    if (!dst) { *dev = nullptr; return KFPOS_OK; }
-    if (on_device(dst)) { *dev = dst; return KFPOS_OK; }
-    CK(b->scratch[slot].reserve(bytes));
-    *dev = b->scratch[slot].p;
-    *needs_copy = true;
+// the anchor table of `n` (x, y, z) triples in a host or device array
+int anchor_table(int n, const double *xyz, AnchorTable *t) {
+    double host[3 * KFPOS_MAX_ANCHORS];
+    int rc = to_host(host, xyz, sizeof(double) * 3 * (size_t)n);
+    if (rc) return rc;
+    memset(t, 0, sizeof *t);
+    for (int i = 0; i < n; ++i) {
+        t->x[i] = host[3 * i];
+        t->y[i] = host[3 * i + 1];
+        t->z[i] = host[3 * i + 2];
+    }
+    t->n = n;
     return KFPOS_OK;
+}
+
+size_t fmt_size(int fmt) { return fmt == KFPOS_FMT_F64_M ? 8 : (fmt == KFPOS_FMT_I32_MM ? 4 : 2); }
+bool fmt_ok(int fmt) { return fmt >= KFPOS_FMT_F64_M && fmt <= KFPOS_FMT_U16_MM; }
+
+// rows of N values one event writes or reads in its log: the M rangings of a TOA event, the payload rows of a
+// sensor event (header, kfpos_event); -1 for an unknown kind
+int event_rows(int kind, int M) {
+    static const int payload[5] = {0, 5, 3, 2, 1}; // -, PX4, IMU, MAG, COMPASS
+    if (kind < KFPOS_EV_TOA || kind > KFPOS_EV_COMPASS) return -1;
+    return kind == KFPOS_EV_TOA ? M : payload[kind];
+}
+
+// T epochs of a [T][M][N] range log as a K8 / T9 schedule of TOA events; dt null: the time steps are per filter
+std::vector<kfpos_event> toa_schedule(size_t T, size_t M, const double *dt) {
+    std::vector<kfpos_event> evs(T); // zero-initialised
+    for (size_t t = 0; t < T; ++t) {
+        evs[t].kind = KFPOS_EV_TOA;
+        evs[t].dt = dt ? dt[t] : 0.0;
+        evs[t].offset = (int64_t)(t * M);
+    }
+    return evs;
 }
 
 int state_dim(int model) {
@@ -189,6 +319,34 @@ void es_bind(kfpos_batch *b, Params &p, int64_t rows) {
     b->es_cursor += rows;
 }
 
+// the fields the T6, K8 and T9 replay parameters share (kept apart in each struct: a shared sub-struct would move
+// the kernel parameter offsets); the launch has `rows` output rows
+template <class Params>
+void bind_replay(kfpos_batch *b, Params &p, const RangeStream &rs, const double *dt_f, double *traj, int64_t rows) {
+    p.anchors = b->anchors;
+    p.rs = rs;
+    p.N = b->N;
+    p.x = b->d_x;
+    p.P = b->d_P;
+    p.status = b->d_status;
+    p.dt_f = dt_f;
+    p.traj = traj;
+    p.counters = b->d_counters;
+    p.truth = b->d_truth;
+    p.partials = b->d_partials;
+    es_bind(b, p, rows);
+}
+
+// after a replay launch: the partials of a registered truth are those of the new state, the folded statistics are
+// stale, and (K8 / T9) the latched IMU covariances the launch wrote move to where the next launch reads them
+int replayed(kfpos_batch *b, cudaStream_t s) {
+    if (b->d_latch_u)
+        CK(cudaMemcpyAsync(b->d_latch_u, b->d_latch_u + 16, sizeof(double) * 16, cudaMemcpyDeviceToDevice, s));
+    b->partials_fresh = b->d_truth != nullptr;
+    b->out4_valid = false;
+    return KFPOS_OK;
+}
+
 } // namespace
 
 // ------------------------------------------------------------------------ misc
@@ -212,11 +370,7 @@ extern "C" int kfpos_batch_create(kfpos_batch **out, int device, int model, int6
                                   const kfpos_config *cfg) {
     if (!out || !cfg || n_filters <= 0 || state_dim(model) == 0) return KFPOS_ERR_INVALID;
     *out = nullptr;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     kfpos_batch *b = new (std::nothrow) kfpos_batch();
@@ -241,7 +395,7 @@ extern "C" int kfpos_batch_create(kfpos_batch **out, int device, int model, int6
         alloc((void **)&b->d_status, sizeof(int32_t) * N);
         alloc((void **)&b->d_partials, sizeof(double) * 4 * ((N + STATS_CHUNK - 1) / STATS_CHUNK));
         alloc((void **)&b->d_out4, sizeof(double) * 4);
-        alloc((void **)&b->d_gather, sizeof(double) * 4 * 1024);
+        if (e == cudaSuccess) e = b->gather.reserve(sizeof(double) * 4 * 1024);
     }
     if (model == KFPOS_MODEL_K8 || model == KFPOS_MODEL_T9) {
         alloc((void **)&b->d_latch, sizeof(double) * 16 * N);
@@ -286,7 +440,7 @@ extern "C" void kfpos_batch_destroy(kfpos_batch *b) {
     cudaFree(b->d_partials);
     cudaFree(b->d_out4);
     cudaFree(b->d_truth_own);
-    cudaFree(b->d_gather);
+    b->gather.release();
     cudaFree(b->d_etruth_own);
     cudaFree(b->d_escratch);
     cudaFree(b->d_efold);
@@ -317,20 +471,11 @@ extern "C" int kfpos_batch_state_dim(const kfpos_batch *b) { return b ? b->n : 0
 
 extern "C" int kfpos_batch_set_anchors(kfpos_batch *b, int n_anchors, const double *xyz) {
     if (!b || !xyz || n_anchors < 0 || n_anchors > KFPOS_MAX_ANCHORS) return KFPOS_ERR_INVALID;
-    std::vector<double> host(3 * (size_t)n_anchors);
-    if (on_device(xyz)) {
-        DeviceGuard g(b->device);
-        CK(cudaMemcpy(host.data(), xyz, host.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    } else {
-        memcpy(host.data(), xyz, host.size() * sizeof(double));
-    }
-    memset(&b->anchors, 0, sizeof b->anchors);
-    for (int i = 0; i < n_anchors; ++i) {
-        b->anchors.x[i] = host[3 * i];
-        b->anchors.y[i] = host[3 * i + 1];
-        b->anchors.z[i] = host[3 * i + 2];
-    }
-    b->anchors.n = n_anchors;
+    DeviceGuard g(b->device);
+    AnchorTable t;
+    int rc = anchor_table(n_anchors, xyz, &t);
+    if (rc) return rc;
+    b->anchors = t;
     b->have_anchors = true;
     return KFPOS_OK;
 }
@@ -340,13 +485,12 @@ extern "C" int kfpos_batch_set_state(kfpos_batch *b, const double *x, const doub
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    const bool xd = on_device(x);
-    CK(cudaMemcpyAsync(b->d_x, x, sizeof(double) * b->n * N, xd ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
-    if (P) {
-        const void *pf = nullptr;
-        int rc = stage_in(b, 0, P, sizeof(double) * b->n * b->n * N, s, &pf);
-        if (rc) return rc;
-        CK(launch_pack_cov(b->n, b->N, (const double *)pf, b->d_P, s));
+    Staging st(b, s);
+    st.copy_in(b->d_x, x, sizeof(double) * b->n * N);
+    const double *d_P = st.in(P, sizeof(double) * b->n * b->n * N);
+    if (st.rc) return st.rc;
+    if (d_P) {
+        CK(launch_pack_cov(b->n, b->N, d_P, b->d_P, s));
     } else {
         CK(cudaMemsetAsync(b->d_P, 0, sizeof(double) * b->np * N, s));
     }
@@ -363,52 +507,34 @@ extern "C" int kfpos_batch_set_state(kfpos_batch *b, const double *x, const doub
     b->out4_valid = false;
     b->es_cursor = 0;
     b->stepped = P != nullptr; // a restored checkpoint is a running filter; P0 = 0 is a fresh one
-    if (!xd || (P && !on_device(P))) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 extern "C" int kfpos_batch_get_latches(kfpos_batch *b, double *latch, int32_t *has, double *latch_u, void *stream) {
     if (!b || !b->d_latch) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
-    cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    bool sync = false;
-    auto out = [&](void *dst, const void *src, size_t bytes) {
-        if (!dst) return cudaSuccess;
-        const bool d = on_device(dst);
-        sync |= !d;
-        return cudaMemcpyAsync(dst, src, bytes, d ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s);
-    };
-    CK(out(latch, b->d_latch, sizeof(double) * 16 * N));
-    CK(out(has, b->d_has, sizeof(int32_t) * N));
-    CK(out(latch_u, b->d_latch_u, sizeof(double) * 16));
-    if (sync) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    Staging st(b, (cudaStream_t)stream);
+    st.copy_out(latch, b->d_latch, sizeof(double) * 16 * N);
+    st.copy_out(has, b->d_has, sizeof(int32_t) * N);
+    st.copy_out(latch_u, b->d_latch_u, sizeof(double) * 16);
+    return st.finish();
 }
 
 extern "C" int kfpos_batch_set_latches(kfpos_batch *b, const double *latch, const int32_t *has, const double *latch_u,
                                        void *stream) {
     if (!b || !b->d_latch) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
-    cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    bool sync = false;
-    auto in = [&](void *dst, const void *src, size_t bytes) {
-        if (!src) return cudaSuccess;
-        const bool d = on_device(src);
-        sync |= !d;
-        return cudaMemcpyAsync(dst, src, bytes, d ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s);
-    };
-    CK(in(b->d_latch, latch, sizeof(double) * 16 * N));
-    CK(in(b->d_has, has, sizeof(int32_t) * N));
-    if (latch_u) {
-        CK(in(b->d_latch_u, latch_u, sizeof(double) * 16));
-        CK(in(b->d_latch_u + 16, latch_u, sizeof(double) * 16));
-    }
+    Staging st(b, (cudaStream_t)stream);
+    st.copy_in(b->d_latch, latch, sizeof(double) * 16 * N);
+    st.copy_in(b->d_has, has, sizeof(int32_t) * N);
+    st.copy_in(b->d_latch_u, latch_u, sizeof(double) * 16);
+    st.copy_in(b->d_latch_u + 16, latch_u, sizeof(double) * 16);
+    if (st.rc) return st.rc;
     if (has) b->imu_seen = true; // T9: a restored filter may carry a latched IMU sample
     b->stepped = true;
-    if (sync) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 extern "C" int kfpos_batch_get_state(kfpos_batch *b, double *x, double *P, int32_t *status, void *stream) {
@@ -416,43 +542,25 @@ extern "C" int kfpos_batch_get_state(kfpos_batch *b, double *x, double *P, int32
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    bool sync = false;
-    if (x) {
-        const bool d = on_device(x);
-        CK(cudaMemcpyAsync(x, b->d_x, sizeof(double) * b->n * N, d ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
-        sync |= !d;
-    }
-    if (P) {
-        void *dev;
-        bool copy;
-        const size_t bytes = sizeof(double) * b->n * b->n * N;
-        int rc = stage_out(b, 0, P, bytes, &dev, &copy);
-        if (rc) return rc;
-        CK(launch_unpack_cov(b->n, b->N, b->d_P, (double *)dev, s));
-        if (copy) {
-            CK(cudaMemcpyAsync(P, dev, bytes, cudaMemcpyDeviceToHost, s));
-            sync = true;
-        }
-    }
-    if (status) {
-        const bool d = on_device(status);
-        CK(cudaMemcpyAsync(status, b->d_status, sizeof(int32_t) * N, d ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
-        sync |= !d;
-    }
-    if (sync) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    Staging st(b, s);
+    st.copy_out(x, b->d_x, sizeof(double) * b->n * N);
+    double *d_P = st.out(P, sizeof(double) * b->n * b->n * N);
+    if (st.rc) return st.rc;
+    if (d_P) CK(launch_unpack_cov(b->n, b->N, b->d_P, d_P, s));
+    st.copy_out(status, b->d_status, sizeof(int32_t) * N);
+    return st.finish();
 }
 
 // ------------------------------------------------------------------- TOA steps
 namespace {
 
-// launches the model's replay kernel over T steps whose ranges (and optional
+// launches the T6 replay kernel over T steps whose ranges (and optional
 // per-ranging errors) are already on the device
-int launch_replay(kfpos_batch *b, int T, const double *d_dt, const void *d_ranges, int fmt,
-                  double err_scalar, const double *d_err, double *d_traj, int32_t *d_sel, cudaStream_t s,
-                  const double *d_dt_f = nullptr);
-int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_ranges, int fmt, double err_scalar,
-               const double *d_err, const double *d_sensors, double *d_traj, cudaStream_t s,
+int launch_t6(kfpos_batch *b, int T, const double *d_dt, const void *d_ranges, int fmt,
+              double err_scalar, const double *d_err, double *d_traj, int32_t *d_sel, cudaStream_t s,
+              const double *d_dt_f = nullptr);
+int run_events(kfpos_batch *b, Staging &st, int n, const kfpos_event *events, const void *d_ranges, int fmt,
+               double err_scalar, const double *d_err, const double *d_sensors, double *d_traj, cudaStream_t s,
                const double *d_dt_f = nullptr);
 
 } // namespace
@@ -460,55 +568,39 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
 extern "C" int kfpos_batch_replay_toa(kfpos_batch *b, int n_steps, const double *dt, const void *ranges,
                                       int fmt, double err_scalar, const double *err_var, double *traj,
                                       int32_t *sel, void *stream) {
-    if (!b || b->model == KFPOS_MODEL_ML || n_steps < 0 || !dt || !ranges) return KFPOS_ERR_INVALID;
-    if (fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
+    if (!b || b->model == KFPOS_MODEL_ML || n_steps < 0 || !dt || !ranges || !fmt_ok(fmt)) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     if (n_steps == 0) return KFPOS_OK;
     if (es_check(b, n_steps)) return KFPOS_ERR_INVALID;
+    if (sel && b->model != KFPOS_MODEL_T6) return KFPOS_ERR_INVALID; // leave-one-out exists only in T6
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n;
     const int T = n_steps;
-
-    // dt: small, always staged
-    CK(b->scratch[1].reserve(sizeof(double) * T));
-    CK(cudaMemcpyAsync(b->scratch[1].p, dt, sizeof(double) * T,
-                       on_device(dt) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
-    const double *d_dt = (const double *)b->scratch[1].p;
-
-    void *d_traj = nullptr, *d_sel = nullptr;
-    bool copy_traj = false, copy_sel = false;
-    int rc = stage_out(b, 2, traj, sizeof(double) * 3 * N * T, &d_traj, &copy_traj);
-    if (rc) return rc;
-    rc = stage_out(b, 3, sel, sizeof(int32_t) * N * T, &d_sel, &copy_sel);
-    if (rc) return rc;
-
-    const bool r_dev = on_device(ranges);
-    const bool e_dev = !err_var || on_device(err_var);
+    const size_t range_bytes = M * N * T * fmt_size(fmt), err_bytes = sizeof(double) * M * N * T;
+    Staging st(b, s);
+    double *d_traj = st.out(traj, sizeof(double) * 3 * N * T);
+    int32_t *d_sel = st.out(sel, sizeof(int32_t) * N * T);
+    int rc = KFPOS_OK;
     if (b->model != KFPOS_MODEL_T6) {
         // K8 / T9: a TOA-only schedule through the event-stream kernel
         std::vector<double> hdt(T);
-        if (on_device(dt)) CK(cudaMemcpy(hdt.data(), dt, sizeof(double) * T, cudaMemcpyDeviceToHost));
-        else memcpy(hdt.data(), dt, sizeof(double) * T);
-        std::vector<kfpos_event> evs(T);
-        for (int t = 0; t < T; ++t) {
-            memset(&evs[t], 0, sizeof(kfpos_event));
-            evs[t].kind = KFPOS_EV_TOA;
-            evs[t].dt = hdt[t];
-            evs[t].offset = (int64_t)t * (int64_t)M;
-        }
-        if (sel) return KFPOS_ERR_INVALID; // leave-one-out exists only in T6
-        const void *d_r = nullptr, *d_e = nullptr;
-        rc = stage_in(b, 4, ranges, M * N * T * fmt_size(fmt), s, &d_r);
-        if (rc) return rc;
-        rc = stage_in(b, 5, err_var, sizeof(double) * M * N * T, s, &d_e);
-        if (rc) return rc;
-        rc = run_events(b, T, evs.data(), d_r, fmt, err_scalar, (const double *)d_e, nullptr, (double *)d_traj, s);
-        if (rc) return rc;
-    } else if (r_dev && e_dev) {
-        rc = launch_replay(b, T, d_dt, ranges, fmt, err_scalar, err_var, (double *)d_traj, (int32_t *)d_sel, s);
-        if (rc) return rc;
-    } else if (!r_dev && err_var == nullptr) {
+        if ((rc = to_host(hdt.data(), dt, sizeof(double) * T))) return rc;
+        const std::vector<kfpos_event> evs = toa_schedule(T, M, hdt.data());
+        const void *d_r = st.in(ranges, range_bytes);
+        const double *d_e = st.in(err_var, err_bytes);
+        rc = run_events(b, st, T, evs.data(), d_r, fmt, err_scalar, d_e, nullptr, d_traj, s);
+        return rc ? rc : st.finish();
+    }
+    const double *d_dt = st.ctl(dt, sizeof(double) * T); // small: always staged
+    if (on_device(ranges) || err_var) {
+        // the whole log on the device (host arrays staged whole)
+        const void *d_r = st.in(ranges, range_bytes);
+        const double *d_e = st.in(err_var, err_bytes);
+        if (st.rc) return st.rc;
+        rc = launch_t6(b, T, d_dt, d_r, fmt, err_scalar, d_e, d_traj, d_sel, s);
+    } else {
+        if (st.rc) return st.rc;
         // HOST range log: stream it through two device staging buffers, the copy
         // of chunk c+1 overlapping the replay kernel of chunk c.
         // Chunk size: the replay of the LAST chunk is the only kernel time the copies do not hide, so chunks are
@@ -533,27 +625,14 @@ extern "C" int kfpos_batch_replay_toa(kfpos_batch *b, int n_steps, const double 
                                cudaMemcpyHostToDevice, b->copy_stream));
             CK(cudaEventRecord(b->ev_copied[k], b->copy_stream));
             CK(cudaStreamWaitEvent(s, b->ev_copied[k], 0));
-            rc = launch_replay(b, (int)tc, d_dt + t0, b->stage[k].p, fmt, err_scalar, nullptr,
-                               d_traj ? (double *)d_traj + t0 * 3 * N : nullptr,
-                               d_sel ? (int32_t *)d_sel + t0 * N : nullptr, s);
+            rc = launch_t6(b, (int)tc, d_dt + t0, b->stage[k].p, fmt, err_scalar, nullptr,
+                           d_traj ? d_traj + t0 * 3 * N : nullptr, d_sel ? d_sel + t0 * N : nullptr, s);
             if (rc) return rc;
             CK(cudaEventRecord(b->ev_done[k], s));
         }
-    } else {
-        // host ranges with per-ranging errors (or mixed): stage both whole
-        const void *d_r = nullptr, *d_e = nullptr;
-        rc = stage_in(b, 4, ranges, M * N * T * fmt_size(fmt), s, &d_r);
-        if (rc) return rc;
-        rc = stage_in(b, 5, err_var, sizeof(double) * M * N * T, s, &d_e);
-        if (rc) return rc;
-        rc = launch_replay(b, T, d_dt, d_r, fmt, err_scalar, (const double *)d_e, (double *)d_traj,
-                           (int32_t *)d_sel, s);
-        if (rc) return rc;
+        st.sync = true; // the host log is read by the chunk copies
     }
-    if (copy_traj) CK(cudaMemcpyAsync(traj, d_traj, sizeof(double) * 3 * N * T, cudaMemcpyDeviceToHost, s));
-    if (copy_sel) CK(cudaMemcpyAsync(sel, d_sel, sizeof(int32_t) * N * T, cudaMemcpyDeviceToHost, s));
-    if (copy_traj || copy_sel || !r_dev || !e_dev) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return rc ? rc : st.finish();
 }
 
 extern "C" int kfpos_batch_replay_epochs(kfpos_batch *b, int n_steps, const double *dt_per_filter, const void *ranges,
@@ -561,39 +640,27 @@ extern "C" int kfpos_batch_replay_epochs(kfpos_batch *b, int n_steps, const doub
                                          void *stream) {
     if (!b || n_steps < 0 || !dt_per_filter || !ranges) return KFPOS_ERR_INVALID;
     if (b->model != KFPOS_MODEL_T6 && b->model != KFPOS_MODEL_K8 && b->model != KFPOS_MODEL_T9) return KFPOS_ERR_INVALID;
-    if (fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
+    if (!fmt_ok(fmt)) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     if (n_steps == 0) return KFPOS_OK;
     if (es_check(b, n_steps)) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n, T = (size_t)n_steps;
-    const void *d_dtf = nullptr, *d_r = nullptr, *d_e = nullptr;
-    int rc = stage_in(b, 1, dt_per_filter, sizeof(double) * N * T, s, &d_dtf);
-    if (rc) return rc;
-    if ((rc = stage_in(b, 4, ranges, M * N * T * fmt_size(fmt), s, &d_r))) return rc;
-    if ((rc = stage_in(b, 5, err_var, sizeof(double) * M * N * T, s, &d_e))) return rc;
-    void *d_traj = nullptr;
-    bool copy_traj = false;
-    if ((rc = stage_out(b, 2, traj, sizeof(double) * 3 * N * T, &d_traj, &copy_traj))) return rc;
+    Staging st(b, s);
+    const double *d_dtf = st.in(dt_per_filter, sizeof(double) * N * T);
+    const void *d_r = st.in(ranges, M * N * T * fmt_size(fmt));
+    const double *d_e = st.in(err_var, sizeof(double) * M * N * T);
+    double *d_traj = st.out(traj, sizeof(double) * 3 * N * T);
+    int rc;
     if (b->model == KFPOS_MODEL_T6) {
-        rc = launch_replay(b, n_steps, nullptr, d_r, fmt, err_scalar, (const double *)d_e, (double *)d_traj, nullptr, s,
-                           (const double *)d_dtf);
+        if (st.rc) return st.rc;
+        rc = launch_t6(b, n_steps, nullptr, d_r, fmt, err_scalar, d_e, d_traj, nullptr, s, d_dtf);
     } else { // K8 / T9: the epochs as a schedule of ranging events whose time steps are per filter
-        std::vector<kfpos_event> evs(T);
-        for (size_t t = 0; t < T; ++t) {
-            memset(&evs[t], 0, sizeof(kfpos_event));
-            evs[t].kind = KFPOS_EV_TOA;
-            evs[t].offset = (int64_t)t * (int64_t)M;
-        }
-        rc = run_events(b, n_steps, evs.data(), d_r, fmt, err_scalar, (const double *)d_e, nullptr, (double *)d_traj, s,
-                        (const double *)d_dtf);
+        const std::vector<kfpos_event> evs = toa_schedule(T, M, nullptr);
+        rc = run_events(b, st, n_steps, evs.data(), d_r, fmt, err_scalar, d_e, nullptr, d_traj, s, d_dtf);
     }
-    if (rc) return rc;
-    if (copy_traj) CK(cudaMemcpyAsync(traj, d_traj, sizeof(double) * 3 * N * T, cudaMemcpyDeviceToHost, s));
-    if (copy_traj || !on_device(ranges) || !on_device(dt_per_filter) || (err_var && !on_device(err_var)))
-        CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return rc ? rc : st.finish();
 }
 
 extern "C" int kfpos_batch_step_toa(kfpos_batch *b, double dt, const void *ranges, int fmt, double err_scalar,
@@ -603,42 +670,23 @@ extern "C" int kfpos_batch_step_toa(kfpos_batch *b, double dt, const void *range
 
 namespace {
 
-int launch_replay(kfpos_batch *b, int T, const double *d_dt, const void *d_ranges, int fmt,
-                  double err_scalar, const double *d_err, double *d_traj, int32_t *d_sel, cudaStream_t s,
-                  const double *d_dt_f) {
-    const RangeStream rs = make_rs(b, d_ranges, fmt, err_scalar, d_err);
+int launch_t6(kfpos_batch *b, int T, const double *d_dt, const void *d_ranges, int fmt,
+              double err_scalar, const double *d_err, double *d_traj, int32_t *d_sel, cudaStream_t s,
+              const double *d_dt_f) {
     b->stepped = true;
-    switch (b->model) {
-    case KFPOS_MODEL_T6: {
-        T6Params p;
-        p.anchors = b->anchors;
-        p.rs = rs;
-        p.N = b->N;
-        p.T = T;
-        p.ignore_worst = b->cfg.ignore_worst_anchor;
-        p.variant = b->cfg.variant;
-        p.n_ignore = b->cfg.num_ignored_rangings;
-        p.best_mode = b->cfg.best_mode;
-        p.ignore_thr = b->cfg.ignore_cost_threshold;
-        p.accel_noise = b->cfg.accel_noise;
-        p.dt = d_dt;
-        p.dt_f = d_dt_f;
-        p.x = b->d_x;
-        p.P = b->d_P;
-        p.status = b->d_status;
-        p.traj = d_traj;
-        p.sel = d_sel;
-        p.counters = b->d_counters;
-        p.truth = b->d_truth;
-        p.partials = b->d_partials;
-        es_bind(b, p, T);
-        CK(launch_t6_replay(p, s));
-        b->partials_fresh = b->d_truth != nullptr;
-        b->out4_valid = false;
-        return KFPOS_OK;
-    }
-    default: return KFPOS_ERR_UNSUPPORTED;
-    }
+    T6Params p;
+    bind_replay(b, p, make_rs(b, d_ranges, fmt, err_scalar, d_err), d_dt_f, d_traj, T);
+    p.T = T;
+    p.ignore_worst = b->cfg.ignore_worst_anchor;
+    p.variant = b->cfg.variant;
+    p.n_ignore = b->cfg.num_ignored_rangings;
+    p.best_mode = b->cfg.best_mode;
+    p.ignore_thr = b->cfg.ignore_cost_threshold;
+    p.accel_noise = b->cfg.accel_noise;
+    p.dt = d_dt;
+    p.sel = d_sel;
+    CK(launch_t6_replay(p, s));
+    return replayed(b, s);
 }
 
 } // namespace
@@ -694,14 +742,17 @@ int fetch_uninit(kfpos_batch *b, cudaStream_t s) {
     return KFPOS_OK;
 }
 
-// events: HOST array; every data pointer already on the device
-int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_ranges, int fmt, double err_scalar,
-               const double *d_err, const double *d_sensors, double *d_traj, cudaStream_t s, const double *d_dt_f) {
+// events: HOST array, staged through `st`; every data pointer already on the device.  The caller's staging errors
+// are returned before anything is launched.
+int run_events(kfpos_batch *b, Staging &st, int n, const kfpos_event *events, const void *d_ranges, int fmt,
+               double err_scalar, const double *d_err, const double *d_sensors, double *d_traj, cudaStream_t s,
+               const double *d_dt_f) {
     static_assert(sizeof(kfpos_event) == sizeof(EventDesc), "kfpos_event and EventDesc must have one layout");
+    if (st.rc) return st.rc;
     if (n <= 0) return KFPOS_OK;
     b->stepped = true;
-    CK(b->scratch[7].reserve(sizeof(EventDesc) * (size_t)n));
-    CK(cudaMemcpyAsync(b->scratch[7].p, events, sizeof(EventDesc) * (size_t)n, cudaMemcpyHostToDevice, s));
+    const EventDesc *d_events = st.ctl((const EventDesc *)events, sizeof(EventDesc) * (size_t)n);
+    if (st.rc) return st.rc;
     const RangeStream rs = make_rs(b, d_ranges, fmt, err_scalar, d_err);
     poll_uninit(b);
     const bool track_uninit = b->uninit_possible;
@@ -714,45 +765,26 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
     switch (b->model) {
     case KFPOS_MODEL_K8: {
         K8Params p;
-        p.anchors = b->anchors;
+        bind_replay(b, p, rs, d_dt_f, d_traj, n_toa);
         p.cfg = make_k8cfg(b);
-        p.rs = rs;
         p.sensors = d_sensors;
-        p.events = (const EventDesc *)b->scratch[7].p;
+        p.events = d_events;
         p.n_events = n;
-        p.N = b->N;
-        p.x = b->d_x;
-        p.P = b->d_P;
-        p.status = b->d_status;
         p.latch = b->d_latch;
         p.has = b->d_has;
         p.latch_u = b->d_latch_u;
         p.uninit = track_uninit ? b->d_uninit : nullptr;
-        p.dt_f = d_dt_f;
-        p.traj = d_traj;
-        p.counters = b->d_counters;
-        p.truth = b->d_truth;
-        p.partials = b->d_partials;
-        es_bind(b, p, n_toa);
         CK(launch_k8_replay(p, s));
-        CK(cudaMemcpyAsync(b->d_latch_u, b->d_latch_u + 16, sizeof(double) * 16, cudaMemcpyDeviceToDevice, s));
-        b->partials_fresh = b->d_truth != nullptr;
-        b->out4_valid = false;
         break;
     }
     case KFPOS_MODEL_T9: {
         T9Params p;
-        p.anchors = b->anchors;
+        bind_replay(b, p, rs, d_dt_f, d_traj, n_toa);
         p.accel_noise = b->cfg.accel_noise;
         p.jolt = b->cfg.jolt;
-        p.rs = rs;
         p.sensors = d_sensors;
-        p.events = (const EventDesc *)b->scratch[7].p;
+        p.events = d_events;
         p.n_events = n;
-        p.N = b->N;
-        p.x = b->d_x;
-        p.P = b->d_P;
-        p.status = b->d_status;
         p.latch = b->d_latch;
         p.has = b->d_has;
         p.latch_u = b->d_latch_u;
@@ -763,27 +795,14 @@ int run_events(kfpos_batch *b, int n, const kfpos_event *events, const void *d_r
         p.best_mode = b->cfg.best_mode;
         p.ml_init = track_uninit ? 1 : 0;
         p.uninit = track_uninit ? b->d_uninit : nullptr;
-        p.dt_f = d_dt_f;
-        p.traj = d_traj;
-        p.counters = b->d_counters;
-        p.truth = b->d_truth;
-        p.partials = b->d_partials;
-        es_bind(b, p, n_toa);
         CK(launch_t9_replay(p, s));
-        CK(cudaMemcpyAsync(b->d_latch_u, b->d_latch_u + 16, sizeof(double) * 16, cudaMemcpyDeviceToDevice, s));
-        b->partials_fresh = b->d_truth != nullptr;
-        b->out4_valid = false;
         break;
     }
     default: return KFPOS_ERR_INVALID;
     }
-    if (track_uninit) {
-        int rc = fetch_uninit(b, s);
-        if (rc) return rc;
-    }
-    // (the host event array may be a temporary of the caller: a copy from pageable memory has left the
-    // caller's buffer when cudaMemcpyAsync returns, so no synchronisation is needed here)
-    return KFPOS_OK;
+    int rc = replayed(b, s);
+    if (!rc && track_uninit) rc = fetch_uninit(b, s);
+    return rc;
 }
 
 } // namespace
@@ -793,7 +812,7 @@ static int replay_events_impl(kfpos_batch *b, int n_events, const kfpos_event *e
                               const double *sensors, int64_t sensor_rows, double *traj, void *stream) {
     if (!b || (b->model != KFPOS_MODEL_K8 && b->model != KFPOS_MODEL_T9) || n_events < 0 || !events)
         return KFPOS_ERR_INVALID;
-    if (fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
+    if (!fmt_ok(fmt)) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     if (n_events == 0) return KFPOS_OK;
     DeviceGuard g(b->device);
@@ -802,39 +821,26 @@ static int replay_events_impl(kfpos_batch *b, int n_events, const kfpos_event *e
     int64_t range_rows = 0, n_toa = 0;
     for (int e = 0; e < n_events; ++e) {
         const kfpos_event &ev = events[e];
-        if (ev.kind < KFPOS_EV_TOA || ev.kind > KFPOS_EV_COMPASS || ev.offset < 0) return KFPOS_ERR_INVALID;
+        const int rows = event_rows(ev.kind, (int)M);
+        if (rows < 0 || ev.offset < 0) return KFPOS_ERR_INVALID;
         if (b->model == KFPOS_MODEL_T9 && ev.kind != KFPOS_EV_TOA && ev.kind != KFPOS_EV_IMU) return KFPOS_ERR_INVALID;
         if (ev.kind == KFPOS_EV_TOA) {
             if (!ranges) return KFPOS_ERR_INVALID;
-            if (ev.offset + (int64_t)M > range_rows) range_rows = ev.offset + (int64_t)M;
+            if (ev.offset + rows > range_rows) range_rows = ev.offset + rows;
             ++n_toa;
         } else {
-            const int rows = ev.kind == KFPOS_EV_PX4 ? 5 : ev.kind == KFPOS_EV_IMU ? 3 : ev.kind == KFPOS_EV_MAG ? 2 : 1;
             if (!sensors || ev.offset + rows > sensor_rows) return KFPOS_ERR_INVALID;
         }
     }
     if (es_check(b, n_toa)) return KFPOS_ERR_INVALID;
-    const void *d_r = nullptr, *d_e = nullptr, *d_s = nullptr;
-    int rc = stage_in(b, 4, ranges, (size_t)range_rows * N * fmt_size(fmt), s, &d_r);
-    if (rc) return rc;
-    rc = stage_in(b, 5, err_var, sizeof(double) * (size_t)range_rows * N, s, &d_e);
-    if (rc) return rc;
-    rc = stage_in(b, 6, sensors, sizeof(double) * (size_t)sensor_rows * N, s, &d_s);
-    if (rc) return rc;
-    void *d_traj = nullptr;
-    bool copy_traj = false;
-    rc = stage_out(b, 2, traj, sizeof(double) * 3 * N * (size_t)n_toa, &d_traj, &copy_traj);
-    if (rc) return rc;
-    const void *d_dtf = nullptr;
-    if ((rc = stage_in(b, 1, dt_per_filter, sizeof(double) * N * (size_t)n_events, s, &d_dtf))) return rc;
-    rc = run_events(b, n_events, events, d_r, fmt, err_scalar, (const double *)d_e, (const double *)d_s,
-                    (double *)d_traj, s, (const double *)d_dtf);
-    if (rc) return rc;
-    if (copy_traj) {
-        CK(cudaMemcpyAsync(traj, d_traj, sizeof(double) * 3 * N * (size_t)n_toa, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return KFPOS_OK;
+    Staging st(b, s);
+    const void *d_r = st.in(ranges, (size_t)range_rows * N * fmt_size(fmt));
+    const double *d_e = st.in(err_var, sizeof(double) * (size_t)range_rows * N);
+    const double *d_s = st.in(sensors, sizeof(double) * (size_t)sensor_rows * N);
+    double *d_traj = st.out(traj, sizeof(double) * 3 * N * (size_t)n_toa);
+    const double *d_dtf = st.in(dt_per_filter, sizeof(double) * N * (size_t)n_events);
+    int rc = run_events(b, st, n_events, events, d_r, fmt, err_scalar, d_e, d_s, d_traj, s, d_dtf);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int kfpos_batch_replay_events(kfpos_batch *b, int n_events, const kfpos_event *events, const void *ranges,
@@ -855,16 +861,15 @@ extern "C" int kfpos_batch_replay_events_ragged(kfpos_batch *b, int n_events, co
 
 namespace {
 
-// one non-TOA event whose payload rows are gathered into scratch slot 6
-int single_sensor_event(kfpos_batch *b, int kind, double dt, const double *const *rows, int n_rows,
+// one non-TOA event whose payload rows are gathered into one device array
+int single_sensor_event(kfpos_batch *b, Staging &st, int kind, double dt, const double *const *rows, int n_rows,
                         const double aux[9], cudaStream_t s) {
     const size_t N = (size_t)b->N;
-    CK(b->scratch[6].reserve(sizeof(double) * N * (size_t)n_rows));
-    double *dst = (double *)b->scratch[6].p;
+    double *dst = st.buf<double>(sizeof(double) * N * (size_t)n_rows);
+    if (st.rc) return st.rc;
     for (int i = 0; i < n_rows; ++i) {
         if (!rows[i]) return KFPOS_ERR_INVALID;
-        CK(cudaMemcpyAsync(dst + (size_t)i * N, rows[i], sizeof(double) * N,
-                           on_device(rows[i]) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+        st.copy_in(dst + (size_t)i * N, rows[i], sizeof(double) * N);
     }
     kfpos_event ev;
     memset(&ev, 0, sizeof ev);
@@ -872,7 +877,8 @@ int single_sensor_event(kfpos_batch *b, int kind, double dt, const double *const
     ev.dt = dt;
     ev.offset = 0;
     if (aux) memcpy(ev.aux, aux, sizeof ev.aux);
-    return run_events(b, 1, &ev, nullptr, KFPOS_FMT_F64_M, 1.0, nullptr, dst, nullptr, s);
+    int rc = run_events(b, st, 1, &ev, nullptr, KFPOS_FMT_F64_M, 1.0, nullptr, dst, nullptr, s);
+    return rc ? rc : st.finish();
 }
 
 } // namespace
@@ -884,14 +890,13 @@ extern "C" int kfpos_batch_step_px4(kfpos_batch *b, double dt, const double *int
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    const void *d_q = nullptr;
-    int rc = stage_in(b, 5, quality, sizeof(int32_t) * N, s, &d_q);
-    if (rc) return rc;
-    CK(b->scratch[3].reserve(sizeof(double) * N));
-    CK(launch_i32_to_f64(b->N, (const int32_t *)d_q, (double *)b->scratch[3].p, s));
-    const double *rows[5] = {integration_x, integration_y, integration_rot_z, integration_time_us,
-                             (const double *)b->scratch[3].p};
-    return single_sensor_event(b, KFPOS_EV_PX4, dt, rows, 5, nullptr, s);
+    Staging st(b, s);
+    const int32_t *d_q = st.in(quality, sizeof(int32_t) * N);
+    double *d_qf = st.buf<double>(sizeof(double) * N);
+    if (st.rc) return st.rc;
+    CK(launch_i32_to_f64(b->N, d_q, d_qf, s));
+    const double *rows[5] = {integration_x, integration_y, integration_rot_z, integration_time_us, d_qf};
+    return single_sensor_event(b, st, KFPOS_EV_PX4, dt, rows, 5, nullptr, s);
 }
 
 extern "C" int kfpos_batch_step_imu(kfpos_batch *b, double dt, const double *ang_vel, const double *cov_ang_vel,
@@ -900,61 +905,63 @@ extern "C" int kfpos_batch_step_imu(kfpos_batch *b, double dt, const double *ang
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
+    Staging st(b, s);
     double aux[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     if (b->model == KFPOS_MODEL_K8) {
         if (!ang_vel) return KFPOS_ERR_INVALID;
         if (cov_acc) { aux[0] = cov_acc[0]; aux[1] = cov_acc[1]; aux[2] = cov_acc[3]; aux[3] = cov_acc[4]; }
         if (cov_ang_vel) aux[4] = cov_ang_vel[8];
         const double *rows[3] = {ang_vel + 2 * N, lin_acc, lin_acc + N};
-        return single_sensor_event(b, KFPOS_EV_IMU, dt, rows, 3, aux, s);
+        return single_sensor_event(b, st, KFPOS_EV_IMU, dt, rows, 3, aux, s);
     }
     if (cov_acc) memcpy(aux, cov_acc, sizeof aux);
     const double *rows[3] = {lin_acc, lin_acc + N, lin_acc + 2 * N};
-    return single_sensor_event(b, KFPOS_EV_IMU, dt, rows, 3, aux, s);
+    return single_sensor_event(b, st, KFPOS_EV_IMU, dt, rows, 3, aux, s);
 }
 
 extern "C" int kfpos_batch_step_mag(kfpos_batch *b, double dt, const double *mag, void *stream) {
     if (!b || b->model != KFPOS_MODEL_K8 || !mag) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
+    Staging st(b, (cudaStream_t)stream);
     const double *rows[2] = {mag, mag + (size_t)b->N};
-    return single_sensor_event(b, KFPOS_EV_MAG, dt, rows, 2, nullptr, (cudaStream_t)stream);
+    return single_sensor_event(b, st, KFPOS_EV_MAG, dt, rows, 2, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int kfpos_batch_step_compass(kfpos_batch *b, double dt, const double *compass, void *stream) {
     if (!b || b->model != KFPOS_MODEL_K8 || !compass) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
+    Staging st(b, (cudaStream_t)stream);
     const double *rows[1] = {compass};
-    return single_sensor_event(b, KFPOS_EV_COMPASS, dt, rows, 1, nullptr, (cudaStream_t)stream);
+    return single_sensor_event(b, st, KFPOS_EV_COMPASS, dt, rows, 1, nullptr, (cudaStream_t)stream);
 }
 
 // --------------------------------------------------------------------- getPose
+namespace {
+// the model's getPose prediction into the device arrays dx (SoA [n][N]) and dP (SoA [n][n][N])
+int enqueue_get_pose(kfpos_batch *b, double dt, double *dx, double *dP, cudaStream_t s) {
+    switch (b->model) {
+    case KFPOS_MODEL_T6: CK(launch_t6_get_pose(b->N, dt, b->cfg.accel_noise, b->d_x, b->d_P, dx, dP, s)); break;
+    case KFPOS_MODEL_K8:
+        CK(launch_k8_get_pose(b->N, dt, b->cfg.accel_noise, b->cfg.jolt, b->d_x, b->d_P, dx, dP, s));
+        break;
+    case KFPOS_MODEL_T9: CK(launch_t9_get_pose(b->N, dt, b->cfg.jolt, b->d_x, b->d_P, dx, dP, s)); break;
+    default: return KFPOS_ERR_UNSUPPORTED;
+    }
+    return KFPOS_OK;
+}
+} // namespace
+
 extern "C" int kfpos_batch_get_pose(kfpos_batch *b, double dt, double *x_pred, double *P_pred, void *stream) {
     if (!b || b->model == KFPOS_MODEL_ML) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    void *dx = nullptr, *dP = nullptr;
-    bool cx = false, cP = false;
-    int rc = stage_out(b, 2, x_pred, sizeof(double) * b->n * N, &dx, &cx);
-    if (rc) return rc;
-    rc = stage_out(b, 3, P_pred, sizeof(double) * b->n * b->n * N, &dP, &cP);
-    if (rc) return rc;
-    switch (b->model) {
-    case KFPOS_MODEL_T6:
-        CK(launch_t6_get_pose(b->N, dt, b->cfg.accel_noise, b->d_x, b->d_P, (double *)dx, (double *)dP, s));
-        break;
-    case KFPOS_MODEL_K8:
-        CK(launch_k8_get_pose(b->N, dt, b->cfg.accel_noise, b->cfg.jolt, b->d_x, b->d_P, (double *)dx, (double *)dP, s));
-        break;
-    case KFPOS_MODEL_T9:
-        CK(launch_t9_get_pose(b->N, dt, b->cfg.jolt, b->d_x, b->d_P, (double *)dx, (double *)dP, s));
-        break;
-    default: return KFPOS_ERR_UNSUPPORTED;
-    }
-    if (cx) CK(cudaMemcpyAsync(x_pred, dx, sizeof(double) * b->n * N, cudaMemcpyDeviceToHost, s));
-    if (cP) CK(cudaMemcpyAsync(P_pred, dP, sizeof(double) * b->n * b->n * N, cudaMemcpyDeviceToHost, s));
-    if (cx || cP) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    Staging st(b, s);
+    double *dx = st.out(x_pred, sizeof(double) * b->n * N);
+    double *dP = st.out(P_pred, sizeof(double) * b->n * b->n * N);
+    if (st.rc) return st.rc;
+    int rc = enqueue_get_pose(b, dt, dx, dP, s);
+    return rc ? rc : st.finish();
 }
 
 extern "C" int kfpos_batch_get_pose_msg(kfpos_batch *b, double dt, double *pose13, double *cov36, void *stream) {
@@ -963,50 +970,37 @@ extern "C" int kfpos_batch_get_pose_msg(kfpos_batch *b, double dt, double *pose1
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N;
-    CK(b->scratch[2].reserve(sizeof(double) * b->n * N));
-    CK(b->scratch[3].reserve(sizeof(double) * b->n * b->n * N));
-    double *dx = (double *)b->scratch[2].p, *dP = (double *)b->scratch[3].p;
-    int rc = kfpos_batch_get_pose(b, dt, dx, dP, stream);
+    Staging st(b, s);
+    double *dx = st.buf<double>(sizeof(double) * b->n * N);
+    double *dP = st.buf<double>(sizeof(double) * b->n * b->n * N);
+    double *d_pose = st.out(pose13, sizeof(double) * 13 * N);
+    double *d_cov = st.out(cov36, sizeof(double) * 36 * N);
+    if (st.rc) return st.rc;
+    int rc = enqueue_get_pose(b, dt, dx, dP, s);
     if (rc) return rc;
-    void *d_pose = nullptr, *d_cov = nullptr;
-    bool c_pose = false, c_cov = false;
-    if ((rc = stage_out(b, 4, pose13, sizeof(double) * 13 * N, &d_pose, &c_pose))) return rc;
-    if ((rc = stage_out(b, 5, cov36, sizeof(double) * 36 * N, &d_cov, &c_cov))) return rc;
     const int model = b->model == KFPOS_MODEL_T6 ? 1 : (b->model == KFPOS_MODEL_K8 ? 2 : 3);
     // K8 without useFixedHeight: the tag height of an ML-initialised filter is its own (KF.cpp:256-257, 328-332)
     const double *tagz = (b->model == KFPOS_MODEL_K8 && b->cfg.ml_initial_position && !b->cfg.use_fixed_height)
                              ? b->d_latch + 9 * N : nullptr;
-    CK(launch_pose_msg(model, b->N, b->cfg.fixed_height, tagz, dx, dP, (double *)d_pose, (double *)d_cov, s));
-    if (c_pose) CK(cudaMemcpyAsync(pose13, d_pose, sizeof(double) * 13 * N, cudaMemcpyDeviceToHost, s));
-    if (c_cov) CK(cudaMemcpyAsync(cov36, d_cov, sizeof(double) * 36 * N, cudaMemcpyDeviceToHost, s));
-    if (c_pose || c_cov) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    CK(launch_pose_msg(model, b->N, b->cfg.fixed_height, tagz, dx, dP, d_pose, d_cov, s));
+    return st.finish();
 }
 
 // -------------------------------------------------------------------------- ML
 extern "C" int kfpos_batch_ml_solve(kfpos_batch *b, const void *ranges, int fmt, double err_scalar,
                                     const double *err_var, double *pos, double *cov, int32_t *iters,
                                     int32_t *sel, int32_t *status, void *stream) {
-    if (!b || b->model != KFPOS_MODEL_ML || !ranges || fmt < 0 || fmt > 2) return KFPOS_ERR_INVALID;
+    if (!b || b->model != KFPOS_MODEL_ML || !ranges || !fmt_ok(fmt)) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n;
-    const void *d_r = nullptr, *d_e = nullptr;
-    int rc = stage_in(b, 0, ranges, M * N * fmt_size(fmt), s, &d_r);
-    if (rc) return rc;
-    rc = stage_in(b, 1, err_var, sizeof(double) * M * N, s, &d_e);
-    if (rc) return rc;
-    void *d_pos, *d_cov, *d_it, *d_sel, *d_st;
-    bool c_pos, c_cov, c_it, c_sel, c_st;
-    if ((rc = stage_out(b, 2, pos, sizeof(double) * 3 * N, &d_pos, &c_pos))) return rc;
-    if ((rc = stage_out(b, 3, cov, sizeof(double) * 9 * N, &d_cov, &c_cov))) return rc;
-    if ((rc = stage_out(b, 4, iters, sizeof(int32_t) * N, &d_it, &c_it))) return rc;
-    if ((rc = stage_out(b, 5, sel, sizeof(int32_t) * 2 * N, &d_sel, &c_sel))) return rc;
-    if ((rc = stage_out(b, 6, status, sizeof(int32_t) * N, &d_st, &c_st))) return rc;
+    Staging st(b, s);
+    const void *d_r = st.in(ranges, M * N * fmt_size(fmt));
+    const double *d_e = st.in(err_var, sizeof(double) * M * N);
     MlParams p;
     p.anchors = b->anchors;
-    p.rs = make_rs(b, d_r, fmt, err_scalar, (const double *)d_e);
+    p.rs = make_rs(b, d_r, fmt, err_scalar, d_e);
     p.N = b->N;
     p.use2d = b->cfg.use2d;
     p.zero_tz = b->cfg.ml2d_zero_tentative_z != 0;
@@ -1019,11 +1013,11 @@ extern "C" int kfpos_batch_ml_solve(kfpos_batch *b, const void *ranges, int fmt,
     p.start[2] = b->cfg.ml_start[2];
     p.min_z = b->cfg.min_z;
     p.max_z = b->cfg.max_z;
-    p.pos = (double *)d_pos;
-    p.cov = (double *)d_cov;
-    p.iters = (int32_t *)d_it;
-    p.sel = (int32_t *)d_sel;
-    p.status = (int32_t *)d_st;
+    p.pos = st.out(pos, sizeof(double) * 3 * N);
+    p.cov = st.out(cov, sizeof(double) * 9 * N);
+    p.iters = st.out(iters, sizeof(int32_t) * N);
+    p.sel = st.out(sel, sizeof(int32_t) * 2 * N);
+    p.status = st.out(status, sizeof(int32_t) * N);
     p.counters = b->d_counters;
     p.queue[0] = b->d_mlq;
     p.queue[1] = (char *)b->d_mlq + (size_t)b->mlq_cap * 64;
@@ -1041,50 +1035,15 @@ extern "C" int kfpos_batch_ml_solve(kfpos_batch *b, const void *ranges, int fmt,
     p.stream_counter = b->d_mlq_count + 3;
     if (p.variant == 2 && !p.use2d && p.exact_mode >= 0) { // parked subset solves of the 3-D BestGroup scan
         const size_t bytes = ml_exact_scratch_bytes(ml_exact_scratch_epochs(b->N));
-        CK(b->scratch[7].reserve(bytes));
-        p.xw_scratch = b->scratch[7].p;
+        p.xw_scratch = st.buf(bytes);
         p.xw_scratch_bytes = bytes;
     }
+    if (st.rc) return st.rc;
     CK(launch_ml_solve(p, s));
-    if (c_pos) CK(cudaMemcpyAsync(pos, d_pos, sizeof(double) * 3 * N, cudaMemcpyDeviceToHost, s));
-    if (c_cov) CK(cudaMemcpyAsync(cov, d_cov, sizeof(double) * 9 * N, cudaMemcpyDeviceToHost, s));
-    if (c_it) CK(cudaMemcpyAsync(iters, d_it, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, s));
-    if (c_sel) CK(cudaMemcpyAsync(sel, d_sel, sizeof(int32_t) * 2 * N, cudaMemcpyDeviceToHost, s));
-    if (c_st) CK(cudaMemcpyAsync(status, d_st, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, s));
-    if (c_pos || c_cov || c_it || c_sel || c_st || !on_device(ranges)) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 // ------------------------------------------------------------ epoch assembler
-namespace {
-// temporary device copy of a host array (or the device pointer itself)
-struct TmpIn {
-    const void *d = nullptr;
-    void *own = nullptr;
-    cudaError_t set(const void *src, size_t bytes, cudaStream_t s) {
-        if (!src || on_device(src)) { d = src; return cudaSuccess; }
-        cudaError_t e = cudaMalloc(&own, bytes);
-        if (e != cudaSuccess) return e;
-        d = own;
-        return cudaMemcpyAsync(own, src, bytes, cudaMemcpyHostToDevice, s);
-    }
-    ~TmpIn() { if (own) cudaFree(own); }
-};
-struct TmpOut {
-    void *d = nullptr, *own = nullptr, *host = nullptr;
-    size_t bytes = 0;
-    cudaError_t set(void *dst, size_t n) {
-        if (!dst || on_device(dst)) { d = dst; return cudaSuccess; }
-        cudaError_t e = cudaMalloc(&own, n);
-        if (e != cudaSuccess) return e;
-        d = own; host = dst; bytes = n;
-        return cudaSuccess;
-    }
-    cudaError_t back(cudaStream_t s) { return host ? cudaMemcpyAsync(host, own, bytes, cudaMemcpyDeviceToHost, s) : cudaSuccess; }
-    ~TmpOut() { if (own) cudaFree(own); }
-};
-} // namespace
-
 extern "C" int kfpos_assemble_epochs(int device, int64_t n_logs, int64_t n_msgs, int n_anchors, const uint8_t *anchor,
                                      const uint8_t *seq, const int32_t *range_mm, const double *err, const double *t,
                                      int64_t max_epochs, int flags, double first_dt, int32_t *ranges_out,
@@ -1100,27 +1059,20 @@ extern "C" int kfpos_assemble_epochs_t(int device, int64_t n_logs, int64_t n_msg
     if (n_logs <= 0 || n_msgs < 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || max_epochs <= 0)
         return KFPOS_ERR_INVALID;
     if (!anchor || !seq || !range_mm || !t || !ranges_out || !dt_out) return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)n_logs, L = (size_t)n_msgs, M = (size_t)n_anchors, T = (size_t)max_epochs;
-    TmpIn i_a, i_s, i_r, i_e, i_t;
-    TmpOut o_r, o_e, o_dt, o_n, o_t;
-    CK(i_a.set(anchor, L * N, s));
-    CK(i_s.set(seq, L * N, s));
-    CK(i_r.set(range_mm, 4 * L * N, s));
-    CK(i_e.set(err, 8 * L * N, s));
-    CK(i_t.set(t, 8 * L * N, s));
-    CK(o_r.set(ranges_out, 4 * T * M * N));
-    CK(o_e.set(err_out, 8 * T * M * N));
-    CK(o_dt.set(dt_out, 8 * T * N));
-    CK(o_n.set(n_epochs, 4 * N));
-    CK(o_t.set(t_out, 8 * T * N));
+    Staging st(s);
+    AssembleParams p;
+    p.anchor = st.in(anchor, L * N); p.seq = st.in(seq, L * N);
+    p.range_mm = st.in(range_mm, 4 * L * N); p.err = st.in(err, 8 * L * N); p.t = st.in(t, 8 * L * N);
+    p.ranges_out = st.out(ranges_out, 4 * T * M * N); p.err_out = st.out(err_out, 8 * T * M * N);
+    p.dt_out = st.out(dt_out, 8 * T * N);
+    p.n_epochs = st.out(n_epochs, 4 * N);
+    p.t_out = st.out(t_out, 8 * T * N);
+    if (st.rc) return st.rc;
     const int fix = (flags & KFPOS_ASM_FIX_ROW_CLEAR) ? 1 : 0;
     const size_t rows = fix ? 1 : 256;
     // the sequence-number table: per-device scratch that is kept between calls (grown on demand)
@@ -1132,28 +1084,14 @@ extern "C" int kfpos_assemble_epochs_t(int device, int64_t n_logs, int64_t n_msg
     CK(te.reserve(8 * rows * M * N));
     CK(cudaMemsetAsync(tr.p, 0xff, 4 * rows * M * N, s)); // initialiseTagList: -1
     CK(cudaMemsetAsync(te.p, 0, 8 * rows * M * N, s));
-    AssembleParams p;
     p.N = n_logs; p.L = n_msgs; p.max_epochs = max_epochs;
     p.M = n_anchors; p.fix_b12 = fix; p.first_dt = first_dt;
-    p.anchor = (const uint8_t *)i_a.d; p.seq = (const uint8_t *)i_s.d;
-    p.range_mm = (const int32_t *)i_r.d; p.err = (const double *)i_e.d; p.t = (const double *)i_t.d;
     p.tbl_r = (int32_t *)tr.p; p.tbl_e = (double *)te.p;
-    p.ranges_out = (int32_t *)o_r.d; p.err_out = (double *)o_e.d; p.dt_out = (double *)o_dt.d;
-    p.n_epochs = (int32_t *)o_n.d;
-    p.t_out = (double *)o_t.d;
     CK(launch_assemble(p, s));
-    CK(o_t.back(s));
-    CK(o_r.back(s));
-    CK(o_e.back(s));
-    CK(o_dt.back(s));
-    CK(o_n.back(s));
-    // temporary copies of host arrays are freed on return: finish the work first.  With device
-    // pointers only, the call is asynchronous on `stream` like the rest of the API (the table
+    // With device pointers only, the call is asynchronous on `stream` like the rest of the API (the table
     // is reused by the next call on the same device, which is ordered behind this one only if it
     // uses the same stream: callers on different streams must synchronise themselves).
-    if (i_a.own || i_s.own || i_r.own || i_e.own || i_t.own || o_r.own || o_e.own || o_dt.own || o_n.own || o_t.own)
-        CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 extern "C" int kfpos_merge_streams(int device, int64_t n_logs, int n_anchors, int64_t n_epochs, const double *t_epoch,
@@ -1165,19 +1103,15 @@ extern "C" int kfpos_merge_streams(int device, int64_t n_logs, int n_anchors, in
     if (n_logs <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || n_epochs < 0 || n_slots <= 0 || !slot_kind ||
         !dt_out)
         return KFPOS_ERR_INVALID;
-    static const int rows_of[5] = {0, 5, 3, 2, 1};
     int64_t range_rows = 0, sensor_rows = 0;
     std::vector<int64_t> slot_row((size_t)n_slots);
     for (int sidx = 0; sidx < n_slots; ++sidx) {
         const int k = slot_kind[sidx];
-        if (k < KFPOS_EV_TOA || k > KFPOS_EV_COMPASS) return KFPOS_ERR_INVALID;
-        if (k == KFPOS_EV_TOA) {
-            slot_row[sidx] = range_rows;
-            range_rows += n_anchors;
-        } else {
-            slot_row[sidx] = sensor_rows;
-            sensor_rows += rows_of[k];
-        }
+        const int rows = event_rows(k, n_anchors);
+        if (rows < 0) return KFPOS_ERR_INVALID;
+        int64_t &used = k == KFPOS_EV_TOA ? range_rows : sensor_rows;
+        slot_row[sidx] = used;
+        used += rows;
         if (events_out) {
             memset(&events_out[sidx], 0, sizeof(kfpos_event));
             events_out[sidx].kind = k;
@@ -1188,68 +1122,42 @@ extern "C" int kfpos_merge_streams(int device, int64_t n_logs, int n_anchors, in
     }
     if ((range_rows > 0 && (!ranges_out || (n_epochs > 0 && (!t_epoch || !ranges)))) || (sensor_rows > 0 && !sensors_out))
         return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)n_logs, M = (size_t)n_anchors;
+    const size_t range_n = (size_t)(range_rows > 0 ? range_rows : 1) * N;
+    const size_t sensor_n = (size_t)(sensor_rows > 0 ? sensor_rows : 1) * N;
+    Staging st(s); // the slot tables are always staged, so the call always synchronises
     MergeParams p;
     memset(&p, 0, sizeof p);
     p.N = n_logs; p.M = n_anchors; p.n_slots = n_slots; p.first_dt = first_dt;
-    TmpIn i_t[5], i_p[5], i_e, i_k, i_row;
-    TmpOut o_dt, o_r, o_e, o_s, o_n;
     p.L[0] = n_epochs;
-    CK(i_t[0].set(t_epoch, 8 * (size_t)n_epochs * N, s));
-    CK(i_p[0].set(ranges, 4 * (size_t)n_epochs * M * N, s));
-    CK(i_e.set(err, 8 * (size_t)n_epochs * M * N, s));
-    p.t_src[0] = (const double *)i_t[0].d; p.ranges = (const int32_t *)i_p[0].d; p.err_src = (const double *)i_e.d;
+    p.t_src[0] = st.in(t_epoch, 8 * (size_t)n_epochs * N);
+    p.ranges = st.in(ranges, 4 * (size_t)n_epochs * M * N);
+    p.err_src = st.in(err, 8 * (size_t)n_epochs * M * N);
     for (int k = 1; k < 5; ++k) {
         const int64_t Lk = n_samples ? n_samples[k - 1] : 0;
         if (Lk <= 0 || !t_sensor || !payload || !t_sensor[k - 1] || !payload[k - 1]) continue;
         p.L[k] = Lk;
-        CK(i_t[k].set(t_sensor[k - 1], 8 * (size_t)Lk * N, s));
-        CK(i_p[k].set(payload[k - 1], 8 * (size_t)Lk * rows_of[k] * N, s));
-        p.t_src[k] = (const double *)i_t[k].d; p.src[k] = (const double *)i_p[k].d;
+        p.t_src[k] = st.in(t_sensor[k - 1], 8 * (size_t)Lk * N);
+        p.src[k] = st.in(payload[k - 1], 8 * (size_t)Lk * event_rows(k, n_anchors) * N);
     }
-    CK(i_k.set(nullptr, 0, s)); // (slot tables are small host arrays: always copied)
-    int32_t *d_kind = nullptr;
-    int64_t *d_row = nullptr;
-    CK(cudaMalloc((void **)&d_kind, sizeof(int32_t) * (size_t)n_slots));
-    cudaError_t e2 = cudaMalloc((void **)&d_row, sizeof(int64_t) * (size_t)n_slots);
-    if (e2 != cudaSuccess) { cudaFree(d_kind); return map_cuda_err(e2); }
-    auto cleanup = [&]() { cudaFree(d_kind); cudaFree(d_row); };
-    auto fail = [&](cudaError_t e) { cudaStreamSynchronize(s); cleanup(); return map_cuda_err(e); };
-    cudaError_t e = cudaMemcpyAsync(d_kind, slot_kind, sizeof(int32_t) * (size_t)n_slots, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_row, slot_row.data(), sizeof(int64_t) * (size_t)n_slots, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess) e = o_dt.set(dt_out, 8 * (size_t)n_slots * N);
-    if (e == cudaSuccess) e = o_r.set(ranges_out, 4 * (size_t)(range_rows > 0 ? range_rows : 1) * N);
-    if (e == cudaSuccess) e = o_e.set(err_out, 8 * (size_t)(range_rows > 0 ? range_rows : 1) * N);
-    if (e == cudaSuccess) e = o_s.set(sensors_out, 8 * (size_t)(sensor_rows > 0 ? sensor_rows : 1) * N);
-    if (e == cudaSuccess) e = o_n.set(n_dropped, 4 * N);
-    if (e != cudaSuccess) return fail(e);
+    p.slot_kind = st.ctl(slot_kind, sizeof(int32_t) * (size_t)n_slots);
+    p.slot_row = st.ctl(slot_row.data(), sizeof(int64_t) * (size_t)n_slots);
+    p.dt_f = st.out(dt_out, 8 * (size_t)n_slots * N);
+    p.ranges_out = st.out(ranges_out, 4 * range_n);
+    p.err_out = st.out(err_out, 8 * range_n);
+    p.sensors_out = st.out(sensors_out, 8 * sensor_n);
+    p.n_dropped = st.out(n_dropped, 4 * N);
+    if (st.rc) return st.rc;
     // slots nobody takes keep "no ranging" / zero payloads
-    if (o_r.d) e = cudaMemsetAsync(o_r.d, 0xff, 4 * (size_t)(range_rows > 0 ? range_rows : 1) * N, s);
-    if (e == cudaSuccess && o_e.d) e = cudaMemsetAsync(o_e.d, 0, 8 * (size_t)(range_rows > 0 ? range_rows : 1) * N, s);
-    if (e == cudaSuccess && o_s.d) e = cudaMemsetAsync(o_s.d, 0, 8 * (size_t)(sensor_rows > 0 ? sensor_rows : 1) * N, s);
-    if (e != cudaSuccess) return fail(e);
-    p.slot_kind = d_kind; p.slot_row = d_row;
-    p.dt_f = (double *)o_dt.d; p.ranges_out = (int32_t *)o_r.d; p.err_out = (double *)o_e.d;
-    p.sensors_out = (double *)o_s.d; p.n_dropped = (int32_t *)o_n.d;
-    e = launch_merge(p, s);
-    if (e == cudaSuccess) e = o_dt.back(s);
-    if (e == cudaSuccess) e = o_r.back(s);
-    if (e == cudaSuccess) e = o_e.back(s);
-    if (e == cudaSuccess) e = o_s.back(s);
-    if (e == cudaSuccess) e = o_n.back(s);
-    if (e != cudaSuccess) return fail(e);
-    // the slot tables (and any staged host arrays) are freed on return: finish the work first
-    e = cudaStreamSynchronize(s);
-    cleanup();
-    return e == cudaSuccess ? KFPOS_OK : map_cuda_err(e);
+    if (p.ranges_out) CK(cudaMemsetAsync(p.ranges_out, 0xff, 4 * range_n, s));
+    if (p.err_out) CK(cudaMemsetAsync(p.err_out, 0, 8 * range_n, s));
+    if (p.sensors_out) CK(cudaMemsetAsync(p.sensors_out, 0, 8 * sensor_n, s));
+    CK(launch_merge(p, s));
+    return st.finish();
 }
 
 // ----------------------------------------------------------------- diagnostics
@@ -1290,18 +1198,18 @@ extern "C" int kfpos_batch_set_truth(kfpos_batch *b, const double *truth, void *
 namespace {
 // leaves [sum |e|^2, sum |e_xy|^2, n, n_bad] of this batch in d_out4.  truth == null: the partials the last
 // replay launch left behind (kfpos_batch_set_truth) are folded; otherwise they are computed first.
-int enqueue_error_stats(kfpos_batch *b, const double *truth, cudaStream_t s) {
-    const void *d_truth = nullptr;
+int enqueue_error_stats(kfpos_batch *b, Staging &st, const double *truth, cudaStream_t s) {
+    const double *d_truth = nullptr;
     if (truth) {
-        int rc = stage_in(b, 0, truth, sizeof(double) * 3 * (size_t)b->N, s, &d_truth);
-        if (rc) return rc;
+        d_truth = st.in(truth, sizeof(double) * 3 * (size_t)b->N);
+        if (st.rc) return st.rc;
     } else if (!b->partials_fresh) {
         if (!b->d_truth) return KFPOS_ERR_NOT_READY;
         d_truth = b->d_truth; // registered, but the state changed since the last replay (single steps, set_state)
     }
     // K8 is planar: z is the configured tag height (KF.cpp:328-332)
     CK(launch_error_stats(b->N, b->d_x, b->model == KFPOS_MODEL_K8 ? -1 : 2, b->cfg.fixed_height, b->d_status,
-                          (const double *)d_truth, b->d_partials, b->d_out4, s));
+                          d_truth, b->d_partials, b->d_out4, s));
     b->partials_fresh = false; // the tree folds the partials in place
     b->out4_valid = true;
     return KFPOS_OK;
@@ -1330,19 +1238,27 @@ NcclApi &nccl_api() {
     }
     return api;
 }
+
+// ONE collective: the `count` doubles at `send` of every rank to every rank, [rank][count] in `recv` (grown to
+// fit); the number of ranks comes back in `n_ranks`
+int all_gather(struct ncclComm *comm, const double *send, size_t count, DevBuf &recv, int *n_ranks, cudaStream_t s) {
+    NcclApi &api = nccl_api();
+    if (!api.all_gather || !api.count) return KFPOS_ERR_UNSUPPORTED;
+    if (api.count(comm, n_ranks) != 0 || *n_ranks < 1 || *n_ranks > 1024) return KFPOS_ERR_INVALID;
+    CK(recv.reserve(sizeof(double) * count * (size_t)*n_ranks));
+    return api.all_gather(send, recv.p, count, 8 /* ncclDouble */, comm, s) != 0 ? KFPOS_ERR_CUDA : KFPOS_OK;
+}
 } // namespace
 
 extern "C" int kfpos_batch_error_stats(kfpos_batch *b, const double *truth, double out[4], void *stream) {
     if (!b || b->model == KFPOS_MODEL_ML) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
-    int rc = enqueue_error_stats(b, truth, s);
+    Staging st(b, s);
+    int rc = enqueue_error_stats(b, st, truth, s);
     if (rc) return rc;
-    if (out) { // out == null: enqueue only, the result stays on the device (kfpos_stats_allreduce reads it)
-        CK(cudaMemcpyAsync(out, b->d_out4, sizeof(double) * 4, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return KFPOS_OK;
+    st.copy_out(out, b->d_out4, sizeof(double) * 4); // out == null: the result stays on the device (allreduce)
+    return st.finish();
 }
 
 extern "C" int kfpos_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, const double *truth, double out[6],
@@ -1350,25 +1266,22 @@ extern "C" int kfpos_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, cons
     if (!b || b->model == KFPOS_MODEL_ML || !out) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
+    Staging st(b, s);
+    int rc;
     // truth == null: what the last kfpos_batch_error_stats left on the device, if the state has not changed since
-    if (truth || !b->out4_valid) {
-        int rc = enqueue_error_stats(b, truth, s);
-        if (rc) return rc;
-    }
+    if ((truth || !b->out4_valid) && (rc = enqueue_error_stats(b, st, truth, s))) return rc;
     const double *d_res = b->d_out4;
     if (comm) {
-        NcclApi &api = nccl_api();
-        if (!api.all_gather || !api.count) return KFPOS_ERR_UNSUPPORTED;
+        // every rank's 4 doubles to every rank, then the same pairwise tree over the rank index on every rank --
+        // the top levels of the global tree, in a fixed order
         int n_ranks = 0;
-        if (api.count(comm, &n_ranks) != 0 || n_ranks < 1 || n_ranks > 1024) return KFPOS_ERR_INVALID;
-        // ONE collective: every rank's 4 doubles to every rank (ncclDouble = 8), then the same pairwise
-        // tree over the rank index on every rank -- the top levels of the global tree, in a fixed order
-        if (api.all_gather(b->d_out4, b->d_gather, 4, 8, comm, s) != 0) return KFPOS_ERR_CUDA;
-        CK(launch_error_stats_tree(n_ranks, b->d_gather, b->d_gather, s));
-        d_res = b->d_gather;
+        if ((rc = all_gather(comm, b->d_out4, 4, b->gather, &n_ranks, s))) return rc;
+        double *gat = (double *)b->gather.p;
+        CK(launch_error_stats_tree(n_ranks, gat, gat, s));
+        d_res = gat;
     }
-    CK(cudaMemcpyAsync(out, d_res, sizeof(double) * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    st.copy_out(out, d_res, sizeof(double) * 4);
+    if ((rc = st.finish())) return rc;
     const double n = out[2] > 1.0 ? out[2] : 1.0;
     out[4] = sqrt(out[0] / n);
     out[5] = sqrt(out[1] / n);
@@ -1443,13 +1356,11 @@ extern "C" int kfpos_batch_epoch_stats(kfpos_batch *b, int64_t n_rows, double *o
     if (rc) return rc;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
-    const bool dev = on_device(out);
-    if ((rc = enqueue_epoch_stats(b, dev ? out : b->d_eout, s))) return rc;
-    if (!dev) {
-        CK(cudaMemcpyAsync(out, b->d_eout, sizeof(double) * ES_W * (size_t)n_rows, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return KFPOS_OK;
+    Staging st(b, s);
+    double *d_out = st.out(out, sizeof(double) * ES_W * (size_t)n_rows);
+    if (st.rc) return st.rc;
+    if ((rc = enqueue_epoch_stats(b, d_out, s))) return rc;
+    return st.finish();
 }
 
 extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, double *out,
@@ -1460,33 +1371,23 @@ extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm
     cudaStream_t s = (cudaStream_t)stream;
     if ((rc = enqueue_epoch_stats(b, b->d_eout, s))) return rc;
     const double *d_res = b->d_eout;
-    const size_t bytes = sizeof(double) * ES_W * (size_t)n_rows;
     if (comm) {
-        NcclApi &api = nccl_api();
-        if (!api.all_gather || !api.count) return KFPOS_ERR_UNSUPPORTED;
+        // every rank's [n_rows][6] to every rank ([rank][row][6]), then per row the pairwise tree over the rank
+        // index -- the top levels of the global tree; row r's result lands on its rank-0 entry
         int n_ranks = 0;
-        if (api.count(comm, &n_ranks) != 0 || n_ranks < 1 || n_ranks > 1024) return KFPOS_ERR_INVALID;
-        CK(b->es_gather.reserve(bytes * (size_t)n_ranks));
+        if ((rc = all_gather(comm, b->d_eout, (size_t)n_rows * ES_W, b->es_gather, &n_ranks, s))) return rc;
         double *gat = (double *)b->es_gather.p;
-        // ONE collective: every rank's [n_rows][6] to every rank ([rank][row][6]), then per row the pairwise tree
-        // over the rank index -- the top levels of the global tree; row r's result lands on its rank-0 entry
-        if (api.all_gather(b->d_eout, gat, (size_t)n_rows * ES_W, 8, comm, s) != 0) return KFPOS_ERR_CUDA;
         CK(launch_stats_tree(ES_W, n_rows, n_ranks, gat, gat, ES_W, n_rows * ES_W, gat, s));
         d_res = gat;
     }
-    const bool dev = on_device(out);
-    CK(cudaMemcpyAsync(out, d_res, bytes, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
-    if (!dev) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    Staging st(b, s);
+    st.copy_out(out, d_res, sizeof(double) * ES_W * (size_t)n_rows);
+    return st.finish();
 }
 
 extern "C" int kfpos_measure_fp64_peak(int device, double *flops_per_s) {
     if (!flops_per_s) return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     CK(measure_fp64_peak(flops_per_s));
@@ -1501,29 +1402,27 @@ extern "C" int kfpos_synth_k8(int device, int64_t n_filters, int64_t first_filte
     if (n_filters <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || !anchors_xyz || n_events < 0 ||
         (n_events > 0 && !events) || range_rows < 0 || sensor_rows < 0)
         return KFPOS_ERR_INVALID;
-    for (int i = 0; i < n_events; ++i) { // every event must write inside the tensors it was given
-        const int rows = events[i].kind == KFPOS_EV_TOA ? n_anchors
-                         : events[i].kind == KFPOS_EV_PX4 ? 5 : events[i].kind == KFPOS_EV_IMU ? 3
-                         : events[i].kind == KFPOS_EV_COMPASS ? 1 : -1;
+    for (int i = 0; i < n_events; ++i) { // every event must write inside the tensors it was given (no MAG samples)
+        const int rows = events[i].kind == KFPOS_EV_MAG ? -1 : event_rows(events[i].kind, n_anchors);
         const int64_t lim = events[i].kind == KFPOS_EV_TOA ? range_rows : sensor_rows;
         if (rows < 0 || events[i].offset < 0 || events[i].offset + rows > lim) return KFPOS_ERR_INVALID;
         if ((events[i].kind == KFPOS_EV_TOA && !ranges) || (events[i].kind != KFPOS_EV_TOA && !sensors))
             return KFPOS_ERR_INVALID;
     }
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t N = (size_t)n_filters;
-    TmpOut o_r, o_s, o_x, o_t;
-    CK(o_r.set(ranges, 4 * (size_t)range_rows * N));
-    CK(o_s.set(sensors, 8 * (size_t)sensor_rows * N));
-    CK(o_x.set(x0, 8 * 8 * N));
-    CK(o_t.set(truth_end, 8 * 3 * N));
+    SynthK8Params p;
+    int rc = anchor_table(n_anchors, anchors_xyz, &p.anchors);
+    if (rc) return rc;
+    Staging st(s);
+    p.ranges = st.out(ranges, 4 * (size_t)range_rows * N);
+    p.sensors = st.out(sensors, 8 * (size_t)sensor_rows * N);
+    p.x0 = st.out(x0, 8 * 8 * N);
+    p.truth_end = st.out(truth_end, 8 * 3 * N);
+    if (st.rc) return st.rc;
     // the schedule goes through a small per-device ring of scratch buffers (a pageable source has left the caller's
     // array when cudaMemcpyAsync returns): with device outputs the call is then asynchronous on `stream`, so that a
     // caller can generate chunk c + 1 on one stream while chunk c is replayed on another
@@ -1535,59 +1434,35 @@ extern "C" int kfpos_synth_k8(int device, int64_t n_filters, int64_t first_filte
         std::lock_guard<std::mutex> lock(mtx);
         DevBuf &slot = ring[device & 63][next[device & 63]++ & 7];
         if (slot.cap < sizeof(SynthEvent) * (size_t)n_events) {
-            CK(cudaStreamSynchronize(s)); // growing a slot frees the old one: nothing may still read it
-            CK(cudaDeviceSynchronize());
+            CK(cudaDeviceSynchronize()); // growing a slot frees the old one: nothing may still read it
             CK(slot.reserve(sizeof(SynthEvent) * (size_t)(n_events < 256 ? 256 : n_events)));
         }
         d_ev = slot.p;
         CK(cudaMemcpyAsync(d_ev, events, sizeof(SynthEvent) * (size_t)n_events, cudaMemcpyHostToDevice, s));
     }
-    SynthK8Params p;
-    memset(&p.anchors, 0, sizeof p.anchors);
-    p.anchors.n = n_anchors;
-    for (int i = 0; i < n_anchors; ++i) {
-        p.anchors.x[i] = anchors_xyz[3 * i]; p.anchors.y[i] = anchors_xyz[3 * i + 1]; p.anchors.z[i] = anchors_xyz[3 * i + 2];
-    }
     p.N = n_filters; p.filter0 = first_filter; p.seed = seed; p.M = n_anchors; p.n_events = n_events;
     p.tag_z = tag_z; p.sigma_r = sigma_r; p.t_end = t_end;
     p.events = (const SynthEvent *)d_ev;
-    p.ranges = (int32_t *)o_r.d; p.sensors = (double *)o_s.d; p.x0 = (double *)o_x.d; p.truth_end = (double *)o_t.d;
-    cudaError_t e = launch_synth_k8(p, s);
-    if (e == cudaSuccess) e = o_r.back(s);
-    if (e == cudaSuccess) e = o_s.back(s);
-    if (e == cudaSuccess) e = o_x.back(s);
-    if (e == cudaSuccess) e = o_t.back(s);
-    if (e != cudaSuccess) return map_cuda_err(e);
-    // host staging is freed on return: finish the work first; device outputs: asynchronous on `stream`
-    if (o_r.own || o_s.own || o_x.own || o_t.own) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    CK(launch_synth_k8(p, s));
+    return st.finish();
 }
 
 extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first_filter, uint64_t seed, int n_times,
                                     const double *t, double tag_z, double *truth, void *stream) {
     if (n_filters <= 0 || n_times < 0 || (n_times > 0 && (!t || !truth))) return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     if (n_times == 0) return KFPOS_OK;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
-    TmpIn i_t;
-    TmpOut o_t;
-    CK(i_t.set(t, sizeof(double) * (size_t)n_times, s));
-    CK(o_t.set(truth, sizeof(double) * 3 * (size_t)n_filters * (size_t)n_times));
+    Staging st(s);
     SynthTruthParams p;
     p.N = n_filters; p.filter0 = first_filter; p.seed = seed; p.n_times = n_times; p.tag_z = tag_z;
-    p.t = (const double *)i_t.d;
-    p.truth = (double *)o_t.d;
+    p.t = st.in(t, sizeof(double) * (size_t)n_times);
+    p.truth = st.out(truth, sizeof(double) * 3 * (size_t)n_filters * (size_t)n_times);
+    if (st.rc) return st.rc;
     CK(launch_synth_k8_truth(p, s));
-    CK(o_t.back(s));
-    // staging is freed on return: finish the work first; device arrays only: asynchronous on `stream`
-    if (i_t.own || o_t.own) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
@@ -1601,25 +1476,20 @@ extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_ancho
         (gen->p_nlos > 0.0 && !(gen->nlos_mean > 0.0)) || gen->first_filter < 0 || gen->first_epoch < 0 ||
         gen->first_epoch + n_epochs > (int64_t)0xFFFFFFFF) // epoch index 0xFFFFFFFF: the per-filter constants
         return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     if (n_epochs == 0) return KFPOS_OK;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t row = fmt_size(fmt) * (size_t)n_anchors * (size_t)n_filters; // bytes of one epoch
-    TmpOut o_r;
-    CK(o_r.set(ranges, row * (size_t)n_epochs));
     // the epoch times travel in the parameter block, SYNTH_TOA_T per launch: nothing to stage, so a device
     // `ranges` leaves the call asynchronous (the next chunk can be generated while this one is replayed)
     SynthToaParams p{};
-    p.anchors.n = n_anchors;
-    for (int i = 0; i < n_anchors; ++i) {
-        p.anchors.x[i] = anchors_xyz[3 * i]; p.anchors.y[i] = anchors_xyz[3 * i + 1]; p.anchors.z[i] = anchors_xyz[3 * i + 2];
-    }
+    int rc = anchor_table(n_anchors, anchors_xyz, &p.anchors);
+    if (rc) return rc;
+    Staging st(s);
+    char *d_r = st.out((char *)ranges, row * (size_t)n_epochs);
+    if (st.rc) return st.rc;
     p.N = n_filters; p.filter0 = gen->first_filter; p.seed = gen->seed; p.M = n_anchors;
     p.tag_z = gen->tag_z; p.sigma_r = gen->sigma_r; p.p_missing = gen->p_missing; p.p_nlos = gen->p_nlos;
     p.nlos_mean = gen->nlos_mean;
@@ -1627,58 +1497,43 @@ extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_ancho
         p.n_epochs = n_epochs - k0 < SYNTH_TOA_T ? n_epochs - k0 : SYNTH_TOA_T;
         p.epoch0 = (uint32_t)(gen->first_epoch + k0);
         memcpy(p.t, t + k0, sizeof(double) * (size_t)p.n_epochs);
-        p.ranges = (char *)o_r.d + row * (size_t)k0;
+        p.ranges = d_r + row * (size_t)k0;
         CK(launch_synth_toa(p, fmt == KFPOS_FMT_U16_MM, s));
     }
-    CK(o_r.back(s));
-    // host staging is freed on return: finish the work first; device output: asynchronous on `stream`
-    if (o_r.own) CK(cudaStreamSynchronize(s));
-    return KFPOS_OK;
+    return st.finish();
 }
 
 extern "C" int kfpos_selftest_math(int device, int64_t n, const double *x, double *rcp, double *rsqrt, double *sn,
                                    double *cs) {
     if (n <= 0 || !x) return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
-    TmpIn i_x;
-    TmpOut o[4];
-    double *outs[4] = {rcp, rsqrt, sn, cs};
-    CK(i_x.set(x, 8 * (size_t)n, nullptr));
-    for (int k = 0; k < 4; ++k) CK(o[k].set(outs[k], 8 * (size_t)n));
-    CK(launch_selftest_math(n, (const double *)i_x.d, (double *)o[0].d, (double *)o[1].d, (double *)o[2].d,
-                            (double *)o[3].d, nullptr));
-    for (int k = 0; k < 4; ++k) CK(o[k].back(nullptr));
-    CK(cudaStreamSynchronize(nullptr));
-    return KFPOS_OK;
+    Staging st(nullptr);
+    st.sync = true; // a self-test returns the errors of its kernel, whatever the arrays
+    const size_t bytes = 8 * (size_t)n;
+    const double *d_x = st.in(x, bytes);
+    double *d_rcp = st.out(rcp, bytes), *d_rsqrt = st.out(rsqrt, bytes), *d_sn = st.out(sn, bytes);
+    double *d_cs = st.out(cs, bytes);
+    if (st.rc) return st.rc;
+    CK(launch_selftest_math(n, d_x, d_rcp, d_rsqrt, d_sn, d_cs, nullptr));
+    return st.finish();
 }
 
 extern "C" int kfpos_selftest_ieee(int device, int64_t n, const double *a, const double *b, double *div_fast,
                                    double *div_ieee, double *sqrt_fast, double *sqrt_ieee, int32_t *flags) {
     if (n <= 0 || !a || !b) return KFPOS_ERR_INVALID;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {
-        cudaGetLastError();
-        return KFPOS_ERR_CUDA;
-    }
+    if (int rc = check_device(device)) return rc;
     DeviceGuard g(device);
     if (!g.ok) return KFPOS_ERR_CUDA;
-    TmpIn i_a, i_b;
-    TmpOut o[4], o_f;
-    double *outs[4] = {div_fast, div_ieee, sqrt_fast, sqrt_ieee};
-    CK(i_a.set(a, 8 * (size_t)n, nullptr));
-    CK(i_b.set(b, 8 * (size_t)n, nullptr));
-    for (int k = 0; k < 4; ++k) CK(o[k].set(outs[k], 8 * (size_t)n));
-    CK(o_f.set(flags, 4 * (size_t)n));
-    CK(launch_selftest_ieee(n, (const double *)i_a.d, (const double *)i_b.d, (double *)o[0].d, (double *)o[1].d,
-                            (double *)o[2].d, (double *)o[3].d, (int32_t *)o_f.d, nullptr));
-    for (int k = 0; k < 4; ++k) CK(o[k].back(nullptr));
-    CK(o_f.back(nullptr));
-    CK(cudaStreamSynchronize(nullptr));
-    return KFPOS_OK;
+    Staging st(nullptr);
+    st.sync = true; // a self-test returns the errors of its kernel, whatever the arrays
+    const size_t bytes = 8 * (size_t)n;
+    const double *d_a = st.in(a, bytes), *d_b = st.in(b, bytes);
+    double *d_df = st.out(div_fast, bytes), *d_di = st.out(div_ieee, bytes);
+    double *d_sf = st.out(sqrt_fast, bytes), *d_si = st.out(sqrt_ieee, bytes);
+    int32_t *d_flags = st.out(flags, 4 * (size_t)n);
+    if (st.rc) return st.rc;
+    CK(launch_selftest_ieee(n, d_a, d_b, d_df, d_di, d_sf, d_si, d_flags, nullptr));
+    return st.finish();
 }
