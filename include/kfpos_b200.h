@@ -466,6 +466,39 @@ int kfpos_batch_epoch_stats(kfpos_batch *b, int64_t n_rows, double *out, void *s
  * (comm == NULL: this batch alone).                                                                    */
 int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, double *out, void *stream);
 
+/* Per-epoch error histograms for Monte Carlo runs (no reference equivalent; the distributions behind the
+ * means of kfpos_batch_epoch_stats: error percentiles such as CEP50 / CEP95 over time, and the fraction of
+ * NEES values inside chi-square bounds).  Registers a histogram of one quantity per output row:
+ *   KFPOS_HIST_ERR     |p - truth| in m           (the value behind epoch_stats column [0])
+ *   KFPOS_HIST_ERR_XY  x-y error in m             (column [1])
+ *   KFPOS_HIST_NEES    NEES, dimensionless        (column [4])
+ * `edges` is a HOST array of 1..255 finite, strictly increasing values (m and >= 0 for the two error
+ * quantities).  Bin k of a value v holds the values with exactly k edges <= v: bin 0 is below edges[0], bin
+ * n_edges is at or above the last edge.  The error quantities are binned as e^2 against the squared edges
+ * (each squared once here, an IEEE multiply), so a host reproduces every bin exactly from the trajectory,
+ * e.g. numpy.searchsorted(edges * edges, e2, side="right").  A filter counts where it counts in epoch_stats
+ * ([2] for the errors, [5] for NEES), so each row's total equals that column.  n_edges == 0 or edges == NULL
+ * unregisters.  The histogram is a batch attribute: it stays registered across kfpos_batch_set_truth_traj,
+ * and it is filled only while a truth trajectory is registered.  Storage [rows][n_edges + 1] uint64 on the
+ * device is (re)allocated and zeroed by whichever of the two registrations comes last, and by every later
+ * truth registration.  Each replay launch overwrites the rows it fills (a re-run after set_state replaces
+ * them).  KFPOS_ERR_INVALID: ML batch, bad quantity, bad edge table.  KFPOS_ERR_NOMEM: no storage.       */
+#define KFPOS_HIST_ERR 0    /* |p - truth|   (the value of epoch_stats column [0]) */
+#define KFPOS_HIST_ERR_XY 1 /* x-y error     (column [1])                          */
+#define KFPOS_HIST_NEES 2   /* NEES          (column [4])                          */
+int kfpos_batch_set_error_hist(kfpos_batch *b, int quantity, int n_edges, const double *edges);
+
+/* counts [n_rows][n_edges + 1] uint64 (host or device; n_rows must equal the registered truth rows), the
+ * number of filters per bin at each output row.  Rows the cursor has not reached are zero.  Device `counts`:
+ * asynchronous on `stream`.  KFPOS_ERR_NOT_READY: no histogram or no truth trajectory registered.          */
+int kfpos_batch_error_hist(kfpos_batch *b, int64_t n_rows, uint64_t *counts, void *stream);
+
+/* The same summed over the ranks of `comm`: one ncclAllGather of n_rows * (n_edges + 1) uint64 per rank,
+ * then an integer sum over the ranks.  Counts are integers, so the result is EXACTLY the single-GPU result
+ * for any shard sizes.  NCCL is bound as for kfpos_stats_allreduce (comm == NULL: this batch alone).      */
+int kfpos_error_hist_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, uint64_t *counts,
+                               void *stream);
+
 /* Roofline denominator for this FP64 CUDA-core path (no reference equivalent):
  * times a DFMA-only kernel on `device` and returns the sustained FLOP/s.        */
 int kfpos_measure_fp64_peak(int device, double *flops_per_s);

@@ -342,6 +342,49 @@ class Batch:
                                                     _stream_ptr(stream)), "kfpos_epoch_stats_allreduce")
         return out
 
+    # ------------------------------------------------ per-epoch error histograms
+    _HIST_QUANTITY = {"err": L.HIST_ERR, "err_xy": L.HIST_ERR_XY, "nees": L.HIST_NEES}
+
+    def set_error_hist(self, edges, quantity="err"):
+        """Registers a per-epoch histogram of `quantity` ("err" = |p - truth| in m, "err_xy" = the x-y error in m,
+        "nees") with the bin edges `edges` (1..255 finite, strictly increasing values; >= 0 for the errors):
+        bin k of a row counts the filters with exactly k edges <= their value (kfpos_batch_set_error_hist).  It
+        is filled while a truth trajectory is registered (set_truth_traj) and survives its re-registration.
+        None (or no edges) unregisters."""
+        if quantity not in self._HIST_QUANTITY:
+            raise ValueError(f"set_error_hist: quantity must be one of {sorted(self._HIST_QUANTITY)}")
+        e = None if edges is None else np.ascontiguousarray(edges, dtype=np.float64).reshape(-1)
+        n = 0 if e is None else len(e)
+        L.check(L.lib().kfpos_batch_set_error_hist(self._h, self._HIST_QUANTITY[quantity], n,
+                                                   C.c_void_p(e.ctypes.data) if n else None),
+                "kfpos_batch_set_error_hist")
+        self._eh_bins = n + 1 if n else 0
+
+    def error_hist(self, readback=True, out=None, stream=None):
+        """[rows][n_edges + 1] uint64 counts per output row (kfpos_batch_error_hist).  out: a device tensor
+        (int64 or uint64) of that shape to fill asynchronously (returned as given); readback False without
+        `out`: a new device int64 tensor, filled asynchronously."""
+        rows, bins = getattr(self, "_es_rows", 0), getattr(self, "_eh_bins", 0)
+        if out is None and readback:
+            out = np.zeros((rows, bins), dtype=np.uint64)
+        if out is None:
+            import torch
+            out = torch.empty((rows, bins), dtype=torch.int64, device="cuda:%d" % self.device)
+        L.check(L.lib().kfpos_batch_error_hist(self._h, C.c_int64(rows), _ptr(out)[0], _stream_ptr(stream)),
+                "kfpos_batch_error_hist")
+        return out
+
+    def error_hist_allreduce(self, comm=None, stream=None):
+        """kfpos_error_hist_allreduce: error_hist summed over the ranks of the NCCL communicator `comm` (a raw
+        ncclComm_t as an int / c_void_p, see shard.nccl_comm; None = this batch alone).  Exact for any shard
+        sizes.  Returns [rows][n_edges + 1] uint64."""
+        rows, bins = getattr(self, "_es_rows", 0), getattr(self, "_eh_bins", 0)
+        out = np.zeros((rows, bins), dtype=np.uint64)
+        c = C.c_void_p(int(comm)) if comm else None
+        L.check(L.lib().kfpos_error_hist_allreduce(self._h, c, C.c_int64(rows), C.c_void_p(out.ctypes.data),
+                                                   _stream_ptr(stream)), "kfpos_error_hist_allreduce")
+        return out
+
 
 def epoch_summary(stats):
     """Per-row summary of epoch_stats / epoch_stats_allreduce output [rows][6]: dict of arrays rmse, rmse_xy
@@ -354,6 +397,33 @@ def epoch_summary(stats):
         return dict(rmse=np.where(n > 0, np.sqrt(s[:, 0] / n), np.nan),
                     rmse_xy=np.where(n > 0, np.sqrt(s[:, 1] / n), np.nan),
                     anees=np.where(ne > 0, s[:, 4] / ne, np.nan), n=n.copy(), n_bad=s[:, 3].copy())
+
+
+def hist_quantiles(counts, edges, q):
+    """Brackets quantiles of each row of error_hist output counts [rows][n_edges + 1] with the edges it was
+    registered with.  For each row and each q in `q` (in [0, 1]) returns the interval [lo, hi) of the bin that
+    holds the q-quantile: the smallest value v with at least max(1, ceil(q * n)) of the row's n values <= v.
+    The quantile is only bracketed, not interpolated inside its bin, so it is known to one bin width.  lo of
+    bin 0 is 0 (errors and NEES are never negative); hi of the last bin is inf.  Empty rows give NaN.
+    Returns (lo, hi), each [rows][len(q)]."""
+    c = np.asarray(counts).astype(np.float64)
+    c = c.reshape(-1, c.shape[-1])
+    e = np.asarray(edges, dtype=np.float64).reshape(-1)
+    if c.shape[1] != len(e) + 1:
+        raise ValueError("hist_quantiles: counts must have len(edges) + 1 bins")
+    qs = np.atleast_1d(np.asarray(q, dtype=np.float64))
+    if np.any(qs < 0) or np.any(qs > 1):
+        raise ValueError("hist_quantiles: q must lie in [0, 1]")
+    cum = np.cumsum(c, axis=1)
+    n = cum[:, -1]
+    # the bin of the k-th smallest value: the first bin whose cumulative count reaches k
+    k = np.maximum(1.0, np.ceil(qs[None, :] * n[:, None]))
+    b = np.minimum((cum[:, :, None] < k[:, None, :]).sum(axis=1), c.shape[1] - 1)
+    lo = np.concatenate([[0.0], e])[b]
+    hi = np.concatenate([e, [np.inf]])[b]
+    lo[n <= 0] = np.nan
+    hi[n <= 0] = np.nan
+    return lo, hi
 
 
 def assemble_epochs(anchor, seq, range_mm, t, n_anchors, max_epochs, err=None, fix_row_clear=False, first_dt=0.1,

@@ -81,6 +81,13 @@ struct kfpos_batch {
     double *d_etruth_own = nullptr, *d_escratch = nullptr, *d_efold = nullptr, *d_eout = nullptr;
     int64_t es_rows = 0, es_cursor = 0, es_fold_rows = 0;
     DevBuf es_gather;
+    // per-epoch error histogram (kfpos_batch_set_error_hist): the quantity, the device edge table [EH_MAX_BINS - 1]
+    // (squared for the error quantities, +inf behind the last edge), and the counts [es_rows][eh_bins], which
+    // exist while a truth trajectory is registered too
+    int eh_quantity = 0, eh_bins = 0; // eh_bins == 0: no histogram
+    double *d_eh_edges = nullptr;
+    unsigned long long *d_eh_counts = nullptr;
+    DevBuf eh_gather;
     // K8 / T9 latched sensor samples, SoA rows (see kfpos_k8.cuh)
     double *d_latch = nullptr;
     double *d_latch_u = nullptr; // batch-wide latched IMU covariances
@@ -307,22 +314,33 @@ int64_t es_warps(const kfpos_batch *b) { return (b->N + 31) / 32; }
 int es_check(const kfpos_batch *b, int64_t rows) {
     return (b->d_escratch && b->es_cursor + rows > b->es_rows) ? KFPOS_ERR_INVALID : KFPOS_OK;
 }
-// the per-epoch statistics pointers of the next launch, then the cursor moves past its `rows` output rows
+// the per-epoch statistics pointers of the next launch, then the cursor moves past its `rows` output rows.  The
+// histogram rows of the launch are zeroed first: a re-run after set_state overwrites them, as it does the sums.
 template <class Params>
-void es_bind(kfpos_batch *b, Params &p, int64_t rows) {
+int es_bind(kfpos_batch *b, Params &p, int64_t rows, cudaStream_t s) {
     p.n_warps = es_warps(b);
     p.etruth = nullptr;
     p.escratch = nullptr;
-    if (!b->d_escratch) return;
+    p.ehist = nullptr;
+    p.eedges = b->d_eh_edges;
+    p.equantity = b->eh_quantity;
+    p.ebins = b->eh_bins;
+    if (!b->d_escratch) return KFPOS_OK;
     p.etruth = b->d_etruth + b->es_cursor * 3 * b->N;
     p.escratch = b->d_escratch + b->es_cursor * p.n_warps * ES_W;
+    if (b->d_eh_counts) {
+        p.ehist = b->d_eh_counts + b->es_cursor * b->eh_bins;
+        CK(cudaMemsetAsync(p.ehist, 0, sizeof(unsigned long long) * (size_t)rows * (size_t)b->eh_bins, s));
+    }
     b->es_cursor += rows;
+    return KFPOS_OK;
 }
 
 // the fields the T6, K8 and T9 replay parameters share (kept apart in each struct: a shared sub-struct would move
 // the kernel parameter offsets); the launch has `rows` output rows
 template <class Params>
-void bind_replay(kfpos_batch *b, Params &p, const RangeStream &rs, const double *dt_f, double *traj, int64_t rows) {
+int bind_replay(kfpos_batch *b, Params &p, const RangeStream &rs, const double *dt_f, double *traj, int64_t rows,
+                cudaStream_t s) {
     p.anchors = b->anchors;
     p.rs = rs;
     p.N = b->N;
@@ -334,7 +352,7 @@ void bind_replay(kfpos_batch *b, Params &p, const RangeStream &rs, const double 
     p.counters = b->d_counters;
     p.truth = b->d_truth;
     p.partials = b->d_partials;
-    es_bind(b, p, rows);
+    return es_bind(b, p, rows, s);
 }
 
 // after a replay launch: the partials of a registered truth are those of the new state, the folded statistics are
@@ -446,6 +464,9 @@ extern "C" void kfpos_batch_destroy(kfpos_batch *b) {
     cudaFree(b->d_efold);
     cudaFree(b->d_eout);
     b->es_gather.release();
+    cudaFree(b->d_eh_edges);
+    cudaFree(b->d_eh_counts);
+    b->eh_gather.release();
     cudaFree(b->d_latch);
     cudaFree(b->d_has);
     cudaFree(b->d_latch_u);
@@ -675,7 +696,7 @@ int launch_t6(kfpos_batch *b, int T, const double *d_dt, const void *d_ranges, i
               const double *d_dt_f) {
     b->stepped = true;
     T6Params p;
-    bind_replay(b, p, make_rs(b, d_ranges, fmt, err_scalar, d_err), d_dt_f, d_traj, T);
+    if (int rc = bind_replay(b, p, make_rs(b, d_ranges, fmt, err_scalar, d_err), d_dt_f, d_traj, T, s)) return rc;
     p.T = T;
     p.ignore_worst = b->cfg.ignore_worst_anchor;
     p.variant = b->cfg.variant;
@@ -765,7 +786,7 @@ int run_events(kfpos_batch *b, Staging &st, int n, const kfpos_event *events, co
     switch (b->model) {
     case KFPOS_MODEL_K8: {
         K8Params p;
-        bind_replay(b, p, rs, d_dt_f, d_traj, n_toa);
+        if (int rc = bind_replay(b, p, rs, d_dt_f, d_traj, n_toa, s)) return rc;
         p.cfg = make_k8cfg(b);
         p.sensors = d_sensors;
         p.events = d_events;
@@ -779,7 +800,7 @@ int run_events(kfpos_batch *b, Staging &st, int n, const kfpos_event *events, co
     }
     case KFPOS_MODEL_T9: {
         T9Params p;
-        bind_replay(b, p, rs, d_dt_f, d_traj, n_toa);
+        if (int rc = bind_replay(b, p, rs, d_dt_f, d_traj, n_toa, s)) return rc;
         p.accel_noise = b->cfg.accel_noise;
         p.jolt = b->cfg.jolt;
         p.sensors = d_sensors;
@@ -1239,14 +1260,16 @@ NcclApi &nccl_api() {
     return api;
 }
 
-// ONE collective: the `count` doubles at `send` of every rank to every rank, [rank][count] in `recv` (grown to
-// fit); the number of ranks comes back in `n_ranks`
-int all_gather(struct ncclComm *comm, const double *send, size_t count, DevBuf &recv, int *n_ranks, cudaStream_t s) {
+// ONE collective: the `count` 8-byte values at `send` of every rank to every rank, [rank][count] in `recv` (grown
+// to fit); the number of ranks comes back in `n_ranks`
+constexpr int NCCL_UINT64 = 5, NCCL_DOUBLE = 8; // ncclDataType_t
+int all_gather(struct ncclComm *comm, const void *send, size_t count, DevBuf &recv, int *n_ranks, cudaStream_t s,
+               int type = NCCL_DOUBLE) {
     NcclApi &api = nccl_api();
     if (!api.all_gather || !api.count) return KFPOS_ERR_UNSUPPORTED;
     if (api.count(comm, n_ranks) != 0 || *n_ranks < 1 || *n_ranks > 1024) return KFPOS_ERR_INVALID;
     CK(recv.reserve(sizeof(double) * count * (size_t)*n_ranks));
-    return api.all_gather(send, recv.p, count, 8 /* ncclDouble */, comm, s) != 0 ? KFPOS_ERR_CUDA : KFPOS_OK;
+    return api.all_gather(send, recv.p, count, type, comm, s) != 0 ? KFPOS_ERR_CUDA : KFPOS_OK;
 }
 } // namespace
 
@@ -1298,7 +1321,9 @@ extern "C" int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const 
     cudaFree(b->d_escratch);
     cudaFree(b->d_efold);
     cudaFree(b->d_eout);
+    cudaFree(b->d_eh_counts);
     b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
+    b->d_eh_counts = nullptr;
     b->d_etruth = nullptr;
     b->es_rows = b->es_cursor = b->es_fold_rows = 0;
     if (!truth) return KFPOS_OK;
@@ -1312,6 +1337,10 @@ extern "C" int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const 
     cudaError_t e = cudaMalloc((void **)&b->d_escratch, row_bytes * (size_t)n_rows);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_efold, row_bytes * (size_t)fold_rows);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_eout, sizeof(double) * ES_W * (size_t)n_rows);
+    // a registered histogram gets its counts with the rows (kfpos_batch_set_error_hist)
+    const size_t hbytes = sizeof(unsigned long long) * (size_t)b->eh_bins * (size_t)n_rows;
+    if (e == cudaSuccess && hbytes) e = cudaMalloc((void **)&b->d_eh_counts, hbytes);
+    if (e == cudaSuccess && hbytes) e = cudaMemsetAsync(b->d_eh_counts, 0, hbytes, s);
     const size_t tbytes = sizeof(double) * 3 * (size_t)b->N * (size_t)n_rows;
     if (e == cudaSuccess && !dev) e = cudaMalloc((void **)&b->d_etruth_own, tbytes);
     if (e == cudaSuccess && !dev) e = cudaMemcpyAsync(b->d_etruth_own, truth, tbytes, cudaMemcpyHostToDevice, s);
@@ -1321,7 +1350,9 @@ extern "C" int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const 
         cudaFree(b->d_escratch);
         cudaFree(b->d_efold);
         cudaFree(b->d_eout);
+        cudaFree(b->d_eh_counts);
         b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
+        b->d_eh_counts = nullptr;
         cudaGetLastError();
         return map_cuda_err(e);
     }
@@ -1382,6 +1413,104 @@ extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm
     }
     Staging st(b, s);
     st.copy_out(out, d_res, sizeof(double) * ES_W * (size_t)n_rows);
+    return st.finish();
+}
+
+// ------------------------------------------------------- per-epoch error histograms
+extern "C" int kfpos_batch_set_error_hist(kfpos_batch *b, int quantity, int n_edges, const double *edges) {
+    if (!b || b->model == KFPOS_MODEL_ML || n_edges < 0) return KFPOS_ERR_INVALID;
+    const bool reg = n_edges > 0 && edges;
+    std::vector<double> tbl(reg ? n_edges : 0);  // the caller's edges, then the device table
+    if (reg) {
+        if (quantity < KFPOS_HIST_ERR || quantity > KFPOS_HIST_NEES || n_edges > EH_MAX_BINS - 1) return KFPOS_ERR_INVALID;
+        int rc = to_host(tbl.data(), edges, sizeof(double) * (size_t)n_edges);
+        if (rc) return rc;
+        const bool metres = quantity != KFPOS_HIST_NEES;
+        for (int i = 0; i < n_edges; ++i) {
+            const double v = tbl[i];
+            if (!std::isfinite(v) || (metres && v < 0.0) || (i > 0 && !(v > tbl[i - 1]))) return KFPOS_ERR_INVALID;
+        }
+        // the error quantities are binned as e^2: the edges are squared here, once, so no kernel takes a root
+        if (metres)
+            for (double &v : tbl) v = v * v;
+        tbl.resize(EH_MAX_BINS - 1, INFINITY); // the kernel's search always spans EH_MAX_BINS - 1 entries
+    }
+    DeviceGuard g(b->device);
+    // (cudaFree waits for the device: no launch still reads the previous table or counts)
+    cudaFree(b->d_eh_edges);
+    cudaFree(b->d_eh_counts);
+    b->d_eh_edges = nullptr;
+    b->d_eh_counts = nullptr;
+    b->eh_bins = b->eh_quantity = 0;
+    if (!reg) return KFPOS_OK;
+    const size_t hbytes = sizeof(unsigned long long) * (size_t)(n_edges + 1) * (size_t)b->es_rows;
+    cudaError_t e = cudaMalloc((void **)&b->d_eh_edges, sizeof(double) * tbl.size());
+    if (e == cudaSuccess) e = cudaMemcpy(b->d_eh_edges, tbl.data(), sizeof(double) * tbl.size(), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && hbytes) e = cudaMalloc((void **)&b->d_eh_counts, hbytes);
+    if (e == cudaSuccess && hbytes) e = cudaMemset(b->d_eh_counts, 0, hbytes);
+    if (e != cudaSuccess) {
+        cudaFree(b->d_eh_edges);
+        cudaFree(b->d_eh_counts);
+        b->d_eh_edges = nullptr;
+        b->d_eh_counts = nullptr;
+        cudaGetLastError();
+        return map_cuda_err(e);
+    }
+    b->eh_quantity = quantity;
+    b->eh_bins = n_edges + 1;
+    return KFPOS_OK;
+}
+
+namespace {
+int eh_ready(const kfpos_batch *b, int64_t n_rows, const uint64_t *counts) {
+    if (!b || b->model == KFPOS_MODEL_ML || !counts) return KFPOS_ERR_INVALID;
+    if (!b->d_eh_counts) return KFPOS_ERR_NOT_READY; // no histogram or no truth trajectory
+    return n_rows == b->es_rows ? KFPOS_OK : KFPOS_ERR_INVALID;
+}
+// [es_rows][eh_bins] of this batch into the device array `d_out`: the rows the cursor has passed, the rest zero
+int enqueue_error_hist(kfpos_batch *b, unsigned long long *d_out, cudaStream_t s) {
+    const int64_t done = b->es_cursor < b->es_rows ? b->es_cursor : b->es_rows;
+    const size_t row_bytes = sizeof(unsigned long long) * (size_t)b->eh_bins;
+    if (done > 0) CK(cudaMemcpyAsync(d_out, b->d_eh_counts, row_bytes * (size_t)done, cudaMemcpyDeviceToDevice, s));
+    if (done < b->es_rows) CK(cudaMemsetAsync(d_out + done * b->eh_bins, 0, row_bytes * (size_t)(b->es_rows - done), s));
+    return KFPOS_OK;
+}
+} // namespace
+
+extern "C" int kfpos_batch_error_hist(kfpos_batch *b, int64_t n_rows, uint64_t *counts, void *stream) {
+    int rc = eh_ready(b, n_rows, counts);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    Staging st(b, s);
+    auto *d_out = (unsigned long long *)st.out(counts, sizeof(uint64_t) * (size_t)b->eh_bins * (size_t)n_rows);
+    if (st.rc) return st.rc;
+    if ((rc = enqueue_error_hist(b, d_out, s))) return rc;
+    return st.finish();
+}
+
+extern "C" int kfpos_error_hist_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, uint64_t *counts,
+                                          void *stream) {
+    int rc = eh_ready(b, n_rows, counts);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t n = (size_t)b->eh_bins * (size_t)n_rows;
+    Staging st(b, s);
+    auto *d_out = (unsigned long long *)st.out(counts, sizeof(uint64_t) * n);
+    if (st.rc) return st.rc;
+    if (!comm) {
+        if ((rc = enqueue_error_hist(b, d_out, s))) return rc;
+        return st.finish();
+    }
+    // every rank's counts to every rank ([rank][row][bin]), then the integer sum over the rank index: exact in
+    // any order, so any split of the filters over the ranks gives the single-GPU counts
+    unsigned long long *d_mine = st.buf<unsigned long long>(sizeof(uint64_t) * n);
+    if (st.rc) return st.rc;
+    if ((rc = enqueue_error_hist(b, d_mine, s))) return rc;
+    int n_ranks = 0;
+    if ((rc = all_gather(comm, d_mine, n, b->eh_gather, &n_ranks, s, NCCL_UINT64))) return rc;
+    CK(launch_sum_ranks_u64(n_ranks, (int64_t)n, (const unsigned long long *)b->eh_gather.p, d_out, s));
     return st.finish();
 }
 

@@ -55,7 +55,8 @@ KF_DEV void prefetch_event(const RawColPriv &raw, const Col &land, const EventDe
 // ES: per-epoch statistics at every TOA event (see kfpos_t6.cu): the terms go to a private shared-memory column, and
 // the warp sums them at the top of the next event or after the last one, behind a __syncwarp -- lanes of a ragged
 // replay (SEL && dt_f) reach that point on different paths.  The NEES is that of the x-y block, z = the tag height.
-template <bool PME, int MT, bool SEL = false, bool MLI = SEL, bool ES = false>
+// EH (only with ES): the per-epoch error histogram, binned beside epoch_stats_row (epoch_hist_flush).
+template <bool PME, int MT, bool SEL = false, bool MLI = SEL, bool ES = false, bool EH = false>
 __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __grid_constant__ K8Params p) {
     extern __shared__ double smem[];
     const int64_t f = (int64_t)blockIdx.x * K8_BLOCK + threadIdx.x;
@@ -114,7 +115,10 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
 
         if (p.n_events > 0) prefetch_event(raw, land, p.events[0], m, p.rs, p.sensors, N, f);
         for (int e = 0; e < p.n_events; ++e) {
-            if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+            if (ES && es_pending) {
+                es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+                if (EH) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(n_toa - 1) * p.ebins, p.eedges, p.equantity);
+            }
             const EventDesc ev = p.events[e];
             cp_async_wait_all();
             double dt_ev = ev.dt;
@@ -325,7 +329,10 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
             }
             if (!(SEL && p.dt_f)) __syncwarp(wmask); // the IEKF trip count differs per lane
         }
-        if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+        if (ES && es_pending) {
+            es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+            if (EH) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(n_toa - 1) * p.ebins, p.eedges, p.equantity);
+        }
         p.x[0 * N + f] = px; p.x[1 * N + f] = py; p.x[2 * N + f] = vx; p.x[3 * N + f] = vy;
         p.x[4 * N + f] = 0.0; p.x[5 * N + f] = 0.0; p.x[6 * N + f] = th; p.x[7 * N + f] = om;
 #pragma unroll
@@ -357,34 +364,35 @@ __global__ void __launch_bounds__(K8_BLOCK, K8_MINB) k8_replay_kernel(const __gr
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, int MT, bool SEL, bool MLI, bool ES>
+template <bool PME, int MT, bool SEL, bool MLI, bool ES, bool EH>
 static cudaError_t launch_k(const K8Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + K8_BLOCK - 1) / K8_BLOCK);
     const size_t smem = (size_t)(k8_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * K8_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(k8_replay_kernel<PME, MT, SEL, MLI, ES>,
+    cudaError_t e = cudaFuncSetAttribute(k8_replay_kernel<PME, MT, SEL, MLI, ES, EH>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    k8_replay_kernel<PME, MT, SEL, MLI, ES><<<grid, K8_BLOCK, smem, s>>>(p);
+    k8_replay_kernel<PME, MT, SEL, MLI, ES, EH><<<grid, K8_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool PME, int MT, bool ES>
+template <bool PME, int MT, bool ES, bool EH>
 static cudaError_t launch_tuned(const K8Params &p, cudaStream_t s) {
-    return p.cfg.ml_init ? launch_k<PME, MT, false, true, ES>(p, s) : launch_k<PME, MT, false, false, ES>(p, s);
+    return p.cfg.ml_init ? launch_k<PME, MT, false, true, ES, EH>(p, s) : launch_k<PME, MT, false, false, ES, EH>(p, s);
 }
 
-template <bool ES>
+template <bool ES, bool EH>
 static cudaError_t launch_replay_es(const K8Params &p, cudaStream_t s) {
     if (p.cfg.variant == 1 || p.cfg.variant == 2 || p.dt_f != nullptr) // the general instantiation
-        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES>(p, s) : launch_k<false, 0, true, true, ES>(p, s);
-    if (p.rs.err != nullptr) return launch_tuned<true, 0, ES>(p, s);
-    if (p.rs.m_slots == 8 && !p.cfg.zero_tz) return launch_tuned<false, 8, ES>(p, s);
-    return launch_tuned<false, 0, ES>(p, s);
+        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES, EH>(p, s) : launch_k<false, 0, true, true, ES, EH>(p, s);
+    if (p.rs.err != nullptr) return launch_tuned<true, 0, ES, EH>(p, s);
+    if (p.rs.m_slots == 8 && !p.cfg.zero_tz) return launch_tuned<false, 8, ES, EH>(p, s);
+    return launch_tuned<false, 0, ES, EH>(p, s);
 }
 
 cudaError_t launch_k8_replay(const K8Params &p, cudaStream_t s) {
     if (p.N <= 0 || p.n_events <= 0) return cudaSuccess;
-    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
+    if (!p.escratch) return launch_replay_es<false, false>(p, s);
+    return p.ehist ? launch_replay_es<true, true>(p, s) : launch_replay_es<true, false>(p, s);
 }
 
 // getPose (KF.cpp:709-747): predict-only, state untouched

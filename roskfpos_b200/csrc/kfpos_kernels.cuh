@@ -127,6 +127,31 @@ KF_DEV bool epoch_stats_row(const Col &v, unsigned wmask, double *es_out, int64_
     return false;
 }
 
+// ---- per-epoch error histograms (kfpos_batch_set_error_hist): a replay kernel compiled with EH = true (always
+// with ES = true) bins one of the terms already in the column wherever it flushes a row of the statistics.
+// Quantity (KFPOS_HIST_*): 0 = e^2 (v[0]), 1 = e_xy^2 (v[1]), counted when v[2] == 1; 2 = NEES (v[4]), counted
+// when v[5] == 1 -- so a row's counts add up to its [2] (or [5]) of kfpos_batch_epoch_stats.  Bin k = the number
+// of table entries <= the value (0 .. n_bins - 1); the table holds the squared edges for the error quantities, so
+// no square root is taken.  The device table always has EH_MAX_BINS - 1 entries, padded with +inf (> every counted
+// value).  Counts are integers: any order of the atomics gives the same result.
+constexpr int EH_MAX_BINS = 256;
+KF_DEV void epoch_hist_flush(const Col &v, unsigned wmask, unsigned long long *counts, const double *edges,
+                             int quantity) {
+    const int lane = threadIdx.x & 31;
+    const bool nees = quantity == 2;
+    const double x = nees ? v[4] : (quantity == 1 ? v[1] : v[0]);
+    const bool ok = (nees ? v[5] : v[2]) == 1.0;
+    // binary search with a trip count common to the warp: the lanes load from the read-only cache side by side
+    int k = 0;
+#pragma unroll
+    for (int s = EH_MAX_BINS / 2; s > 0; s >>= 1)
+        if (__ldg(edges + k + s - 1) <= x) k += s;
+    // one atomic per distinct bin of the warp; the lanes that count nothing form the key -1 and add nothing
+    const int key = ok ? k : -1;
+    const unsigned peers = __match_any_sync(wmask, key);
+    if (ok && lane == __ffs(peers) - 1) atomicAdd(counts + k, (unsigned long long)__popc(peers));
+}
+
 struct T6Params {
     AnchorTable anchors;
     RangeStream rs;
@@ -151,6 +176,13 @@ struct T6Params {
     const double *etruth;
     double *escratch;
     int64_t n_warps;
+    // per-epoch error histogram (the launchers pick the EH = true twins of the ES kernels when non-null): counts
+    // [rows][ebins] of this launch's first output row, the device edge table [EH_MAX_BINS - 1] (squared for the
+    // error quantities, +inf behind the last edge) and the quantity (KFPOS_HIST_*).  Last in the struct: the offsets of the fields above stay.
+    unsigned long long *ehist;
+    const double *eedges;
+    int equantity;
+    int ebins;
 };
 
 struct MlParams {
@@ -251,6 +283,10 @@ struct K8Params {
     const double *etruth; // see T6Params (output rows = TOA events)
     double *escratch;
     int64_t n_warps;
+    unsigned long long *ehist; // see T6Params
+    const double *eedges;
+    int equantity;
+    int ebins;
 };
 
 cudaError_t launch_t6_replay(const T6Params &p, cudaStream_t s);
@@ -291,6 +327,10 @@ struct T9Params {
     const double *etruth; // see T6Params (output rows = TOA events)
     double *escratch;
     int64_t n_warps;
+    unsigned long long *ehist; // see T6Params
+    const double *eedges;
+    int equantity;
+    int ebins;
 };
 cudaError_t launch_t9_replay(const T9Params &p, cudaStream_t s);
 cudaError_t launch_t9_get_pose(int64_t N, double dt, double jolt, const double *x, const double *P, double *x_pred,
@@ -323,6 +363,9 @@ cudaError_t launch_stats_tree(int width, int64_t rows, int64_t n, const double *
 cudaError_t launch_pose_msg(int model, int64_t N, double tag_z, const double *tagz, const double *x_pred,
                             const double *P_pred_full, double *pose13, double *cov36, cudaStream_t s);
 cudaError_t launch_fill(double *p, int64_t n, double v, cudaStream_t s);
+// out[i] = sum of src[r * n + i] over r < n_ranks (the rank fold of the error histograms)
+cudaError_t launch_sum_ranks_u64(int n_ranks, int64_t n, const unsigned long long *src, unsigned long long *out,
+                                 cudaStream_t s);
 
 // epoch assembler (kfpos_assemble.cu): N logs of L messages, SoA [L][N]
 struct AssembleParams {

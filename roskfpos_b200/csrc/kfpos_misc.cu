@@ -227,6 +227,21 @@ cudaError_t launch_fill(double *p, int64_t n, double v, cudaStream_t s) {
     return cudaGetLastError();
 }
 
+// out[i] = sum over r of src[r * n + i] (the rank fold of kfpos_error_hist_allreduce; integers: exact in any order)
+__global__ void sum_ranks_u64_kernel(int n_ranks, int64_t n, const unsigned long long *src, unsigned long long *out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    unsigned long long a = 0;
+    for (int r = 0; r < n_ranks; ++r) a += src[(int64_t)r * n + i];
+    out[i] = a;
+}
+cudaError_t launch_sum_ranks_u64(int n_ranks, int64_t n, const unsigned long long *src, unsigned long long *out,
+                                 cudaStream_t s) {
+    if (n <= 0) return cudaSuccess;
+    sum_ranks_u64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n_ranks, n, src, out);
+    return cudaGetLastError();
+}
+
 // the fast elementary functions of kfpos_math.cuh evaluated on caller data (accuracy self-test)
 __global__ void selftest_math_kernel(int64_t n, const double *x, double *rcp, double *rsq, double *sn, double *cs) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

@@ -35,7 +35,8 @@ __host__ __device__ inline int t6_smem_rows(int m, int fmt, bool pme, bool in_re
 // ES: per-epoch statistics (kfpos_batch_set_truth_traj): after every epoch the filter's error terms go to a private
 // shared-memory column (6 rows behind the others), and at the top of the next epoch -- the one point every lane of
 // the warp passes, stepping or not -- the warp sums them (epoch_stats_flush).  The ES = false code is unchanged.
-template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false>
+// EH (only with ES): the per-epoch error histogram, binned at the same two points as the sums (epoch_hist_flush).
+template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false, bool EH = false>
 __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __grid_constant__ T6Params p) {
     extern __shared__ double smem[];
     const int fmt = FMT >= 0 ? FMT : p.rs.fmt;
@@ -82,6 +83,7 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
         double dt_next = dt_f ? __ldg(dt_f + f) : 0.0;
         for (int t = 0; t < p.T; ++t) {
             if (ES && t > 0) epoch_stats_flush(es, wmask, es_out + (int64_t)(t - 1) * p.n_warps * ES_W);
+            if (EH && t > 0) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(t - 1) * p.ebins, p.eedges, p.equantity);
             // per-filter time steps (assembled logs): a negative dt = this filter has no epoch t.
             // The lanes that do step are the ones that re-converge below.
             const double dt = dt_f ? dt_next : __ldg(p.dt + t);
@@ -198,6 +200,7 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
             }
         }
         if (ES) epoch_stats_flush(es, wmask, es_out + (int64_t)(p.T - 1) * p.n_warps * ES_W);
+        if (EH) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(p.T - 1) * p.ebins, p.eedges, p.equantity);
 
 #pragma unroll
         for (int k = 0; k < 3; ++k) p.x[(int64_t)k * N + f] = pos[k];
@@ -221,51 +224,52 @@ __global__ void __launch_bounds__(T6_BLOCK, T6_MINB) t6_replay_kernel(const __gr
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false>
+template <bool PME, bool LOO, int MT, bool SEL = false, int FMT = -1, bool ES = false, bool EH = false>
 static cudaError_t launch_k(const T6Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + T6_BLOCK - 1) / T6_BLOCK);
     const size_t smem = (size_t)(t6_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * T6_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES>,
+    cudaError_t e = cudaFuncSetAttribute(t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES, EH>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES><<<grid, T6_BLOCK, smem, s>>>(p);
+    t6_replay_kernel<PME, LOO, MT, SEL, FMT, ES, EH><<<grid, T6_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
 }
 // the plain replay with a compile-time anchor count: one instantiation per wire format
-template <int MT, bool ES>
+template <int MT, bool ES, bool EH>
 static cudaError_t launch_tuned(const T6Params &p, cudaStream_t s) {
-    if (p.dt_f != nullptr) return launch_k<false, false, MT, false, -1, ES>(p, s); // per-filter time steps
+    if (p.dt_f != nullptr) return launch_k<false, false, MT, false, -1, ES, EH>(p, s); // per-filter time steps
     switch (p.rs.fmt) {
-    case 1: return launch_k<false, false, MT, false, 1, ES>(p, s);
-    case 2: return launch_k<false, false, MT, false, 2, ES>(p, s);
-    default: return launch_k<false, false, MT, false, 0, ES>(p, s);
+    case 1: return launch_k<false, false, MT, false, 1, ES, EH>(p, s);
+    case 2: return launch_k<false, false, MT, false, 2, ES, EH>(p, s);
+    default: return launch_k<false, false, MT, false, 0, ES, EH>(p, s);
     }
 }
 
-template <bool ES>
+template <bool ES, bool EH>
 static cudaError_t launch_replay_es(const T6Params &p, cudaStream_t s) {
     const bool pme = p.rs.err != nullptr;
     const int m = p.rs.m_slots;
     if (p.variant == 1 || p.variant == 2) {
         if (p.ignore_worst) return cudaErrorInvalidValue; // the two heuristics are alternatives
-        return pme ? launch_k<true, false, 0, true, -1, ES>(p, s) : launch_k<false, false, 0, true, -1, ES>(p, s);
+        return pme ? launch_k<true, false, 0, true, -1, ES, EH>(p, s) : launch_k<false, false, 0, true, -1, ES, EH>(p, s);
     }
     if (p.ignore_worst) {
-        if (pme) return launch_k<true, true, 0, false, -1, ES>(p, s);
-        if (m == 8) return launch_k<false, true, 8, false, -1, ES>(p, s);
-        if (m == 16) return launch_k<false, true, 16, false, -1, ES>(p, s);
-        return launch_k<false, true, 0, false, -1, ES>(p, s);
+        if (pme) return launch_k<true, true, 0, false, -1, ES, EH>(p, s);
+        if (m == 8) return launch_k<false, true, 8, false, -1, ES, EH>(p, s);
+        if (m == 16) return launch_k<false, true, 16, false, -1, ES, EH>(p, s);
+        return launch_k<false, true, 0, false, -1, ES, EH>(p, s);
     }
-    if (pme) return launch_k<true, false, 0, false, -1, ES>(p, s);
-    if (m == 4) return launch_k<false, false, 4, false, -1, ES>(p, s);
-    if (m == 8) return launch_tuned<8, ES>(p, s);
-    if (m == 16) return launch_tuned<16, ES>(p, s);
-    return launch_k<false, false, 0, false, -1, ES>(p, s);
+    if (pme) return launch_k<true, false, 0, false, -1, ES, EH>(p, s);
+    if (m == 4) return launch_k<false, false, 4, false, -1, ES, EH>(p, s);
+    if (m == 8) return launch_tuned<8, ES, EH>(p, s);
+    if (m == 16) return launch_tuned<16, ES, EH>(p, s);
+    return launch_k<false, false, 0, false, -1, ES, EH>(p, s);
 }
 
 cudaError_t launch_t6_replay(const T6Params &p, cudaStream_t s) {
     if (p.N <= 0 || p.T <= 0) return cudaSuccess;
-    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
+    if (!p.escratch) return launch_replay_es<false, false>(p, s);
+    return p.ehist ? launch_replay_es<true, true>(p, s) : launch_replay_es<true, false>(p, s);
 }
 
 // getPose (TOA.cpp:438-473): predict-only, state untouched

@@ -193,7 +193,8 @@ KF_DEV int t9_update(const AnchorTable &A, const EpochT<PME, MT> &ep, bool has_r
 // IMU event): no register copy of the 9x9 covariance anywhere, 4 blocks per SM like T6.
 // SEL: the EKF-side NLOS variants (see kfpos_t6.cu), 3-D selection from the predicted position.
 // ES: per-epoch statistics at every TOA event (see kfpos_t6.cu / kfpos_k8.cu), NEES of the 3x3 position block.
-template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false>
+// EH (only with ES): the per-epoch error histogram, binned beside epoch_stats_row (epoch_hist_flush).
+template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false, bool EH = false>
 __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_kernel(const __grid_constant__ T9Params p) {
     extern __shared__ double smem[];
     const int64_t f = (int64_t)blockIdx.x * T9_BLOCK + threadIdx.x;
@@ -255,7 +256,10 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
         };
         if (p.n_events > 0) prefetch(p.events[0]);
         for (int e = 0; e < p.n_events; ++e) {
-            if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+            if (ES && es_pending) {
+                es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+                if (EH) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(n_toa - 1) * p.ebins, p.eedges, p.equantity);
+            }
             const EventDesc ev = p.events[e];
             double dt = ev.dt;
             if (SEL && p.dt_f) { // ragged replay: every filter has its own time steps
@@ -403,7 +407,10 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
                 ++n_toa;
             }
         }
-        if (ES && es_pending) es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+        if (ES && es_pending) {
+            es_pending = epoch_stats_row(es, wmask, es_out, n_toa - 1, p.n_warps);
+            if (EH) epoch_hist_flush(es, wmask, p.ehist + (int64_t)(n_toa - 1) * p.ebins, p.eedges, p.equantity);
+        }
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             p.x[(int64_t)k * N + f] = pos[k];
@@ -439,34 +446,35 @@ __global__ void __launch_bounds__(T9_BLOCK, IMU ? 2 : T9_LEAN_MINB) t9_replay_ke
     if (p.truth) block_stats_partial(errv, smem, p.partials + (int64_t)blockIdx.x * 4);
 }
 
-template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false>
+template <bool PME, int MT, bool IMU, bool SEL = false, bool ES = false, bool EH = false>
 static cudaError_t launch_k(const T9Params &p, cudaStream_t s) {
     const unsigned grid = (unsigned)((p.N + T9_BLOCK - 1) / T9_BLOCK);
     const size_t smem = (size_t)(t9_smem_rows(p.rs.m_slots, p.rs.fmt, PME, MT > 0) + (ES ? ES_W : 0)) * T9_BLOCK * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(t9_replay_kernel<PME, MT, IMU, SEL, ES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(t9_replay_kernel<PME, MT, IMU, SEL, ES, EH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
     if (e != cudaSuccess) return e;
-    t9_replay_kernel<PME, MT, IMU, SEL, ES><<<grid, T9_BLOCK, smem, s>>>(p);
+    t9_replay_kernel<PME, MT, IMU, SEL, ES, EH><<<grid, T9_BLOCK, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool ES>
+template <bool ES, bool EH>
 static cudaError_t launch_replay_es(const T9Params &p, cudaStream_t s) {
     if (p.variant == 1 || p.variant == 2 || p.dt_f != nullptr || p.ml_init) // the general instantiation
-        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES>(p, s) : launch_k<false, 0, true, true, ES>(p, s);
+        return p.rs.err != nullptr ? launch_k<true, 0, true, true, ES, EH>(p, s) : launch_k<false, 0, true, true, ES, EH>(p, s);
     if (p.no_imu) {
-        if (p.rs.err != nullptr) return launch_k<true, 0, false, false, ES>(p, s);
-        if (p.rs.m_slots == 8) return launch_k<false, 8, false, false, ES>(p, s);
-        return launch_k<false, 0, false, false, ES>(p, s);
+        if (p.rs.err != nullptr) return launch_k<true, 0, false, false, ES, EH>(p, s);
+        if (p.rs.m_slots == 8) return launch_k<false, 8, false, false, ES, EH>(p, s);
+        return launch_k<false, 0, false, false, ES, EH>(p, s);
     }
-    if (p.rs.err != nullptr) return launch_k<true, 0, true, false, ES>(p, s);
-    if (p.rs.m_slots == 8) return launch_k<false, 8, true, false, ES>(p, s);
-    return launch_k<false, 0, true, false, ES>(p, s);
+    if (p.rs.err != nullptr) return launch_k<true, 0, true, false, ES, EH>(p, s);
+    if (p.rs.m_slots == 8) return launch_k<false, 8, true, false, ES, EH>(p, s);
+    return launch_k<false, 0, true, false, ES, EH>(p, s);
 }
 
 cudaError_t launch_t9_replay(const T9Params &p, cudaStream_t s) {
     if (p.N <= 0 || p.n_events <= 0) return cudaSuccess;
-    return p.escratch ? launch_replay_es<true>(p, s) : launch_replay_es<false>(p, s);
+    if (!p.escratch) return launch_replay_es<false, false>(p, s);
+    return p.ehist ? launch_replay_es<true, true>(p, s) : launch_replay_es<true, false>(p, s);
 }
 
 // getPose (TOAIMU.cpp:476-510): predict-only, state untouched

@@ -19,6 +19,7 @@ FMT_F64_M, FMT_I32_MM, FMT_U16_MM = 0, 1, 2
 ST_NO_MEAS, ST_ML_FEW, ST_SINGULAR, ST_NAN, ST_ML_NAN, ST_MAXITER, ST_ASYM_R = 1, 2, 4, 8, 16, 32, 64
 ST_Z_GATE = 128
 ST_UNINIT = 256
+HIST_ERR, HIST_ERR_XY, HIST_NEES = 0, 1, 2
 
 
 class KfposConfig(C.Structure):
@@ -108,6 +109,9 @@ SIGNATURES = {
     "kfpos_epoch_stats_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
     "kfpos_synth_k8_truth": (_I, [_I, _I64, _I64, C.c_uint64, _I, _VP, _D, _VP, _VP]),
     "kfpos_synth_toa_ranges": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _VP]),
+    "kfpos_batch_set_error_hist": (_I, [_VP, _I, _I, _VP]),
+    "kfpos_batch_error_hist": (_I, [_VP, _I64, _VP, _VP]),
+    "kfpos_error_hist_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

@@ -353,14 +353,17 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
 def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
                    nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
-                   stream=None):
+                   stream=None, hist=None):
     """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
     for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
     truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
     Batch.epoch_stats reads its rows.  init_state: start from the truth at t = 0 with zero velocity (and the
     batch's initial covariance); False continues from the batch's state at epoch epoch0.  The batch's filter f
     is global filter first_filter + f.  Returns the [n_epochs][6] rows of kfpos_batch_epoch_stats for
-    batch.epoch_summary (RMSE(t), ANEES(t)); the truth is unregistered on return."""
+    batch.epoch_summary (RMSE(t), ANEES(t)); the truth is unregistered on return.
+    hist=(edges, quantity): also a per-epoch histogram (Batch.set_error_hist), read chunk by chunk beside the
+    statistics; then returns (rows, counts [n_epochs][len(edges) + 1] uint64), and the histogram is
+    unregistered on return as well."""
     from . import lib as L
     if batch.model != L.MODEL_T6:
         raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
@@ -368,7 +371,9 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
         raise ValueError("toa_montecarlo: n_epochs and chunk must be positive")
     kw = dict(seed=seed, period=period, sigma_r=sigma_r, p_missing=p_missing, p_nlos=p_nlos, nlos_mean=nlos_mean,
               tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream)
-    rows, bufs = [], {}
+    rows, counts, bufs = [], [], {}
+    if hist is not None:
+        batch.set_error_hist(hist[0], hist[1])
     try:
         for k0 in range(0, int(n_epochs), int(chunk)):
             n = min(int(chunk), int(n_epochs) - k0)
@@ -379,6 +384,12 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
             batch.set_truth_traj(w["truth"], stream=stream)
             batch.replay_toa(w["dt"], w["ranges"], err=err, stream=stream)
             rows.append(batch.epoch_stats(stream=stream))
+            if hist is not None:
+                counts.append(batch.error_hist(stream=stream))
     finally:
         batch.set_truth_traj(None, stream=stream)
+        if hist is not None:
+            batch.set_error_hist(None)
+    if hist is not None:
+        return np.concatenate(rows, axis=0), np.concatenate(counts, axis=0)
     return np.concatenate(rows, axis=0)
