@@ -573,6 +573,46 @@ int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const d
                            int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
                            void *ranges, void *stream);
 
+/* The same log with its NLOS ground truth: nlos SoA [n_epochs][N] uint32 (host or device), bit a set when ranging
+ * a drew a bias (v < p_nlos above) AND is present in the log (value > 0 after the missing test and the floor).
+ * All zero without impairments.  `ranges` is byte for byte what kfpos_synth_toa_ranges writes for the same
+ * arguments.  Arguments, errors and the sync rule are those of kfpos_synth_toa_ranges (the call is asynchronous
+ * when `ranges` and `nlos` are both device pointers); a NULL nlos is KFPOS_ERR_INVALID.                     */
+int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
+                                void *ranges, uint32_t *nlos, void *stream);
+
+/* NLOS detection scores of a ranging selection (no reference equivalent; DESIGN §4.5d): how the selection of
+ * rows [0, n_rows) of a log this batch has just replayed (T6, kfpos_batch_replay_toa) or solved (ML,
+ * kfpos_batch_ml_solve) compares with the NLOS truth.  ranges: the log, SoA [n_rows][n_anchors][N] in any fmt; a
+ * ranging is present when its value is > 0 (mm > 0, metres > 0; NaN is not), the replay's rule.  nlos: SoA
+ * [n_rows][N] uint32 masks (kfpos_synth_toa_ranges_nlos), or NULL: no ranging is NLOS (drop rates of real logs).
+ * `sel` is read as the batch's configuration wrote it:
+ *   T6, variant 1 or 2:         sel [n_rows][N] = the bit mask of the slots used, read as uint32 (with 32 anchors a
+ *                               full mask is -1);
+ *   T6, ignore_worst_anchor:    sel [n_rows][N] = the slot left out, or -1 for none;
+ *   T6 otherwise:               nothing is dropped; sel is not read and may be NULL;
+ *   ML, variant 1 or 2:         n_rows == 1 and sel = the [2][N] output of kfpos_batch_ml_solve; row 0, the mask of
+ *                               the final solve, is read.  Epochs with too few rangings (KFPOS_ST_ML_FEW) hold the
+ *                               present set there, so they drop nothing.  So do epochs whose all-ranging solve
+ *                               failed (KFPOS_ST_SINGULAR), and variant-2 epochs in which a subset solve failed
+ *                               (the reference selects nothing then).  A variant-1 epoch whose re-solve after the
+ *                               drop failed keeps the reduced set: its drop counts;
+ *   ML, variant 0:              nothing is dropped; sel is not read (n_rows == 1 still).
+ * used = that set, dropped = present & ~used.  counts [n_rows][KFPOS_SCORE_COLS] uint64 (host or device),
+ * overwritten, per row summed over the filters:
+ *   [0] rangings present          [1] rangings dropped
+ *   [2] NLOS rangings (present, mask bit set)                  [3] NLOS rangings dropped
+ *   [4] filters with at least one NLOS ranging                 [5] of [4], filters whose used set has no NLOS ranging
+ *   [6] filters that dropped at least one ranging              [7] of [6], filters without any NLOS ranging
+ * Detection rate [3]/[2], false-drop rate ([1]-[3])/([0]-[2]), clean-filter rate [5]/[4], filter false-alarm rate
+ * [7]/(N-[4]).  Counts are integers: a sharded run sums them exactly with any integer all-reduce.
+ * KFPOS_ERR_UNSUPPORTED: K8 and T9 batches.  KFPOS_ERR_INVALID: n_rows <= 0, a bad fmt, NULL ranges or counts, a
+ * NULL sel where it is read, n_rows != 1 for ML.  KFPOS_ERR_NOT_READY: no anchors.                           */
+#define KFPOS_SCORE_COLS 8
+int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const void *ranges, int fmt, const int32_t *sel,
+                                const uint32_t *nlos, uint64_t *counts, void *stream);
+
 /* Accuracy self-test of the kernels' elementary functions (no reference equivalent): evaluates the
  * MUFU-seeded reciprocal and reciprocal square root and the reduced-range sincos on x[0..n) so that
  * a test can compare them with IEEE division / sqrt / libm.  Outputs may be NULL.               */

@@ -385,6 +385,28 @@ class Batch:
                                                    _stream_ptr(stream)), "kfpos_error_hist_allreduce")
         return out
 
+    # ------------------------------------------------------- selection scores
+    def score_selection(self, ranges, sel=None, nlos=None, out=None, readback=True, stream=None):
+        """NLOS detection scores of the selection this batch just made (kfpos_batch_score_selection): T6 ranges
+        [T][M][N] with the `sel` [T][N] of replay_toa; ML ranges [M][N] with the `sel` [2][N] of ml_solve.  nlos:
+        the [rows][N] masks of synth.toa_montecarlo_chunk(want_nlos=True) (int32 holding the uint32 bits), or None
+        (no ranging is NLOS).  sel may be None where the configuration drops nothing (plain T6, ML variant 0).
+        Returns counts [rows][8] (columns in selection_summary) as uint64 numpy; out: a device tensor (int64 or
+        uint64) of that shape to fill asynchronously (returned as given); readback False without `out`: a new
+        device int64 tensor, filled asynchronously."""
+        rows = 1 if self.model == L.MODEL_ML else int(ranges.shape[0])
+        if out is None and readback:
+            out = np.zeros((rows, L.SCORE_COLS), dtype=np.uint64)
+        if out is None:
+            import torch
+            out = torch.empty((rows, L.SCORE_COLS), dtype=torch.int64, device="cuda:%d" % self.device)
+        pr, kr = _ptr(ranges)
+        ps, ks = _ptr(sel, np.int32)
+        pn, kn = _ptr(nlos, np.uint32)
+        L.check(L.lib().kfpos_batch_score_selection(self._h, rows, pr, _fmt_of(ranges), ps, pn, _ptr(out)[0],
+                                                    _stream_ptr(stream)), "kfpos_batch_score_selection")
+        return out
+
 
 def epoch_summary(stats):
     """Per-row summary of epoch_stats / epoch_stats_allreduce output [rows][6]: dict of arrays rmse, rmse_xy
@@ -397,6 +419,21 @@ def epoch_summary(stats):
         return dict(rmse=np.where(n > 0, np.sqrt(s[:, 0] / n), np.nan),
                     rmse_xy=np.where(n > 0, np.sqrt(s[:, 1] / n), np.nan),
                     anees=np.where(ne > 0, s[:, 4] / ne, np.nan), n=n.copy(), n_bad=s[:, 3].copy())
+
+
+def selection_summary(counts, n_filters):
+    """Per-row rates of score_selection output counts [rows][8] over a batch of n_filters filters (the sum of the
+    shards' sizes for summed counts): detection = NLOS rangings dropped / NLOS rangings present; false_drop = LOS
+    rangings dropped / LOS rangings present; clean = filters with an NLOS ranging whose used set has none / filters
+    with an NLOS ranging; false_alarm = filters without an NLOS ranging that dropped one / filters without an NLOS
+    ranging.  A zero denominator gives NaN."""
+    c = np.asarray(counts).astype(np.float64).reshape(-1, 8)
+
+    def rate(num, den):
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.where(den > 0, num / np.where(den > 0, den, 1.0), np.nan)
+    return dict(detection=rate(c[:, 3], c[:, 2]), false_drop=rate(c[:, 1] - c[:, 3], c[:, 0] - c[:, 2]),
+                clean=rate(c[:, 5], c[:, 4]), false_alarm=rate(c[:, 7], float(n_filters) - c[:, 4]))
 
 
 def hist_quantiles(counts, edges, q):

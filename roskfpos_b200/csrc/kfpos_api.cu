@@ -1594,9 +1594,10 @@ extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first
     return st.finish();
 }
 
-extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
-                                      int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
-                                      void *ranges, void *stream) {
+namespace {
+// kfpos_synth_toa_ranges with an optional NLOS mask output (kfpos_synth_toa_ranges_nlos)
+int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz, int n_epochs,
+                     const double *t, const kfpos_synth_toa *gen, int fmt, void *ranges, uint32_t *nlos, void *stream) {
     const auto prob = [](double q) { return q >= 0.0 && q <= 1.0; }; // false for NaN
     if (n_filters <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || !anchors_xyz || n_epochs < 0 ||
         (n_epochs > 0 && (!t || !ranges)) || !gen || (fmt != KFPOS_FMT_I32_MM && fmt != KFPOS_FMT_U16_MM))
@@ -1611,13 +1612,15 @@ extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_ancho
     if (!g.ok) return KFPOS_ERR_CUDA;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t row = fmt_size(fmt) * (size_t)n_anchors * (size_t)n_filters; // bytes of one epoch
-    // the epoch times travel in the parameter block, SYNTH_TOA_T per launch: nothing to stage, so a device
-    // `ranges` leaves the call asynchronous (the next chunk can be generated while this one is replayed)
+    const size_t mask_row = sizeof(uint32_t) * (size_t)n_filters;
+    // the epoch times travel in the parameter block, SYNTH_TOA_T per launch: nothing to stage, so device outputs
+    // leave the call asynchronous (the next chunk can be generated while this one is replayed)
     SynthToaParams p{};
     int rc = anchor_table(n_anchors, anchors_xyz, &p.anchors);
     if (rc) return rc;
     Staging st(s);
     char *d_r = st.out((char *)ranges, row * (size_t)n_epochs);
+    uint32_t *d_m = st.out(nlos, mask_row * (size_t)n_epochs);
     if (st.rc) return st.rc;
     p.N = n_filters; p.filter0 = gen->first_filter; p.seed = gen->seed; p.M = n_anchors;
     p.tag_z = gen->tag_z; p.sigma_r = gen->sigma_r; p.p_missing = gen->p_missing; p.p_nlos = gen->p_nlos;
@@ -1627,8 +1630,51 @@ extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_ancho
         p.epoch0 = (uint32_t)(gen->first_epoch + k0);
         memcpy(p.t, t + k0, sizeof(double) * (size_t)p.n_epochs);
         p.ranges = d_r + row * (size_t)k0;
+        p.nlos = d_m ? d_m + (size_t)n_filters * (size_t)k0 : nullptr;
         CK(launch_synth_toa(p, fmt == KFPOS_FMT_U16_MM, s));
     }
+    return st.finish();
+}
+} // namespace
+
+extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                      int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
+                                      void *ranges, void *stream) {
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, fmt, ranges, nullptr, stream);
+}
+
+extern "C" int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                           int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
+                                           void *ranges, uint32_t *nlos, void *stream) {
+    if (!nlos) return KFPOS_ERR_INVALID;
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, fmt, ranges, nlos, stream);
+}
+
+extern "C" int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const void *ranges, int fmt, const int32_t *sel,
+                                           const uint32_t *nlos, uint64_t *counts, void *stream) {
+    static_assert(KFPOS_SCORE_COLS == SCORE_COLS, "one column count");
+    if (!b) return KFPOS_ERR_INVALID;
+    if (b->model == KFPOS_MODEL_K8 || b->model == KFPOS_MODEL_T9) return KFPOS_ERR_UNSUPPORTED;
+    const bool ml = b->model == KFPOS_MODEL_ML;
+    if (n_rows <= 0 || !fmt_ok(fmt) || !ranges || !counts || (ml && n_rows != 1)) return KFPOS_ERR_INVALID;
+    if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
+    // how `sel` is read: as the replay (T6) or the solve (ML, row 0 of its [2][N]) wrote it
+    const bool variant = b->cfg.variant == 1 || b->cfg.variant == 2;
+    const int mode = variant ? SCORE_MASK : (!ml && b->cfg.ignore_worst_anchor) ? SCORE_LOO : SCORE_NONE;
+    if (mode != SCORE_NONE && !sel) return KFPOS_ERR_INVALID;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t N = (size_t)b->N, M = (size_t)b->anchors.n, R = (size_t)n_rows;
+    Staging st(b, s);
+    ScoreParams p;
+    p.ranges = st.in(ranges, fmt_size(fmt) * M * N * R);
+    p.sel = mode == SCORE_NONE ? nullptr : st.in(sel, sizeof(int32_t) * N * R);
+    p.nlos = st.in(nlos, sizeof(uint32_t) * N * R);
+    p.counts = (unsigned long long *)st.out(counts, sizeof(uint64_t) * SCORE_COLS * R);
+    if (st.rc) return st.rc;
+    p.N = b->N; p.n_rows = n_rows; p.M = (int)M; p.fmt = fmt; p.mode = mode;
+    CK(cudaMemsetAsync(p.counts, 0, sizeof(uint64_t) * SCORE_COLS * R, s));
+    CK(launch_score_selection(p, s));
     return st.finish();
 }
 

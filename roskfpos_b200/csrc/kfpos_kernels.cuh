@@ -449,8 +449,24 @@ struct SynthToaParams {
     double tag_z, sigma_r, p_missing, p_nlos, nlos_mean;
     void *ranges; // SoA [n_epochs][M][N], int32 or uint16 mm
     double t[SYNTH_TOA_T];
+    uint32_t *nlos; // SoA [n_epochs][N] NLOS bit masks, or null (last: the offsets of the fields above stay)
 };
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s); // u16: uint16 mm, else int32 mm
+
+// selection scores against the NLOS truth (kfpos_score.cu, kfpos_batch_score_selection): counts [n_rows][8],
+// zeroed by the caller.  How `sel` [n_rows][N] is read: SCORE_NONE not at all (nothing dropped), SCORE_LOO the
+// ignored slot or -1, SCORE_MASK the bit mask of the slots used.
+constexpr int SCORE_COLS = 8;
+enum { SCORE_NONE = 0, SCORE_LOO = 1, SCORE_MASK = 2 };
+struct ScoreParams {
+    const void *ranges;   // SoA [n_rows][M][N] in fmt
+    const int32_t *sel;   // SoA [n_rows][N], or null with SCORE_NONE
+    const uint32_t *nlos; // SoA [n_rows][N], or null: no ranging is NLOS
+    unsigned long long *counts;
+    int64_t N, n_rows;
+    int M, fmt, mode;
+};
+cudaError_t launch_score_selection(const ScoreParams &p, cudaStream_t s);
 
 // DFMA-only microbenchmark on the current device (the FP64 roofline denominator)
 cudaError_t measure_fp64_peak(double *flops_per_s);

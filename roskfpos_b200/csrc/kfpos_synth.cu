@@ -118,9 +118,11 @@ cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s) {
 //   IMPAIR: (u, v) = uniform2(Philox(gf, g, 0x80000000 | a)): missing when u < p_missing, NLOS bias
 //           -nlos_mean log(v / p_nlos) when v < p_nlos (v / p_nlos is uniform then: one draw gives both);
 //   mm = floor((d_a + sigma_r n_a + bias) * 1000), 0 ("no ranging", TOA.cpp:50) when missing or <= 0.
+// MASK: also the NLOS truth, SoA [k][N] uint32 with bit a set when ranging a drew a bias and was written (> 0),
+// gathered in a register and stored once per epoch (kfpos_synth_toa_ranges_nlos).
 // The epoch times and the anchors are read from the parameter block: every lane reads the same one at the
 // same time (constant-bank broadcast).  Stores: SoA [k][a][N], filter index fastest -- coalesced.
-template <typename Out, bool IMPAIR>
+template <typename Out, bool IMPAIR, bool MASK = false>
 __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
     if (f >= p.N) return;
@@ -133,6 +135,7 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
     for (int k = 0; k < p.n_epochs; ++k) {
         const Kin kn = kin_at(p.t[k], pa, pb, th0);
         const uint32_t g = p.epoch0 + (uint32_t)k;
+        uint32_t bits = 0u;
         for (int a = 0; a < p.M; a += 2) {
             double n0, n1;
             normal2(p.seed, gf, g, (uint32_t)(a >> 1), n0, n1);
@@ -140,19 +143,29 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
                 const int i = a + q;
                 const double ex = kn.px - p.anchors.x[i], ey = kn.py - p.anchors.y[i], ez = p.tag_z - p.anchors.z[i];
                 double r = sqrt(ex * ex + ey * ey + ez * ez) + p.sigma_r * (q ? n1 : n0);
-                bool missing = false;
+                bool missing = false, biased = false;
                 if (IMPAIR) {
                     double u, v;
                     uniform2(philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), g, 0x80000000u | (uint32_t)i,
                                            (uint32_t)p.seed, (uint32_t)(p.seed >> 32)), u, v);
                     missing = u < p.p_missing;
-                    if (v < p.p_nlos) r += -p.nlos_mean * log(v / p.p_nlos);
+                    biased = v < p.p_nlos;
+                    if (biased) r += -p.nlos_mean * log(v / p.p_nlos);
                 }
                 const double mm = floor(r * 1000.0);
-                out[((int64_t)k * p.M + i) * N] = (missing || !(mm > 0)) ? (Out)0 : (Out)fmin(mm, lim);
+                const bool absent = missing || !(mm > 0);
+                out[((int64_t)k * p.M + i) * N] = absent ? (Out)0 : (Out)fmin(mm, lim);
+                if (MASK && biased && !absent) bits |= 1u << i;
             }
         }
+        if (MASK) p.nlos[(int64_t)k * N + f] = bits;
     }
+}
+
+template <typename Out, bool MASK>
+static void launch_synth_toa_k(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
+    if (imp) synth_toa_kernel<Out, true, MASK><<<grid, 128, 0, s>>>(p);
+    else synth_toa_kernel<Out, false, MASK><<<grid, 128, 0, s>>>(p);
 }
 
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) {
@@ -160,11 +173,11 @@ cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) 
     const bool imp = p.p_missing > 0 || p.p_nlos > 0;
     const unsigned grid = (unsigned)((p.N + 127) / 128);
     if (u16) {
-        if (imp) synth_toa_kernel<uint16_t, true><<<grid, 128, 0, s>>>(p);
-        else synth_toa_kernel<uint16_t, false><<<grid, 128, 0, s>>>(p);
+        if (p.nlos) launch_synth_toa_k<uint16_t, true>(p, imp, grid, s);
+        else launch_synth_toa_k<uint16_t, false>(p, imp, grid, s);
     } else {
-        if (imp) synth_toa_kernel<int32_t, true><<<grid, 128, 0, s>>>(p);
-        else synth_toa_kernel<int32_t, false><<<grid, 128, 0, s>>>(p);
+        if (p.nlos) launch_synth_toa_k<int32_t, true>(p, imp, grid, s);
+        else launch_synth_toa_k<int32_t, false>(p, imp, grid, s);
     }
     return cudaGetLastError();
 }

@@ -20,6 +20,7 @@ ST_NO_MEAS, ST_ML_FEW, ST_SINGULAR, ST_NAN, ST_ML_NAN, ST_MAXITER, ST_ASYM_R = 1
 ST_Z_GATE = 128
 ST_UNINIT = 256
 HIST_ERR, HIST_ERR_XY, HIST_NEES = 0, 1, 2
+SCORE_COLS = 8  # KFPOS_SCORE_COLS: the columns of kfpos_batch_score_selection
 
 
 class KfposConfig(C.Structure):
@@ -112,6 +113,8 @@ SIGNATURES = {
     "kfpos_batch_set_error_hist": (_I, [_VP, _I, _I, _VP]),
     "kfpos_batch_error_hist": (_I, [_VP, _I64, _VP, _VP]),
     "kfpos_error_hist_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
+    "kfpos_synth_toa_ranges_nlos": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _VP, _VP]),
+    "kfpos_batch_score_selection": (_I, [_VP, _I, _VP, _I, _VP, _VP, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

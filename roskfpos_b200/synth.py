@@ -291,7 +291,7 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
 
 def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED, period=0.1, sigma_r=0.10,
                          p_missing=0.0, p_nlos=0.0, nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None,
-                         want_x0=False, want_truth=False, out=None, stream=None):
+                         want_x0=False, want_truth=False, out=None, stream=None, want_nlos=False):
     """Ranging epochs [epoch0, epoch0 + n_epochs) of the T6 Monte Carlo workload, generated ON THE DEVICE by
     kfpos_synth_toa_ranges (Philox4x32-10; a ranging depends only on seed, the global filter index
     first_filter + f, the global epoch index and the anchor, so sharding and chunking change nothing).  Epoch k
@@ -301,8 +301,10 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
     Returns dict(ranges [n][M][N] on `device`, dt = period, t (host [n]), truth_end [3][N] = the truth at
     t[-1], x0 [6][N] (the truth at t = 0 with zero velocity, a T6 state) if want_x0, truth [n][3][N] (from
-    kfpos_synth_k8_truth, what Batch.set_truth_traj takes for the chunk) if want_truth).  `out` may hold the
-    tensors of a previous chunk of the same shape to be reused.  ML batches take `ranges` row by row."""
+    kfpos_synth_k8_truth, what Batch.set_truth_traj takes for the chunk) if want_truth, nlos [n][N] if want_nlos:
+    the NLOS ground truth of kfpos_synth_toa_ranges_nlos, bit a set where ranging a carries a bias and is present,
+    as int32 holding the uint32 bits).  `out` may hold the tensors of a previous chunk of the same shape to be
+    reused.  ML batches take `ranges` row by row."""
     import ctypes as C
     import torch
     from . import lib as L
@@ -326,9 +328,15 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
                           sigma_r=float(sigma_r), p_missing=float(p_missing), p_nlos=float(p_nlos),
                           nlos_mean=float(nlos_mean))
     sp = None if stream is None else C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
-    L.check(L.lib().kfpos_synth_toa_ranges(dev.index or 0, N, M, C.c_void_p(anc.ctypes.data), n,
-                                           C.c_void_p(t.ctypes.data), C.byref(gen), fmt,
-                                           C.c_void_p(ranges.data_ptr()), sp), "kfpos_synth_toa_ranges")
+    args = (dev.index or 0, N, M, C.c_void_p(anc.ctypes.data), n, C.c_void_p(t.ctypes.data), C.byref(gen), fmt,
+            C.c_void_p(ranges.data_ptr()))
+    nlos = None
+    if want_nlos:
+        nlos = buf("nlos", (n, N), torch.int32)  # torch has no general uint32: the bits of the uint32 masks
+        L.check(L.lib().kfpos_synth_toa_ranges_nlos(*args, C.c_void_p(nlos.data_ptr()), sp),
+                "kfpos_synth_toa_ranges_nlos")
+    else:
+        L.check(L.lib().kfpos_synth_toa_ranges(*args, sp), "kfpos_synth_toa_ranges")
 
     def truth_at(name, times):
         times = np.ascontiguousarray(times, dtype=np.float64)
@@ -338,6 +346,8 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
                                              sp), "kfpos_synth_k8_truth")
         return tr
     res = dict(ranges=ranges, dt=float(period), t=t)
+    if want_nlos:
+        res["nlos"] = nlos
     if want_truth:
         res["truth"] = truth_at("truth", t)
         res["truth_end"] = res["truth"][-1]
@@ -353,7 +363,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
 def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
                    nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
-                   stream=None, hist=None):
+                   stream=None, hist=None, score=False):
     """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
     for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
     truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
@@ -363,7 +373,10 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
     batch.epoch_summary (RMSE(t), ANEES(t)); the truth is unregistered on return.
     hist=(edges, quantity): also a per-epoch histogram (Batch.set_error_hist), read chunk by chunk beside the
     statistics; then returns (rows, counts [n_epochs][len(edges) + 1] uint64), and the histogram is
-    unregistered on return as well."""
+    unregistered on return as well.
+    score=True: each chunk also generates its NLOS mask, the replay writes its selection into a reused device
+    buffer and Batch.score_selection scores it; the [n_epochs][8] uint64 scores (batch.selection_summary) are
+    appended as the last element of the return value, a tuple then."""
     from . import lib as L
     if batch.model != L.MODEL_T6:
         raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
@@ -371,25 +384,34 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
         raise ValueError("toa_montecarlo: n_epochs and chunk must be positive")
     kw = dict(seed=seed, period=period, sigma_r=sigma_r, p_missing=p_missing, p_nlos=p_nlos, nlos_mean=nlos_mean,
               tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream)
-    rows, counts, bufs = [], [], {}
+    rows, counts, scores, bufs = [], [], [], {}
+    sel = None
     if hist is not None:
         batch.set_error_hist(hist[0], hist[1])
     try:
         for k0 in range(0, int(n_epochs), int(chunk)):
             n = min(int(chunk), int(n_epochs) - k0)
             w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
-                                     want_x0=init_state and k0 == 0, out=bufs, **kw)
+                                     want_x0=init_state and k0 == 0, out=bufs, want_nlos=score, **kw)
             if init_state and k0 == 0:
                 batch.set_state(w["x0"], None, stream=stream)
             batch.set_truth_traj(w["truth"], stream=stream)
-            batch.replay_toa(w["dt"], w["ranges"], err=err, stream=stream)
+            if score and (sel is None or sel.shape[0] != n):
+                import torch
+                sel = torch.empty((n, batch.N), dtype=torch.int32, device="cuda:%d" % batch.device)
+            batch.replay_toa(w["dt"], w["ranges"], err=err, sel=sel, stream=stream)
             rows.append(batch.epoch_stats(stream=stream))
             if hist is not None:
                 counts.append(batch.error_hist(stream=stream))
+            if score:
+                scores.append(batch.score_selection(w["ranges"], sel, w["nlos"], stream=stream))
     finally:
         batch.set_truth_traj(None, stream=stream)
         if hist is not None:
             batch.set_error_hist(None)
+    out = (np.concatenate(rows, axis=0),)
     if hist is not None:
-        return np.concatenate(rows, axis=0), np.concatenate(counts, axis=0)
-    return np.concatenate(rows, axis=0)
+        out += (np.concatenate(counts, axis=0),)
+    if score:
+        out += (np.concatenate(scores, axis=0),)
+    return out if len(out) > 1 else out[0]
