@@ -613,6 +613,38 @@ int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_anchors, co
 int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const void *ranges, int fmt, const int32_t *sel,
                                 const uint32_t *nlos, uint64_t *counts, void *stream);
 
+/* Cramer-Rao lower bound of the position per epoch (no reference equivalent; DESIGN §4.5e): the position-error
+ * floor of the rangings of rows [0, n_rows) of a log, for the set `set` of each filter:
+ *   KFPOS_CRLB_PRESENT: the rangings present in the log (value > 0, NaN is not: the scorer's rule);
+ *   KFPOS_CRLB_LOS:     present and not set in the `nlos` mask -- the set a perfect NLOS detector keeps;
+ *   KFPOS_CRLB_USED:    present and kept by the batch's selection, `sel` read exactly as
+ *                       kfpos_batch_score_selection reads it (nothing dropped: plain T6, ML variant 0).
+ * With the true position p (truth, SoA [n_rows][3][N]; ML: [3][N]) and the batch's anchors b_a, the Fisher
+ * information of the epoch is J = sum_{a in S} g_a g_a^T / v_a, g_a = (p - b_a) / |p - b_a|.  D = 3 for T6, T9
+ * and 3-D ML batches; D = 2 for K8 and ML batches with use2d, whose height is known: g_a is then the x-y part of
+ * the same 3-D unit vector.  v_a = var[r][a][f] (SoA [n_rows][n_anchors][N], or NULL: var_scalar) is the TRUE
+ * variance of the ranging noise, not the filters' errorEstimation.  A filter's terms are
+ *   [0] tr J^-1   [1] (J^-1)_xx + (J^-1)_yy   [2] 1   [3] 0
+ * or 0, 0, 0, 1 when it has no bound: |S| < D, a non-finite truth, a v_a (a in S) that is not finite and > 0, a
+ * non-positive or non-finite pivot of the LDL^T of J, or a non-finite trace.  out [n_rows][KFPOS_CRLB_COLS]
+ * doubles (host or device), overwritten: per row the terms summed over the filters in a fixed order -- each 32
+ * filters by the 32-leaf tree of kfpos_batch_epoch_stats, then pairwise over the 32-filter groups -- which
+ * depends on the filter index only: chunks of rows change nothing, and the rows of aligned power-of-two shards
+ * (multiples of 32 filters) added pairwise in rank order equal the whole batch's bit for bit.  sqrt([0] / [2])
+ * is the RMS floor of the epoch.  Reads nothing and changes nothing of the batch's state.  Scratch: 32 B per 32
+ * filters per row, at most 256 MB, kept by the batch.
+ * KFPOS_ERR_INVALID: a bad set, n_rows <= 0, a bad fmt, NULL truth, ranges or out, var NULL with var_scalar not
+ * finite and > 0, KFPOS_CRLB_LOS with a NULL nlos, KFPOS_CRLB_USED with a NULL sel where it is read, n_rows != 1
+ * for ML.  KFPOS_ERR_UNSUPPORTED: KFPOS_CRLB_USED on K8 and T9 batches (they keep no selection).
+ * KFPOS_ERR_NOT_READY: no anchors.                                                                              */
+#define KFPOS_CRLB_PRESENT 0
+#define KFPOS_CRLB_LOS 1
+#define KFPOS_CRLB_USED 2
+#define KFPOS_CRLB_COLS 4
+int kfpos_batch_crlb(kfpos_batch *b, int set, int n_rows, const double *truth, const void *ranges, int fmt,
+                     double var_scalar, const double *var, const int32_t *sel, const uint32_t *nlos, double *out,
+                     void *stream);
+
 /* Accuracy self-test of the kernels' elementary functions (no reference equivalent): evaluates the
  * MUFU-seeded reciprocal and reciprocal square root and the reduced-range sincos on x[0..n) so that
  * a test can compare them with IEEE division / sqrt / libm.  Outputs may be NULL.               */

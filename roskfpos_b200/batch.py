@@ -407,6 +407,35 @@ class Batch:
                                                     _stream_ptr(stream)), "kfpos_batch_score_selection")
         return out
 
+    # ------------------------------------------------------- Cramer-Rao bound
+    _CRLB_SET = {"present": L.CRLB_PRESENT, "los": L.CRLB_LOS, "used": L.CRLB_USED}
+
+    def crlb(self, truth, ranges, var, sel=None, nlos=None, set="present", out=None, readback=True, stream=None):
+        """Per-epoch Cramer-Rao bound of the position (kfpos_batch_crlb) for the rangings of each filter in the set
+        `set`: "present" (in the log), "los" (present and not NLOS in `nlos`) or "used" (kept by this batch's
+        selection `sel`, read as score_selection reads it).  T6 / K8 / T9: truth [T][3][N], ranges [T][M][N], sel
+        [T][N] of replay_toa; ML: truth [3][N], ranges [M][N], sel [2][N] of ml_solve.  var: the true ranging
+        variance in m^2, a scalar or [rows][M][N].  nlos: the masks of synth.toa_montecarlo_chunk(want_nlos=True).
+        Returns [rows][4] sums over the filters (columns in crlb_summary) as float64 numpy; out: a device tensor of
+        that shape to fill asynchronously (returned as given); readback False without `out`: a new device tensor,
+        filled asynchronously."""
+        if set not in self._CRLB_SET:
+            raise ValueError(f"crlb: set must be one of {sorted(self._CRLB_SET)}")
+        rows = 1 if self.model == L.MODEL_ML else int(ranges.shape[0])
+        if out is None and readback:
+            out = np.zeros((rows, L.CRLB_COLS))
+        if out is None:
+            import torch
+            out = torch.empty((rows, L.CRLB_COLS), dtype=torch.float64, device="cuda:%d" % self.device)
+        vs, pv, kv = (float(var), None, None) if np.isscalar(var) else (0.0, *_ptr(var, np.float64))
+        pt, kt = _ptr(truth, np.float64)
+        pr, kr = _ptr(ranges)
+        ps, ks = _ptr(sel, np.int32)
+        pn, kn = _ptr(nlos, np.uint32)
+        L.check(L.lib().kfpos_batch_crlb(self._h, self._CRLB_SET[set], rows, pt, pr, _fmt_of(ranges), vs, pv, ps, pn,
+                                         _ptr(out)[0], _stream_ptr(stream)), "kfpos_batch_crlb")
+        return out
+
 
 def epoch_summary(stats):
     """Per-row summary of epoch_stats / epoch_stats_allreduce output [rows][6]: dict of arrays rmse, rmse_xy
@@ -434,6 +463,33 @@ def selection_summary(counts, n_filters):
             return np.where(den > 0, num / np.where(den > 0, den, 1.0), np.nan)
     return dict(detection=rate(c[:, 3], c[:, 2]), false_drop=rate(c[:, 1] - c[:, 3], c[:, 0] - c[:, 2]),
                 clean=rate(c[:, 5], c[:, 4]), false_alarm=rate(c[:, 7], float(n_filters) - c[:, 4]))
+
+
+def crlb_summary(rows):
+    """Per-row summary of crlb output [rows][4]: dict of arrays rmse_bound = sqrt(mean tr J^-1) and rmse_xy_bound
+    (the RMS position-error floors over the filters with a bound, to set beside epoch_summary's rmse and
+    rmse_xy), n (filters with a bound) and n_none (filters without).  Rows without a bound give NaN."""
+    c = np.asarray(rows, dtype=np.float64).reshape(-1, 4)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        n = c[:, 2]
+        return dict(rmse_bound=np.where(n > 0, np.sqrt(c[:, 0] / n), np.nan),
+                    rmse_xy_bound=np.where(n > 0, np.sqrt(c[:, 1] / n), np.nan), n=n.copy(), n_none=c[:, 3].copy())
+
+
+def rank_tree(rows_per_rank):
+    """The rows of the ranks of a sharded run ([n_ranks][rows][W], rank order: e.g. torch.distributed.all_gather of
+    each rank's crlb output) added by the pairwise tree over the rank index, level by level a[i] += a[i + stride]
+    -- the adds of the library's error_stats_tree, in its order.  With aligned power-of-two shards (multiples of
+    32 filters) the result equals the whole batch's rows bit for bit.  Returns [rows][W]."""
+    a = np.array(rows_per_rank, dtype=np.float64)
+    if a.ndim < 2 or a.shape[0] == 0:
+        raise ValueError("rank_tree: expects [n_ranks][rows][W] with at least one rank")
+    stride = 1
+    while stride < a.shape[0]:
+        i = np.arange(0, a.shape[0] - stride, 2 * stride)
+        a[i] = a[i] + a[i + stride]
+        stride *= 2
+    return a[0]
 
 
 def hist_quantiles(counts, edges, q):

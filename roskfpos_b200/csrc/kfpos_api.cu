@@ -88,6 +88,7 @@ struct kfpos_batch {
     double *d_eh_edges = nullptr;
     unsigned long long *d_eh_counts = nullptr;
     DevBuf eh_gather;
+    DevBuf crlb; // per-warp partials of kfpos_batch_crlb, [rows][n_warps][4], at most 256 MB
     // K8 / T9 latched sensor samples, SoA rows (see kfpos_k8.cuh)
     double *d_latch = nullptr;
     double *d_latch_u = nullptr; // batch-wide latched IMU covariances
@@ -467,6 +468,7 @@ extern "C" void kfpos_batch_destroy(kfpos_batch *b) {
     cudaFree(b->d_eh_edges);
     cudaFree(b->d_eh_counts);
     b->eh_gather.release();
+    b->crlb.release();
     cudaFree(b->d_latch);
     cudaFree(b->d_has);
     cudaFree(b->d_latch_u);
@@ -1650,6 +1652,15 @@ extern "C" int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_
     return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, fmt, ranges, nlos, stream);
 }
 
+namespace {
+// how the selection of a T6 or ML batch is read from `sel` (used_mask): as the replay (T6) or the solve (ML, row 0
+// of its [2][N]) wrote it
+int sel_mode(const kfpos_batch *b) {
+    const bool variant = b->cfg.variant == 1 || b->cfg.variant == 2;
+    return variant ? SCORE_MASK : (b->model != KFPOS_MODEL_ML && b->cfg.ignore_worst_anchor) ? SCORE_LOO : SCORE_NONE;
+}
+} // namespace
+
 extern "C" int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const void *ranges, int fmt, const int32_t *sel,
                                            const uint32_t *nlos, uint64_t *counts, void *stream) {
     static_assert(KFPOS_SCORE_COLS == SCORE_COLS, "one column count");
@@ -1658,9 +1669,7 @@ extern "C" int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const voi
     const bool ml = b->model == KFPOS_MODEL_ML;
     if (n_rows <= 0 || !fmt_ok(fmt) || !ranges || !counts || (ml && n_rows != 1)) return KFPOS_ERR_INVALID;
     if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
-    // how `sel` is read: as the replay (T6) or the solve (ML, row 0 of its [2][N]) wrote it
-    const bool variant = b->cfg.variant == 1 || b->cfg.variant == 2;
-    const int mode = variant ? SCORE_MASK : (!ml && b->cfg.ignore_worst_anchor) ? SCORE_LOO : SCORE_NONE;
+    const int mode = sel_mode(b);
     if (mode != SCORE_NONE && !sel) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
@@ -1675,6 +1684,60 @@ extern "C" int kfpos_batch_score_selection(kfpos_batch *b, int n_rows, const voi
     p.N = b->N; p.n_rows = n_rows; p.M = (int)M; p.fmt = fmt; p.mode = mode;
     CK(cudaMemsetAsync(p.counts, 0, sizeof(uint64_t) * SCORE_COLS * R, s));
     CK(launch_score_selection(p, s));
+    return st.finish();
+}
+
+extern "C" int kfpos_batch_crlb(kfpos_batch *b, int set, int n_rows, const double *truth, const void *ranges, int fmt,
+                                double var_scalar, const double *var, const int32_t *sel, const uint32_t *nlos,
+                                double *out, void *stream) {
+    static_assert(KFPOS_CRLB_COLS == CRLB_W && KFPOS_CRLB_PRESENT == CRLB_PRESENT && KFPOS_CRLB_LOS == CRLB_LOS &&
+                  KFPOS_CRLB_USED == CRLB_USED, "one set of constants");
+    if (!b) return KFPOS_ERR_INVALID;
+    const bool ml = b->model == KFPOS_MODEL_ML;
+    if (set < KFPOS_CRLB_PRESENT || set > KFPOS_CRLB_USED || n_rows <= 0 || !fmt_ok(fmt) || !truth || !ranges ||
+        !out || (!var && !(var_scalar > 0.0 && var_scalar < INFINITY)) || (set == KFPOS_CRLB_LOS && !nlos) ||
+        (ml && n_rows != 1))
+        return KFPOS_ERR_INVALID;
+    if (set == KFPOS_CRLB_USED && (b->model == KFPOS_MODEL_K8 || b->model == KFPOS_MODEL_T9))
+        return KFPOS_ERR_UNSUPPORTED;
+    if (!b->have_anchors) return KFPOS_ERR_NOT_READY;
+    const int mode = set == KFPOS_CRLB_USED ? sel_mode(b) : SCORE_NONE;
+    if (mode != SCORE_NONE && !sel) return KFPOS_ERR_INVALID;
+    DeviceGuard g(b->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t W = (b->N + 31) / 32;
+    const size_t N = (size_t)b->N, M = (size_t)b->anchors.n, R = (size_t)n_rows;
+    const size_t row_bytes = sizeof(double) * CRLB_W * (size_t)W;
+    // the per-warp partials of a batch of rows, folded before the next batch: at most 256 MB of scratch
+    int64_t batch_rows = (int64_t)(((size_t)256 << 20) / row_bytes);
+    if (batch_rows < 1) batch_rows = 1;
+    if (batch_rows > n_rows) batch_rows = n_rows;
+    CK(b->crlb.reserve(row_bytes * (size_t)batch_rows));
+    Staging st(b, s);
+    CrlbParams p;
+    p.anchors = b->anchors;
+    const double *d_truth = st.in(truth, sizeof(double) * 3 * N * R);
+    const char *d_ranges = (const char *)st.in(ranges, fmt_size(fmt) * M * N * R);
+    const double *d_var = st.in(var, sizeof(double) * M * N * R);
+    const int32_t *d_sel = mode == SCORE_NONE ? nullptr : st.in(sel, sizeof(int32_t) * N * R);
+    const uint32_t *d_nlos = set == KFPOS_CRLB_LOS ? st.in(nlos, sizeof(uint32_t) * N * R) : nullptr;
+    double *d_out = st.out(out, sizeof(double) * CRLB_W * R);
+    if (st.rc) return st.rc;
+    p.partials = (double *)b->crlb.p;
+    p.w_scalar = var ? 0.0 : 1.0 / var_scalar;
+    p.N = b->N; p.n_warps = W; p.M = (int)M; p.fmt = fmt; p.set = set; p.sel_mode = mode;
+    p.dim = b->model == KFPOS_MODEL_K8 || (ml && b->cfg.use2d) ? 2 : 3;
+    for (int64_t r0 = 0; r0 < n_rows; r0 += batch_rows) {
+        const size_t o = (size_t)r0 * N;
+        p.n_rows = n_rows - r0 < batch_rows ? n_rows - r0 : batch_rows;
+        p.truth = d_truth + 3 * o;
+        p.ranges = d_ranges + fmt_size(fmt) * M * o;
+        p.var = d_var ? d_var + M * o : nullptr;
+        p.sel = d_sel ? d_sel + o : nullptr;
+        p.nlos = d_nlos ? d_nlos + o : nullptr;
+        CK(launch_crlb(p, s));
+        CK(launch_stats_tree(CRLB_W, p.n_rows, W, p.partials, p.partials, W * CRLB_W, CRLB_W, d_out + r0 * CRLB_W, s));
+    }
     return st.finish();
 }
 

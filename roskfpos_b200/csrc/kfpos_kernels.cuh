@@ -99,24 +99,26 @@ KF_DEV void epoch_terms_zero(const Col &out) {
 #pragma unroll
     for (int q = 0; q < ES_W; ++q) out[q] = 0.0;
 }
-// the warp's sum of the 6 terms in `v` (every lane of wmask calls it; wmask = the lanes with a filter, a prefix)
+// the warp's sum of the W terms in `v` (every lane of wmask calls it; wmask = the lanes with a filter, a prefix);
+// W = 4: the Cramer-Rao terms of kfpos_crlb.cu
+template <int W = ES_W>
 KF_DEV void epoch_stats_flush(const Col &v, unsigned wmask, double *out) {
     const int lane = threadIdx.x & 31;
-    double a[ES_W];
+    double a[W];
 #pragma unroll
-    for (int q = 0; q < ES_W; ++q) a[q] = v[q];
+    for (int q = 0; q < W; ++q) a[q] = v[q];
 #pragma unroll
     for (int s = 16; s > 0; s >>= 1) {
         const bool has = lane + s < 32 && ((wmask >> (lane + s)) & 1u);
 #pragma unroll
-        for (int q = 0; q < ES_W; ++q) {
+        for (int q = 0; q < W; ++q) {
             const double o = __shfl_down_sync(wmask, a[q], s);
             a[q] += has ? o : 0.0;
         }
     }
     if (lane == 0) {
 #pragma unroll
-        for (int q = 0; q < ES_W; ++q) out[q] = a[q];
+        for (int q = 0; q < W; ++q) out[q] = a[q];
     }
 }
 
@@ -467,6 +469,56 @@ struct ScoreParams {
     int M, fmt, mode;
 };
 cudaError_t launch_score_selection(const ScoreParams &p, cudaStream_t s);
+
+// The rangings of filter f in one epoch of a SoA log: bit a set when ranging a is present, the replay's rule of
+// convert_epoch (value > 0; NaN is not).  base = the index of (row, anchor 0, f), m anchors of stride N.
+template <int FMT>
+KF_DEV unsigned present_mask(const void *ranges, int64_t base, int m, int64_t N) {
+    unsigned present = 0u;
+#pragma unroll 8
+    for (int a = 0; a < m; ++a) {
+        const int64_t i = base + (int64_t)a * N;
+        bool on;
+        if (FMT == 0) on = __ldg(reinterpret_cast<const double *>(ranges) + i) > 0.0; // false for NaN
+        else if (FMT == 1) on = __ldg(reinterpret_cast<const int32_t *>(ranges) + i) > 0;
+        else on = __ldg(reinterpret_cast<const uint16_t *>(ranges) + i) != 0;
+        present |= (unsigned)on << a;
+    }
+    return present;
+}
+// The rangings filter f kept in row r, decoded from `sel` (SoA [rows][N]) as the batch's configuration wrote it
+// (mode SCORE_*): the one place that reads a selection, for the scorer and the Cramer-Rao bound alike.  May name
+// absent slots (SCORE_MASK).
+KF_DEV unsigned used_mask(unsigned present, const int32_t *sel, int64_t r, int64_t N, int64_t f, int mode) {
+    unsigned used = present;
+    if (mode == SCORE_LOO) {
+        const int s = __ldg(sel + r * N + f);
+        if (s >= 0 && s < 32) used &= ~(1u << s);
+    } else if (mode == SCORE_MASK) {
+        used = (unsigned)__ldg(sel + r * N + f);
+    }
+    return used;
+}
+
+// Cramer-Rao bound of the position per epoch (kfpos_crlb.cu, kfpos_batch_crlb): for each (filter, row) the four
+// terms {tr J^-1, (J^-1)_xx + (J^-1)_yy, 1, 0} (or {0, 0, 0, 1} without a bound) of the Fisher information J of
+// the set `set` (KFPOS_CRLB_*), summed per 32-filter warp by epoch_stats_flush<4> into
+// partials[(row * n_warps + f / 32) * 4]; the caller folds them over the warp index with launch_stats_tree(4, ...).
+constexpr int CRLB_W = 4;
+enum { CRLB_PRESENT = 0, CRLB_LOS = 1, CRLB_USED = 2 };
+struct CrlbParams {
+    AnchorTable anchors;
+    const double *truth;  // SoA [n_rows][3][N]
+    const void *ranges;   // SoA [n_rows][M][N] in fmt
+    const double *var;    // SoA [n_rows][M][N] true ranging variances, or null: 1 / w_scalar for all
+    const int32_t *sel;   // SoA [n_rows][N] read with sel_mode (KFPOS_CRLB_USED), else null
+    const uint32_t *nlos; // SoA [n_rows][N] (KFPOS_CRLB_LOS), else null
+    double *partials;     // [n_rows][n_warps][4]
+    double w_scalar;      // 1 / var_scalar
+    int64_t N, n_rows, n_warps;
+    int M, fmt, set, sel_mode, dim; // dim: 3, or 2 (K8, ML use2d: x-y information, known height)
+};
+cudaError_t launch_crlb(const CrlbParams &p, cudaStream_t s);
 
 // DFMA-only microbenchmark on the current device (the FP64 roofline denominator)
 cudaError_t measure_fp64_peak(double *flops_per_s);

@@ -16,21 +16,6 @@ constexpr int SCORE_BLOCK = 256;
 constexpr int SCORE_WARPS = SCORE_BLOCK / 32;
 
 template <int FMT>
-__device__ __forceinline__ unsigned present_mask(const void *ranges, int64_t base, int m, int64_t N) {
-    unsigned present = 0u;
-#pragma unroll 8
-    for (int a = 0; a < m; ++a) {
-        const int64_t i = base + (int64_t)a * N;
-        bool on;
-        if (FMT == 0) on = __ldg(reinterpret_cast<const double *>(ranges) + i) > 0.0; // false for NaN
-        else if (FMT == 1) on = __ldg(reinterpret_cast<const int32_t *>(ranges) + i) > 0;
-        else on = __ldg(reinterpret_cast<const uint16_t *>(ranges) + i) != 0;
-        present |= (unsigned)on << a;
-    }
-    return present;
-}
-
-template <int FMT>
 __global__ void __launch_bounds__(SCORE_BLOCK) score_selection_kernel(const ScoreParams p) {
     __shared__ unsigned part[SCORE_WARPS][SCORE_COLS];
     const int64_t N = p.N, r = blockIdx.x;
@@ -40,13 +25,7 @@ __global__ void __launch_bounds__(SCORE_BLOCK) score_selection_kernel(const Scor
         unsigned c[SCORE_COLS] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
         if (f < N) {
             const unsigned present = present_mask<FMT>(p.ranges, r * p.M * N + f, p.M, N);
-            unsigned used = present;
-            if (p.mode == SCORE_LOO) {
-                const int s = __ldg(p.sel + r * N + f);
-                if (s >= 0 && s < 32) used &= ~(1u << s);
-            } else if (p.mode == SCORE_MASK) {
-                used = (unsigned)__ldg(p.sel + r * N + f);
-            }
+            const unsigned used = used_mask(present, p.sel, r, N, f, p.mode);
             const unsigned dropped = present & ~used;
             const unsigned nl = p.nlos ? __ldg(p.nlos + r * N + f) & present : 0u;
             c[0] = __popc(present);

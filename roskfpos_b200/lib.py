@@ -21,6 +21,8 @@ ST_Z_GATE = 128
 ST_UNINIT = 256
 HIST_ERR, HIST_ERR_XY, HIST_NEES = 0, 1, 2
 SCORE_COLS = 8  # KFPOS_SCORE_COLS: the columns of kfpos_batch_score_selection
+CRLB_PRESENT, CRLB_LOS, CRLB_USED = 0, 1, 2
+CRLB_COLS = 4  # KFPOS_CRLB_COLS: the columns of kfpos_batch_crlb
 
 
 class KfposConfig(C.Structure):
@@ -115,6 +117,7 @@ SIGNATURES = {
     "kfpos_error_hist_allreduce": (_I, [_VP, _VP, _I64, _VP, _VP]),
     "kfpos_synth_toa_ranges_nlos": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _VP, _VP]),
     "kfpos_batch_score_selection": (_I, [_VP, _I, _VP, _I, _VP, _VP, _VP, _VP]),
+    "kfpos_batch_crlb": (_I, [_VP, _I, _I, _VP, _VP, _I, _D, _VP, _VP, _VP, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

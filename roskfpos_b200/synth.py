@@ -363,7 +363,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
 def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
                    nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
-                   stream=None, hist=None, score=False):
+                   stream=None, hist=None, score=False, *, crlb=None):
     """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
     for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
     truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
@@ -376,7 +376,11 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
     unregistered on return as well.
     score=True: each chunk also generates its NLOS mask, the replay writes its selection into a reused device
     buffer and Batch.score_selection scores it; the [n_epochs][8] uint64 scores (batch.selection_summary) are
-    appended as the last element of the return value, a tuple then."""
+    appended as the last element of the return value, a tuple then.
+    crlb=("present", "los", "used") or any of them: each chunk also calls Batch.crlb for each set with its truth,
+    log, NLOS mask and selection, at the generator's ranging variance sigma_r^2 + (1 mm)^2 / 12 (its noise and its
+    floor to whole millimetres); a dict {set: [n_epochs][4]} (batch.crlb_summary) is appended as the last element
+    of the return value, a tuple then."""
     from . import lib as L
     if batch.model != L.MODEL_T6:
         raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
@@ -384,6 +388,10 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
         raise ValueError("toa_montecarlo: n_epochs and chunk must be positive")
     kw = dict(seed=seed, period=period, sigma_r=sigma_r, p_missing=p_missing, p_nlos=p_nlos, nlos_mean=nlos_mean,
               tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream)
+    crlb = (crlb,) if isinstance(crlb, str) else tuple(crlb or ())
+    bounds = {name: [] for name in crlb}
+    want_sel, want_nlos = score or "used" in crlb, score or "los" in crlb
+    var = float(sigma_r) ** 2 + 1e-6 / 12.0
     rows, counts, scores, bufs = [], [], [], {}
     sel = None
     if hist is not None:
@@ -392,11 +400,11 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
         for k0 in range(0, int(n_epochs), int(chunk)):
             n = min(int(chunk), int(n_epochs) - k0)
             w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
-                                     want_x0=init_state and k0 == 0, out=bufs, want_nlos=score, **kw)
+                                     want_x0=init_state and k0 == 0, out=bufs, want_nlos=want_nlos, **kw)
             if init_state and k0 == 0:
                 batch.set_state(w["x0"], None, stream=stream)
             batch.set_truth_traj(w["truth"], stream=stream)
-            if score and (sel is None or sel.shape[0] != n):
+            if want_sel and (sel is None or sel.shape[0] != n):
                 import torch
                 sel = torch.empty((n, batch.N), dtype=torch.int32, device="cuda:%d" % batch.device)
             batch.replay_toa(w["dt"], w["ranges"], err=err, sel=sel, stream=stream)
@@ -405,6 +413,9 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
                 counts.append(batch.error_hist(stream=stream))
             if score:
                 scores.append(batch.score_selection(w["ranges"], sel, w["nlos"], stream=stream))
+            for name in crlb:
+                bounds[name].append(batch.crlb(w["truth"], w["ranges"], var, sel, w.get("nlos"), set=name,
+                                               stream=stream))
     finally:
         batch.set_truth_traj(None, stream=stream)
         if hist is not None:
@@ -414,4 +425,6 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
         out += (np.concatenate(counts, axis=0),)
     if score:
         out += (np.concatenate(scores, axis=0),)
+    if crlb:
+        out += ({name: np.concatenate(b, axis=0) for name, b in bounds.items()},)
     return out if len(out) > 1 else out[0]
