@@ -582,6 +582,39 @@ int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_anchors, co
                                 int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
                                 void *ranges, uint32_t *nlos, void *stream);
 
+/* Obstacle-based NLOS (DESIGN §4.5f): the log of kfpos_synth_toa_ranges in a room with axis-aligned boxes that
+ * bias or remove the rangings whose direct path crosses them.  For the ranging of filter gf, epoch g and anchor
+ * a, with truth T = (x, y, tag_z), anchor A and Dv = A - T, the segment T + s Dv, s in [0, 1], meets box o when
+ * the slab test gives enter < exit: enter = 0, exit = 1, and per axis i with Dv_i != 0 (inv_i = 1 / Dv_i)
+ *   s1 = (lo_i - T_i) inv_i, s2 = (hi_i - T_i) inv_i, enter = max(enter, min(s1, s2)), exit = min(exit, max(s1, s2));
+ * an axis with Dv_i == 0 lets the box block only when lo_i < T_i < hi_i.  Boxes are open: a segment that only
+ * touches a face is not blocked.  Every step is one IEEE operation, so a host reproduces the decision exactly
+ * from the truth of kfpos_synth_k8_truth.  L_o = (exit - enter) d_a is the length of the path inside box o.
+ * When at least one box blocks the ranging, after the noise and the i.i.d. bias of kfpos_synth_toa_ranges:
+ *   r += sum_o excess_per_m_o L_o over the blocking boxes, in box order;
+ *   (u, v) = two uniforms of the counter (gf, g, 0x40000000 | a);
+ *   the ranging is absent when u < 1 - prod_o (1 - p_loss_o) (blocking boxes, in box order);
+ *   r += -S log(v) when S = sum_o spread_o > 0 (an exponential of mean S).
+ * Then mm = floor(r * 1000) as before; the ranging is absent when missing, lost or mm <= 0.  nlos (or NULL):
+ * bit a set when ranging a drew an i.i.d. bias OR was blocked, and is present -- a blocked ranging with no
+ * bias is NLOS too, its direct path is obstructed.  n_obstacles == 0, or boxes that block nothing, give the
+ * log and mask of kfpos_synth_toa_ranges / _nlos byte for byte.  obstacles: HOST array, copied before the call
+ * returns.  Errors and the sync rule are kfpos_synth_toa_ranges's; KFPOS_ERR_INVALID also for n_obstacles
+ * outside [0, KFPOS_MAX_OBSTACLES], NULL obstacles with n_obstacles > 0, a non-finite corner, !(lo < hi) on an
+ * axis, excess_per_m or spread negative or not finite, p_loss outside [0, 1].                                 */
+typedef struct kfpos_obstacle {
+    double lo[3], hi[3];  /* box corners, m; lo < hi on every axis                                     */
+    double excess_per_m;  /* range excess per metre of direct path inside the box, >= 0 (a dielectric
+                             slab of permittivity eps_r delays by (sqrt(eps_r) - 1) per metre)          */
+    double spread;        /* mean of an exponential bias added when the box blocks the ranging, m, >= 0 */
+    double p_loss;        /* probability that a ranging this box blocks is absent, [0, 1]               */
+} kfpos_obstacle;
+#define KFPOS_MAX_OBSTACLES 32
+int kfpos_synth_toa_ranges_geo(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                               int n_epochs, const double *t, const kfpos_synth_toa *gen,
+                               int n_obstacles, const kfpos_obstacle *obstacles, int fmt,
+                               void *ranges, uint32_t *nlos, void *stream);
+
 /* NLOS detection scores of a ranging selection (no reference equivalent; DESIGN §4.5d): how the selection of
  * rows [0, n_rows) of a log this batch has just replayed (T6, kfpos_batch_replay_toa) or solved (ML,
  * kfpos_batch_ml_solve) compares with the NLOS truth.  ranges: the log, SoA [n_rows][n_anchors][N] in any fmt; a

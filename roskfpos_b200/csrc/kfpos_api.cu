@@ -1597,9 +1597,13 @@ extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first
 }
 
 namespace {
-// kfpos_synth_toa_ranges with an optional NLOS mask output (kfpos_synth_toa_ranges_nlos)
+// kfpos_synth_toa_ranges with an optional NLOS mask output (kfpos_synth_toa_ranges_nlos) and optional obstacles
+// (kfpos_synth_toa_ranges_geo)
 int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz, int n_epochs,
-                     const double *t, const kfpos_synth_toa *gen, int fmt, void *ranges, uint32_t *nlos, void *stream) {
+                     const double *t, const kfpos_synth_toa *gen, int n_obstacles, const kfpos_obstacle *obstacles,
+                     int fmt, void *ranges, uint32_t *nlos, void *stream) {
+    static_assert(sizeof(kfpos_obstacle) == sizeof(SynthObstacle) && KFPOS_MAX_OBSTACLES == SYNTH_TOA_OBSTACLES,
+                  "the kernel's obstacle table mirrors kfpos_obstacle");
     const auto prob = [](double q) { return q >= 0.0 && q <= 1.0; }; // false for NaN
     if (n_filters <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || !anchors_xyz || n_epochs < 0 ||
         (n_epochs > 0 && (!t || !ranges)) || !gen || (fmt != KFPOS_FMT_I32_MM && fmt != KFPOS_FMT_U16_MM))
@@ -1608,6 +1612,16 @@ int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double 
         (gen->p_nlos > 0.0 && !(gen->nlos_mean > 0.0)) || gen->first_filter < 0 || gen->first_epoch < 0 ||
         gen->first_epoch + n_epochs > (int64_t)0xFFFFFFFF) // epoch index 0xFFFFFFFF: the per-filter constants
         return KFPOS_ERR_INVALID;
+    if (n_obstacles < 0 || n_obstacles > KFPOS_MAX_OBSTACLES || (n_obstacles > 0 && !obstacles))
+        return KFPOS_ERR_INVALID;
+    for (int o = 0; o < n_obstacles; ++o) {
+        const kfpos_obstacle &b = obstacles[o];
+        for (int j = 0; j < 3; ++j)
+            if (!std::isfinite(b.lo[j]) || !std::isfinite(b.hi[j]) || !(b.lo[j] < b.hi[j])) return KFPOS_ERR_INVALID;
+        if (!(b.excess_per_m >= 0.0) || !std::isfinite(b.excess_per_m) || !(b.spread >= 0.0) ||
+            !std::isfinite(b.spread) || !prob(b.p_loss))
+            return KFPOS_ERR_INVALID;
+    }
     if (int rc = check_device(device)) return rc;
     if (n_epochs == 0) return KFPOS_OK;
     DeviceGuard g(device);
@@ -1627,6 +1641,8 @@ int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double 
     p.N = n_filters; p.filter0 = gen->first_filter; p.seed = gen->seed; p.M = n_anchors;
     p.tag_z = gen->tag_z; p.sigma_r = gen->sigma_r; p.p_missing = gen->p_missing; p.p_nlos = gen->p_nlos;
     p.nlos_mean = gen->nlos_mean;
+    p.n_obstacles = n_obstacles;
+    if (n_obstacles > 0) memcpy(p.obstacles, obstacles, sizeof(kfpos_obstacle) * (size_t)n_obstacles);
     for (int k0 = 0; k0 < n_epochs; k0 += SYNTH_TOA_T) {
         p.n_epochs = n_epochs - k0 < SYNTH_TOA_T ? n_epochs - k0 : SYNTH_TOA_T;
         p.epoch0 = (uint32_t)(gen->first_epoch + k0);
@@ -1642,14 +1658,24 @@ int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double 
 extern "C" int kfpos_synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
                                       int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
                                       void *ranges, void *stream) {
-    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, fmt, ranges, nullptr, stream);
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, 0, nullptr, fmt, ranges,
+                            nullptr, stream);
 }
 
 extern "C" int kfpos_synth_toa_ranges_nlos(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
                                            int n_epochs, const double *t, const kfpos_synth_toa *gen, int fmt,
                                            void *ranges, uint32_t *nlos, void *stream) {
     if (!nlos) return KFPOS_ERR_INVALID;
-    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, fmt, ranges, nlos, stream);
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, 0, nullptr, fmt, ranges, nlos,
+                            stream);
+}
+
+extern "C" int kfpos_synth_toa_ranges_geo(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                          int n_epochs, const double *t, const kfpos_synth_toa *gen, int n_obstacles,
+                                          const kfpos_obstacle *obstacles, int fmt, void *ranges, uint32_t *nlos,
+                                          void *stream) {
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, n_obstacles, obstacles, fmt,
+                            ranges, nlos, stream);
 }
 
 namespace {

@@ -442,6 +442,10 @@ cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s);
 // ranging epochs of the same truth for [T][M][N] range logs (kfpos_synth_toa_ranges); a launch covers at most
 // SYNTH_TOA_T epochs, whose times travel in the parameter block (8 KB of the 32 KB it may hold)
 constexpr int SYNTH_TOA_T = 1024;
+constexpr int SYNTH_TOA_OBSTACLES = 32; // KFPOS_MAX_OBSTACLES
+struct SynthObstacle {                  // kfpos_obstacle
+    double lo[3], hi[3], excess_per_m, spread, p_loss;
+};
 struct SynthToaParams {
     AnchorTable anchors;
     int64_t N, filter0;
@@ -452,6 +456,8 @@ struct SynthToaParams {
     void *ranges; // SoA [n_epochs][M][N], int32 or uint16 mm
     double t[SYNTH_TOA_T];
     uint32_t *nlos; // SoA [n_epochs][N] NLOS bit masks, or null (last: the offsets of the fields above stay)
+    int n_obstacles; // boxes of kfpos_synth_toa_ranges_geo, 0: none (after the fields above, which keep their offsets)
+    SynthObstacle obstacles[SYNTH_TOA_OBSTACLES];
 };
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s); // u16: uint16 mm, else int32 mm
 

@@ -5,7 +5,8 @@
 // tensors the replay kernel streams -- a 64 M-filter x 1000-step run never has its inputs resident (they
 // would be 280 GB), only the chunk in flight.
 // synth_toa_kernel: ranging epochs for every consumer of a [T][M][N] millimetre range log (T6 / K8 / T9
-// ranging replays, the ML batch), with optional missing rangings and exponential NLOS biases (DESIGN §4.5c).
+// ranging replays, the ML batch), with optional missing rangings and exponential NLOS biases (DESIGN §4.5c), and
+// optional boxes in the room that bias or remove the rangings whose direct path crosses them (DESIGN §4.5f).
 //
 // Every value is a pure function of (seed, global filter index, event index, sample index) through
 // the counter-based Philox4x32-10 generator (Salmon et al., SC'11; kfpos_synth.cuh), so a filter's stream
@@ -120,9 +121,12 @@ cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s) {
 //   mm = floor((d_a + sigma_r n_a + bias) * 1000), 0 ("no ranging", TOA.cpp:50) when missing or <= 0.
 // MASK: also the NLOS truth, SoA [k][N] uint32 with bit a set when ranging a drew a bias and was written (> 0),
 // gathered in a register and stored once per epoch (kfpos_synth_toa_ranges_nlos).
+// GEO: the boxes of kfpos_synth_toa_ranges_geo (DESIGN §4.5f).  The slab test of the segment truth -> anchor uses
+// only single IEEE operations (no contraction), so a host reproduces every decision from the device truth; the
+// Philox draw (gf, g, 0x40000000 | a) of the loss and the exponential bias is made for blocked rangings only.
 // The epoch times and the anchors are read from the parameter block: every lane reads the same one at the
 // same time (constant-bank broadcast).  Stores: SoA [k][a][N], filter index fastest -- coalesced.
-template <typename Out, bool IMPAIR, bool MASK = false>
+template <typename Out, bool IMPAIR, bool MASK = false, bool GEO = false>
 __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
     if (f >= p.N) return;
@@ -142,7 +146,8 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
             for (int q = 0; q < 2 && a + q < p.M; ++q) {
                 const int i = a + q;
                 const double ex = kn.px - p.anchors.x[i], ey = kn.py - p.anchors.y[i], ez = p.tag_z - p.anchors.z[i];
-                double r = sqrt(ex * ex + ey * ey + ez * ez) + p.sigma_r * (q ? n1 : n0);
+                const double d = sqrt(ex * ex + ey * ey + ez * ez);
+                double r = d + p.sigma_r * (q ? n1 : n0);
                 bool missing = false, biased = false;
                 if (IMPAIR) {
                     double u, v;
@@ -151,6 +156,47 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
                     missing = u < p.p_missing;
                     biased = v < p.p_nlos;
                     if (biased) r += -p.nlos_mean * log(v / p.p_nlos);
+                }
+                if (GEO) {
+                    const double tp[3] = {kn.px, kn.py, p.tag_z};
+                    const double dv[3] = {__dsub_rn(p.anchors.x[i], kn.px), __dsub_rn(p.anchors.y[i], kn.py),
+                                          __dsub_rn(p.anchors.z[i], p.tag_z)};
+                    double inv[3];
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) inv[j] = __ddiv_rn(1.0, dv[j]);
+                    bool blocked = false;
+                    double excess = 0.0, spread = 0.0, keep = 1.0;
+                    for (int o = 0; o < p.n_obstacles; ++o) {
+                        const SynthObstacle &b = p.obstacles[o];
+                        double enter = 0.0, exit = 1.0;
+                        bool inside = true; // every axis with dv == 0 has the truth strictly between the faces
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) {
+                            if (dv[j] != 0.0) {
+                                const double s1 = __dmul_rn(__dsub_rn(b.lo[j], tp[j]), inv[j]);
+                                const double s2 = __dmul_rn(__dsub_rn(b.hi[j], tp[j]), inv[j]);
+                                enter = fmax(enter, fmin(s1, s2));
+                                exit = fmin(exit, fmax(s1, s2));
+                            } else {
+                                inside = inside && b.lo[j] < tp[j] && tp[j] < b.hi[j];
+                            }
+                        }
+                        if (inside && enter < exit) {
+                            blocked = true;
+                            excess += b.excess_per_m * ((exit - enter) * d);
+                            spread += b.spread;
+                            keep *= 1.0 - b.p_loss;
+                        }
+                    }
+                    if (blocked) {
+                        double u, v;
+                        uniform2(philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), g, 0x40000000u | (uint32_t)i,
+                                               (uint32_t)p.seed, (uint32_t)(p.seed >> 32)), u, v);
+                        r += excess;
+                        missing = missing || u < 1.0 - keep;
+                        if (spread > 0.0) r += -spread * log(v);
+                        biased = true;
+                    }
                 }
                 const double mm = floor(r * 1000.0);
                 const bool absent = missing || !(mm > 0);
@@ -162,10 +208,16 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
     }
 }
 
-template <typename Out, bool MASK>
+template <typename Out, bool MASK, bool GEO>
 static void launch_synth_toa_k(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
-    if (imp) synth_toa_kernel<Out, true, MASK><<<grid, 128, 0, s>>>(p);
-    else synth_toa_kernel<Out, false, MASK><<<grid, 128, 0, s>>>(p);
+    if (imp) synth_toa_kernel<Out, true, MASK, GEO><<<grid, 128, 0, s>>>(p);
+    else synth_toa_kernel<Out, false, MASK, GEO><<<grid, 128, 0, s>>>(p);
+}
+
+template <typename Out, bool GEO>
+static void launch_synth_toa_m(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
+    if (p.nlos) launch_synth_toa_k<Out, true, GEO>(p, imp, grid, s);
+    else launch_synth_toa_k<Out, false, GEO>(p, imp, grid, s);
 }
 
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) {
@@ -173,11 +225,11 @@ cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) 
     const bool imp = p.p_missing > 0 || p.p_nlos > 0;
     const unsigned grid = (unsigned)((p.N + 127) / 128);
     if (u16) {
-        if (p.nlos) launch_synth_toa_k<uint16_t, true>(p, imp, grid, s);
-        else launch_synth_toa_k<uint16_t, false>(p, imp, grid, s);
+        if (p.n_obstacles > 0) launch_synth_toa_m<uint16_t, true>(p, imp, grid, s);
+        else launch_synth_toa_m<uint16_t, false>(p, imp, grid, s);
     } else {
-        if (p.nlos) launch_synth_toa_k<int32_t, true>(p, imp, grid, s);
-        else launch_synth_toa_k<int32_t, false>(p, imp, grid, s);
+        if (p.n_obstacles > 0) launch_synth_toa_m<int32_t, true>(p, imp, grid, s);
+        else launch_synth_toa_m<int32_t, false>(p, imp, grid, s);
     }
     return cudaGetLastError();
 }

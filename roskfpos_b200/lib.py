@@ -23,6 +23,7 @@ HIST_ERR, HIST_ERR_XY, HIST_NEES = 0, 1, 2
 SCORE_COLS = 8  # KFPOS_SCORE_COLS: the columns of kfpos_batch_score_selection
 CRLB_PRESENT, CRLB_LOS, CRLB_USED = 0, 1, 2
 CRLB_COLS = 4  # KFPOS_CRLB_COLS: the columns of kfpos_batch_crlb
+MAX_OBSTACLES = 32  # KFPOS_MAX_OBSTACLES: the boxes of kfpos_synth_toa_ranges_geo
 
 
 class KfposConfig(C.Structure):
@@ -63,6 +64,12 @@ class KfposSynthToa(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("first_filter", C.c_int64), ("first_epoch", C.c_int64),
                 ("tag_z", C.c_double), ("sigma_r", C.c_double), ("p_missing", C.c_double), ("p_nlos", C.c_double),
                 ("nlos_mean", C.c_double)]
+
+
+class KfposObstacle(C.Structure):
+    """kfpos_obstacle: an axis-aligned box of kfpos_synth_toa_ranges_geo."""
+    _fields_ = [("lo", C.c_double * 3), ("hi", C.c_double * 3), ("excess_per_m", C.c_double), ("spread", C.c_double),
+                ("p_loss", C.c_double)]
 
 
 _LIB = None
@@ -118,6 +125,8 @@ SIGNATURES = {
     "kfpos_synth_toa_ranges_nlos": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _VP, _VP]),
     "kfpos_batch_score_selection": (_I, [_VP, _I, _VP, _I, _VP, _VP, _VP, _VP]),
     "kfpos_batch_crlb": (_I, [_VP, _I, _I, _VP, _VP, _I, _D, _VP, _VP, _VP, _VP, _VP]),
+    "kfpos_synth_toa_ranges_geo": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _I, _VP, _VP,
+                                        _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

@@ -291,7 +291,7 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
 
 def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED, period=0.1, sigma_r=0.10,
                          p_missing=0.0, p_nlos=0.0, nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None,
-                         want_x0=False, want_truth=False, out=None, stream=None, want_nlos=False):
+                         want_x0=False, want_truth=False, out=None, stream=None, want_nlos=False, obstacles=None):
     """Ranging epochs [epoch0, epoch0 + n_epochs) of the T6 Monte Carlo workload, generated ON THE DEVICE by
     kfpos_synth_toa_ranges (Philox4x32-10; a ranging depends only on seed, the global filter index
     first_filter + f, the global epoch index and the anchor, so sharding and chunking change nothing).  Epoch k
@@ -304,7 +304,10 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     kfpos_synth_k8_truth, what Batch.set_truth_traj takes for the chunk) if want_truth, nlos [n][N] if want_nlos:
     the NLOS ground truth of kfpos_synth_toa_ranges_nlos, bit a set where ranging a carries a bias and is present,
     as int32 holding the uint32 bits).  `out` may hold the tensors of a previous chunk of the same shape to be
-    reused.  ML batches take `ranges` row by row."""
+    reused.  ML batches take `ranges` row by row.
+    obstacles: [n][9] boxes (lo x y z, hi x y z, excess_per_m, spread, p_loss; DESIGN §4.5f) whose crossing biases
+    or removes a ranging (kfpos_synth_toa_ranges_geo); the nlos mask then also marks the blocked rangings.  None or
+    an empty array: no boxes, the calls above."""
     import ctypes as C
     import torch
     from . import lib as L
@@ -330,9 +333,17 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     sp = None if stream is None else C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
     args = (dev.index or 0, N, M, C.c_void_p(anc.ctypes.data), n, C.c_void_p(t.ctypes.data), C.byref(gen), fmt,
             C.c_void_p(ranges.data_ptr()))
-    nlos = None
-    if want_nlos:
-        nlos = buf("nlos", (n, N), torch.int32)  # torch has no general uint32: the bits of the uint32 masks
+    nlos = buf("nlos", (n, N), torch.int32) if want_nlos else None  # torch has no general uint32: the mask bits
+    box = np.zeros((0, 9)) if obstacles is None else np.asarray(obstacles, dtype=np.float64).reshape(-1, 9)
+    if len(box):
+        tbl = (L.KfposObstacle * len(box))()
+        for o, b in zip(tbl, box):
+            o.lo[:], o.hi[:] = b[0:3], b[3:6]
+            o.excess_per_m, o.spread, o.p_loss = b[6], b[7], b[8]
+        L.check(L.lib().kfpos_synth_toa_ranges_geo(*args[:7], len(box), C.cast(tbl, C.c_void_p), *args[7:],
+                                                   None if nlos is None else C.c_void_p(nlos.data_ptr()), sp),
+                "kfpos_synth_toa_ranges_geo")
+    elif want_nlos:
         L.check(L.lib().kfpos_synth_toa_ranges_nlos(*args, C.c_void_p(nlos.data_ptr()), sp),
                 "kfpos_synth_toa_ranges_nlos")
     else:
@@ -363,7 +374,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
 def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
                    nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
-                   stream=None, hist=None, score=False, *, crlb=None):
+                   stream=None, hist=None, score=False, *, crlb=None, obstacles=None):
     """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
     for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
     truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
@@ -380,14 +391,16 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
     crlb=("present", "los", "used") or any of them: each chunk also calls Batch.crlb for each set with its truth,
     log, NLOS mask and selection, at the generator's ranging variance sigma_r^2 + (1 mm)^2 / 12 (its noise and its
     floor to whole millimetres); a dict {set: [n_epochs][4]} (batch.crlb_summary) is appended as the last element
-    of the return value, a tuple then."""
+    of the return value, a tuple then.
+    obstacles: the boxes of toa_montecarlo_chunk (DESIGN §4.5f); score and crlb "los" then use the mask that also
+    marks the rangings they block."""
     from . import lib as L
     if batch.model != L.MODEL_T6:
         raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
     if int(chunk) <= 0 or int(n_epochs) <= 0:
         raise ValueError("toa_montecarlo: n_epochs and chunk must be positive")
     kw = dict(seed=seed, period=period, sigma_r=sigma_r, p_missing=p_missing, p_nlos=p_nlos, nlos_mean=nlos_mean,
-              tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream)
+              tag_z=tag_z, first_filter=first_filter, fmt=fmt, stream=stream, obstacles=obstacles)
     crlb = (crlb,) if isinstance(crlb, str) else tuple(crlb or ())
     bounds = {name: [] for name in crlb}
     want_sel, want_nlos = score or "used" in crlb, score or "los" in crlb
