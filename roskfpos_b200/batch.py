@@ -47,6 +47,11 @@ def _stream_ptr(stream) -> Optional[C.c_void_p]:
     return C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
 
 
+def _comm_ptr(comm) -> Optional[C.c_void_p]:
+    """A raw ncclComm_t (an int or c_void_p, see shard.nccl_comm) as the library takes it; None = no communicator."""
+    return C.c_void_p(int(comm)) if comm else None
+
+
 def make_config(**kw) -> L.KfposConfig:
     cfg = L.KfposConfig()
     L.lib().kfpos_config_default(C.byref(cfg))
@@ -270,6 +275,16 @@ class Batch:
                 "kfpos_batch_ml_solve")
         return out
 
+    def _result(self, out, readback, shape, counts=False):
+        """The array a reader fills: `out` when given, else zeros on the host when `readback`, else a new device
+        tensor on this batch's GPU.  float64, or for counts uint64 on the host and int64 on the device."""
+        if out is not None:
+            return out
+        if readback:
+            return np.zeros(shape, dtype=np.uint64 if counts else np.float64)
+        import torch
+        return torch.empty(shape, dtype=torch.int64 if counts else torch.float64, device="cuda:%d" % self.device)
+
     # ------------------------------------------------------------ diagnostics
     def counters(self, reset=False, stream=None):
         buf = (C.c_double * 8)()
@@ -301,8 +316,8 @@ class Batch:
         Returns [sum |e|^2, sum |e_xy|^2, n, n_bad, rmse, rmse_xy]."""
         buf = (C.c_double * 6)()
         p, k = _ptr(truth, np.float64)
-        c = C.c_void_p(int(comm)) if comm else None
-        L.check(L.lib().kfpos_stats_allreduce(self._h, c, p, C.byref(buf), _stream_ptr(stream)), "kfpos_stats_allreduce")
+        L.check(L.lib().kfpos_stats_allreduce(self._h, _comm_ptr(comm), p, C.byref(buf), _stream_ptr(stream)),
+                "kfpos_stats_allreduce")
         return np.array(list(buf))
 
     # ------------------------------------------------- per-epoch statistics
@@ -323,11 +338,7 @@ class Batch:
         n in the NEES (kfpos_batch_epoch_stats).  out: a device tensor [rows][6] to fill asynchronously
         (returned as given); readback False without `out`: a new device tensor, filled asynchronously."""
         rows = getattr(self, "_es_rows", 0)
-        if out is None and readback:
-            out = np.zeros((rows, 6))
-        if out is None:
-            import torch
-            out = torch.empty((rows, 6), dtype=torch.float64, device="cuda:%d" % self.device)
+        out = self._result(out, readback, (rows, 6))
         L.check(L.lib().kfpos_batch_epoch_stats(self._h, C.c_int64(rows), _ptr(out)[0], _stream_ptr(stream)),
                 "kfpos_batch_epoch_stats")
         return out
@@ -337,9 +348,9 @@ class Batch:
         ncclComm_t as an int / c_void_p, see shard.nccl_comm; None = this batch alone).  Returns [rows][6]."""
         rows = getattr(self, "_es_rows", 0)
         out = np.zeros((rows, 6))
-        c = C.c_void_p(int(comm)) if comm else None
-        L.check(L.lib().kfpos_epoch_stats_allreduce(self._h, c, C.c_int64(rows), C.c_void_p(out.ctypes.data),
-                                                    _stream_ptr(stream)), "kfpos_epoch_stats_allreduce")
+        L.check(L.lib().kfpos_epoch_stats_allreduce(self._h, _comm_ptr(comm), C.c_int64(rows),
+                                                    C.c_void_p(out.ctypes.data), _stream_ptr(stream)),
+                "kfpos_epoch_stats_allreduce")
         return out
 
     # ------------------------------------------------ per-epoch error histograms
@@ -365,11 +376,7 @@ class Batch:
         (int64 or uint64) of that shape to fill asynchronously (returned as given); readback False without
         `out`: a new device int64 tensor, filled asynchronously."""
         rows, bins = getattr(self, "_es_rows", 0), getattr(self, "_eh_bins", 0)
-        if out is None and readback:
-            out = np.zeros((rows, bins), dtype=np.uint64)
-        if out is None:
-            import torch
-            out = torch.empty((rows, bins), dtype=torch.int64, device="cuda:%d" % self.device)
+        out = self._result(out, readback, (rows, bins), counts=True)
         L.check(L.lib().kfpos_batch_error_hist(self._h, C.c_int64(rows), _ptr(out)[0], _stream_ptr(stream)),
                 "kfpos_batch_error_hist")
         return out
@@ -380,9 +387,9 @@ class Batch:
         sizes.  Returns [rows][n_edges + 1] uint64."""
         rows, bins = getattr(self, "_es_rows", 0), getattr(self, "_eh_bins", 0)
         out = np.zeros((rows, bins), dtype=np.uint64)
-        c = C.c_void_p(int(comm)) if comm else None
-        L.check(L.lib().kfpos_error_hist_allreduce(self._h, c, C.c_int64(rows), C.c_void_p(out.ctypes.data),
-                                                   _stream_ptr(stream)), "kfpos_error_hist_allreduce")
+        L.check(L.lib().kfpos_error_hist_allreduce(self._h, _comm_ptr(comm), C.c_int64(rows),
+                                                   C.c_void_p(out.ctypes.data), _stream_ptr(stream)),
+                "kfpos_error_hist_allreduce")
         return out
 
     # ------------------------------------------------------- selection scores
@@ -395,11 +402,7 @@ class Batch:
         uint64) of that shape to fill asynchronously (returned as given); readback False without `out`: a new
         device int64 tensor, filled asynchronously."""
         rows = 1 if self.model == L.MODEL_ML else int(ranges.shape[0])
-        if out is None and readback:
-            out = np.zeros((rows, L.SCORE_COLS), dtype=np.uint64)
-        if out is None:
-            import torch
-            out = torch.empty((rows, L.SCORE_COLS), dtype=torch.int64, device="cuda:%d" % self.device)
+        out = self._result(out, readback, (rows, L.SCORE_COLS), counts=True)
         pr, kr = _ptr(ranges)
         ps, ks = _ptr(sel, np.int32)
         pn, kn = _ptr(nlos, np.uint32)
@@ -422,11 +425,7 @@ class Batch:
         if set not in self._CRLB_SET:
             raise ValueError(f"crlb: set must be one of {sorted(self._CRLB_SET)}")
         rows = 1 if self.model == L.MODEL_ML else int(ranges.shape[0])
-        if out is None and readback:
-            out = np.zeros((rows, L.CRLB_COLS))
-        if out is None:
-            import torch
-            out = torch.empty((rows, L.CRLB_COLS), dtype=torch.float64, device="cuda:%d" % self.device)
+        out = self._result(out, readback, (rows, L.CRLB_COLS))
         vs, pv, kv = (float(var), None, None) if np.isscalar(var) else (0.0, *_ptr(var, np.float64))
         pt, kt = _ptr(truth, np.float64)
         pr, kr = _ptr(ranges)

@@ -71,24 +71,23 @@ struct kfpos_batch {
     // ground truth registered with kfpos_batch_set_truth: the replay kernels then leave the error
     // partials of their final state in d_partials (the reduction fused into the last replay step)
     const double *d_truth = nullptr;
-    double *d_truth_own = nullptr;
+    DevBuf truth_own; // the copy of a host truth array
     bool partials_fresh = false;
     bool out4_valid = false; // d_out4 holds the statistics of the current state
-    DevBuf gather; // [n_ranks][4] of kfpos_stats_allreduce
-    // per-epoch statistics (kfpos_batch_set_truth_traj): truth rows SoA [es_rows][3][N], per-warp sums
-    // [es_rows][n_warps][6] left by the replay kernels, the next output row, and the fold buffers
+    // per-epoch statistics (kfpos_batch_set_truth_traj): truth rows SoA [es_rows][3][N] (a borrowed device array or
+    // etruth_own), per-warp sums [es_rows][n_warps][6] left by the replay kernels, and the next output row
     const double *d_etruth = nullptr;
-    double *d_etruth_own = nullptr, *d_escratch = nullptr, *d_efold = nullptr, *d_eout = nullptr;
-    int64_t es_rows = 0, es_cursor = 0, es_fold_rows = 0;
-    DevBuf es_gather;
+    DevBuf etruth_own, escratch;
+    int64_t es_rows = 0, es_cursor = 0;
     // per-epoch error histogram (kfpos_batch_set_error_hist): the quantity, the device edge table [EH_MAX_BINS - 1]
     // (squared for the error quantities, +inf behind the last edge), and the counts [es_rows][eh_bins], which
     // exist while a truth trajectory is registered too
     int eh_quantity = 0, eh_bins = 0; // eh_bins == 0: no histogram
-    double *d_eh_edges = nullptr;
-    unsigned long long *d_eh_counts = nullptr;
-    DevBuf eh_gather;
-    DevBuf crlb; // per-warp partials of kfpos_batch_crlb, [rows][n_warps][4], at most 256 MB
+    DevBuf eh_edges, eh_counts;
+    // scratch of one call at a time (calls on one handle are serialised): the per-warp partials of a batch of rows
+    // that kfpos_batch_epoch_stats and kfpos_batch_crlb fold (at most 256 MB, fold_rows), and the receive buffer
+    // [n_ranks][count] of the all-gathers
+    DevBuf fold, gather;
     // K8 / T9 latched sensor samples, SoA rows (see kfpos_k8.cuh)
     double *d_latch = nullptr;
     double *d_latch_u = nullptr; // batch-wide latched IMU covariances
@@ -311,9 +310,17 @@ RangeStream make_rs(const kfpos_batch *b, const void *ranges, int fmt, double er
 }
 
 int64_t es_warps(const kfpos_batch *b) { return (b->N + 31) / 32; }
+// the output rows the replay launches have filled since the cursor was last reset
+int64_t es_done(const kfpos_batch *b) { return b->es_cursor < b->es_rows ? b->es_cursor : b->es_rows; }
+// rows per batch of a fold over the warp index, so that the per-warp partials of a batch (`row_bytes` per row) fit
+// in 256 MB of scratch
+int64_t fold_rows(size_t row_bytes, int64_t n_rows) {
+    const int64_t r = (int64_t)(((size_t)256 << 20) / row_bytes);
+    return r < 1 ? 1 : (r > n_rows ? n_rows : r);
+}
 // a launch with `rows` output rows: fits the registered truth trajectory (or none is registered)?
 int es_check(const kfpos_batch *b, int64_t rows) {
-    return (b->d_escratch && b->es_cursor + rows > b->es_rows) ? KFPOS_ERR_INVALID : KFPOS_OK;
+    return (b->escratch.p && b->es_cursor + rows > b->es_rows) ? KFPOS_ERR_INVALID : KFPOS_OK;
 }
 // the per-epoch statistics pointers of the next launch, then the cursor moves past its `rows` output rows.  The
 // histogram rows of the launch are zeroed first: a re-run after set_state overwrites them, as it does the sums.
@@ -323,14 +330,14 @@ int es_bind(kfpos_batch *b, Params &p, int64_t rows, cudaStream_t s) {
     p.etruth = nullptr;
     p.escratch = nullptr;
     p.ehist = nullptr;
-    p.eedges = b->d_eh_edges;
+    p.eedges = (const double *)b->eh_edges.p;
     p.equantity = b->eh_quantity;
     p.ebins = b->eh_bins;
-    if (!b->d_escratch) return KFPOS_OK;
+    if (!b->escratch.p) return KFPOS_OK;
     p.etruth = b->d_etruth + b->es_cursor * 3 * b->N;
-    p.escratch = b->d_escratch + b->es_cursor * p.n_warps * ES_W;
-    if (b->d_eh_counts) {
-        p.ehist = b->d_eh_counts + b->es_cursor * b->eh_bins;
+    p.escratch = (double *)b->escratch.p + b->es_cursor * p.n_warps * ES_W;
+    if (b->eh_counts.p) {
+        p.ehist = (unsigned long long *)b->eh_counts.p + b->es_cursor * b->eh_bins;
         CK(cudaMemsetAsync(p.ehist, 0, sizeof(unsigned long long) * (size_t)rows * (size_t)b->eh_bins, s));
     }
     b->es_cursor += rows;
@@ -458,17 +465,8 @@ extern "C" void kfpos_batch_destroy(kfpos_batch *b) {
     cudaFree(b->d_counters);
     cudaFree(b->d_partials);
     cudaFree(b->d_out4);
-    cudaFree(b->d_truth_own);
-    b->gather.release();
-    cudaFree(b->d_etruth_own);
-    cudaFree(b->d_escratch);
-    cudaFree(b->d_efold);
-    cudaFree(b->d_eout);
-    b->es_gather.release();
-    cudaFree(b->d_eh_edges);
-    cudaFree(b->d_eh_counts);
-    b->eh_gather.release();
-    b->crlb.release();
+    for (DevBuf *d : {&b->truth_own, &b->etruth_own, &b->escratch, &b->eh_edges, &b->eh_counts, &b->fold, &b->gather})
+        d->release();
     cudaFree(b->d_latch);
     cudaFree(b->d_has);
     cudaFree(b->d_latch_u);
@@ -1196,6 +1194,22 @@ extern "C" int kfpos_batch_get_counters(kfpos_batch *b, double out[8], int reset
     return KFPOS_OK;
 }
 
+namespace {
+// the device array of a truth the caller registers, in *d: a device array is borrowed (the caller keeps it alive
+// while it is registered); a host array of `bytes` is copied into `own`, then the stream is synchronised
+cudaError_t truth_on_device(const double *truth, size_t bytes, DevBuf &own, cudaStream_t s, const double **d) {
+    if (on_device(truth)) {
+        *d = truth;
+        return cudaSuccess;
+    }
+    cudaError_t e = own.reserve(bytes);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(own.p, truth, bytes, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e == cudaSuccess) *d = (const double *)own.p;
+    return e;
+}
+} // namespace
+
 extern "C" int kfpos_batch_set_truth(kfpos_batch *b, const double *truth, void *stream) {
     if (!b || b->model == KFPOS_MODEL_ML) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
@@ -1206,15 +1220,7 @@ extern "C" int kfpos_batch_set_truth(kfpos_batch *b, const double *truth, void *
         b->d_truth = nullptr;
         return KFPOS_OK;
     }
-    if (on_device(truth)) { // borrowed: the caller keeps it alive while it is registered
-        b->d_truth = truth;
-        return KFPOS_OK;
-    }
-    const size_t bytes = sizeof(double) * 3 * (size_t)b->N;
-    if (!b->d_truth_own) CK(cudaMalloc((void **)&b->d_truth_own, bytes));
-    CK(cudaMemcpyAsync(b->d_truth_own, truth, bytes, cudaMemcpyHostToDevice, s));
-    CK(cudaStreamSynchronize(s));
-    b->d_truth = b->d_truth_own;
+    CK(truth_on_device(truth, sizeof(double) * 3 * (size_t)b->N, b->truth_own, s, &b->d_truth));
     return KFPOS_OK;
 }
 
@@ -1314,64 +1320,60 @@ extern "C" int kfpos_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, cons
 }
 
 // ------------------------------------------------------- per-epoch statistics
+namespace {
+// (re)allocates the histogram counts [es_rows][eh_bins] and zeroes them on `s`: none unless both a histogram and a
+// truth trajectory are registered
+cudaError_t alloc_counts(kfpos_batch *b, cudaStream_t s) {
+    b->eh_counts.release();
+    const size_t bytes = sizeof(unsigned long long) * (size_t)b->eh_bins * (size_t)b->es_rows;
+    if (!bytes) return cudaSuccess;
+    cudaError_t e = b->eh_counts.reserve(bytes);
+    return e == cudaSuccess ? cudaMemsetAsync(b->eh_counts.p, 0, bytes, s) : e;
+}
+// forgets the truth trajectory (cudaFree waits for the device: no launch still reads its buffers)
+void drop_truth_traj(kfpos_batch *b) {
+    b->etruth_own.release();
+    b->escratch.release();
+    b->eh_counts.release();
+    b->d_etruth = nullptr;
+    b->es_rows = b->es_cursor = 0;
+}
+} // namespace
+
 extern "C" int kfpos_batch_set_truth_traj(kfpos_batch *b, int64_t n_rows, const double *truth, void *stream) {
     if (!b || b->model == KFPOS_MODEL_ML || (truth && n_rows <= 0)) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
-    // (cudaFree waits for the device: no launch still reads the buffers of the previous registration)
-    cudaFree(b->d_etruth_own);
-    cudaFree(b->d_escratch);
-    cudaFree(b->d_efold);
-    cudaFree(b->d_eout);
-    cudaFree(b->d_eh_counts);
-    b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
-    b->d_eh_counts = nullptr;
-    b->d_etruth = nullptr;
-    b->es_rows = b->es_cursor = b->es_fold_rows = 0;
+    drop_truth_traj(b);
     if (!truth) return KFPOS_OK;
-    const int64_t W = es_warps(b);
-    const size_t row_bytes = sizeof(double) * ES_W * (size_t)W;
-    // the fold of kfpos_batch_epoch_stats works on batches of rows in a buffer of at most 256 MB
-    int64_t fold_rows = (int64_t)(((size_t)256 << 20) / row_bytes);
-    if (fold_rows < 1) fold_rows = 1;
-    if (fold_rows > n_rows) fold_rows = n_rows;
-    const bool dev = on_device(truth);
-    cudaError_t e = cudaMalloc((void **)&b->d_escratch, row_bytes * (size_t)n_rows);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_efold, row_bytes * (size_t)fold_rows);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_eout, sizeof(double) * ES_W * (size_t)n_rows);
-    // a registered histogram gets its counts with the rows (kfpos_batch_set_error_hist)
-    const size_t hbytes = sizeof(unsigned long long) * (size_t)b->eh_bins * (size_t)n_rows;
-    if (e == cudaSuccess && hbytes) e = cudaMalloc((void **)&b->d_eh_counts, hbytes);
-    if (e == cudaSuccess && hbytes) e = cudaMemsetAsync(b->d_eh_counts, 0, hbytes, s);
-    const size_t tbytes = sizeof(double) * 3 * (size_t)b->N * (size_t)n_rows;
-    if (e == cudaSuccess && !dev) e = cudaMalloc((void **)&b->d_etruth_own, tbytes);
-    if (e == cudaSuccess && !dev) e = cudaMemcpyAsync(b->d_etruth_own, truth, tbytes, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess && !dev) e = cudaStreamSynchronize(s);
+    const size_t row_bytes = sizeof(double) * ES_W * (size_t)es_warps(b);
+    b->es_rows = n_rows;
+    cudaError_t e = b->escratch.reserve(row_bytes * (size_t)n_rows);
+    // the fold of kfpos_batch_epoch_stats, so that a registration it could not read fails here
+    if (e == cudaSuccess) e = b->fold.reserve(row_bytes * (size_t)fold_rows(row_bytes, n_rows));
+    if (e == cudaSuccess) e = alloc_counts(b, s); // a registered histogram gets its counts with the rows
+    if (e == cudaSuccess)
+        e = truth_on_device(truth, sizeof(double) * 3 * (size_t)b->N * (size_t)n_rows, b->etruth_own, s, &b->d_etruth);
     if (e != cudaSuccess) {
-        cudaFree(b->d_etruth_own);
-        cudaFree(b->d_escratch);
-        cudaFree(b->d_efold);
-        cudaFree(b->d_eout);
-        cudaFree(b->d_eh_counts);
-        b->d_etruth_own = b->d_escratch = b->d_efold = b->d_eout = nullptr;
-        b->d_eh_counts = nullptr;
+        drop_truth_traj(b);
         cudaGetLastError();
         return map_cuda_err(e);
     }
-    b->d_etruth = dev ? truth : b->d_etruth_own; // a device array is borrowed: the caller keeps it alive
-    b->es_rows = n_rows;
-    b->es_fold_rows = fold_rows;
     return KFPOS_OK;
 }
 
 namespace {
-// [n_rows][6] of this batch into the device array `d_out`: rows [0, cursor) folded over the warp index (batches
-// of es_fold_rows rows through d_efold, the per-warp sums stay as they are), the rest zero
+// [es_rows][6] of this batch into the device array `d_out`: the rows the cursor has passed folded over the warp
+// index (batches of fold_rows rows through `fold`, the per-warp sums stay as they are), the rest zero
 int enqueue_epoch_stats(kfpos_batch *b, double *d_out, cudaStream_t s) {
-    const int64_t W = es_warps(b), done = b->es_cursor < b->es_rows ? b->es_cursor : b->es_rows;
-    for (int64_t r0 = 0; r0 < done; r0 += b->es_fold_rows) {
-        const int64_t rb = done - r0 < b->es_fold_rows ? done - r0 : b->es_fold_rows;
-        CK(launch_stats_tree(ES_W, rb, W, b->d_escratch + r0 * W * ES_W, b->d_efold, W * ES_W, ES_W, d_out + r0 * ES_W, s));
+    const int64_t W = es_warps(b), done = es_done(b);
+    const size_t row_bytes = sizeof(double) * ES_W * (size_t)W;
+    const int64_t rows = fold_rows(row_bytes, b->es_rows);
+    CK(b->fold.reserve(row_bytes * (size_t)rows)); // held since the registration, unless a failed kfpos_batch_crlb freed it
+    for (int64_t r0 = 0; r0 < done; r0 += rows) {
+        const int64_t rb = done - r0 < rows ? done - r0 : rows;
+        CK(launch_stats_tree(ES_W, rb, W, (double *)b->escratch.p + r0 * W * ES_W, (double *)b->fold.p, W * ES_W, ES_W,
+                             d_out + r0 * ES_W, s));
     }
     if (done < b->es_rows)
         CK(cudaMemsetAsync(d_out + done * ES_W, 0, sizeof(double) * ES_W * (size_t)(b->es_rows - done), s));
@@ -1379,21 +1381,13 @@ int enqueue_epoch_stats(kfpos_batch *b, double *d_out, cudaStream_t s) {
 }
 int es_ready(const kfpos_batch *b, int64_t n_rows, const double *out) {
     if (!b || b->model == KFPOS_MODEL_ML || !out) return KFPOS_ERR_INVALID;
-    if (!b->d_escratch) return KFPOS_ERR_NOT_READY;
+    if (!b->escratch.p) return KFPOS_ERR_NOT_READY;
     return n_rows == b->es_rows ? KFPOS_OK : KFPOS_ERR_INVALID;
 }
 } // namespace
 
 extern "C" int kfpos_batch_epoch_stats(kfpos_batch *b, int64_t n_rows, double *out, void *stream) {
-    int rc = es_ready(b, n_rows, out);
-    if (rc) return rc;
-    DeviceGuard g(b->device);
-    cudaStream_t s = (cudaStream_t)stream;
-    Staging st(b, s);
-    double *d_out = st.out(out, sizeof(double) * ES_W * (size_t)n_rows);
-    if (st.rc) return st.rc;
-    if ((rc = enqueue_epoch_stats(b, d_out, s))) return rc;
-    return st.finish();
+    return kfpos_epoch_stats_allreduce(b, nullptr, n_rows, out, stream);
 }
 
 extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, double *out,
@@ -1402,23 +1396,33 @@ extern "C" int kfpos_epoch_stats_allreduce(kfpos_batch *b, struct ncclComm *comm
     if (rc) return rc;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
-    if ((rc = enqueue_epoch_stats(b, b->d_eout, s))) return rc;
-    const double *d_res = b->d_eout;
+    const size_t n = (size_t)n_rows * ES_W;
+    Staging st(b, s);
+    double *d_out = st.out(out, sizeof(double) * n);
+    double *d_mine = comm ? st.buf<double>(sizeof(double) * n) : d_out; // comm: the send buffer of the collective
+    if (st.rc) return st.rc;
+    if ((rc = enqueue_epoch_stats(b, d_mine, s))) return rc;
     if (comm) {
         // every rank's [n_rows][6] to every rank ([rank][row][6]), then per row the pairwise tree over the rank
-        // index -- the top levels of the global tree; row r's result lands on its rank-0 entry
+        // index -- the top levels of the global tree
         int n_ranks = 0;
-        if ((rc = all_gather(comm, b->d_eout, (size_t)n_rows * ES_W, b->es_gather, &n_ranks, s))) return rc;
-        double *gat = (double *)b->es_gather.p;
-        CK(launch_stats_tree(ES_W, n_rows, n_ranks, gat, gat, ES_W, n_rows * ES_W, gat, s));
-        d_res = gat;
+        if ((rc = all_gather(comm, d_mine, n, b->gather, &n_ranks, s))) return rc;
+        double *gat = (double *)b->gather.p;
+        CK(launch_stats_tree(ES_W, n_rows, n_ranks, gat, gat, ES_W, n_rows * ES_W, d_out, s));
     }
-    Staging st(b, s);
-    st.copy_out(out, d_res, sizeof(double) * ES_W * (size_t)n_rows);
     return st.finish();
 }
 
 // ------------------------------------------------------- per-epoch error histograms
+namespace {
+// forgets the histogram (cudaFree waits for the device: no launch still reads the table or the counts)
+void drop_error_hist(kfpos_batch *b) {
+    b->eh_edges.release();
+    b->eh_counts.release();
+    b->eh_bins = b->eh_quantity = 0;
+}
+} // namespace
+
 extern "C" int kfpos_batch_set_error_hist(kfpos_batch *b, int quantity, int n_edges, const double *edges) {
     if (!b || b->model == KFPOS_MODEL_ML || n_edges < 0) return KFPOS_ERR_INVALID;
     const bool reg = n_edges > 0 && edges;
@@ -1438,57 +1442,39 @@ extern "C" int kfpos_batch_set_error_hist(kfpos_batch *b, int quantity, int n_ed
         tbl.resize(EH_MAX_BINS - 1, INFINITY); // the kernel's search always spans EH_MAX_BINS - 1 entries
     }
     DeviceGuard g(b->device);
-    // (cudaFree waits for the device: no launch still reads the previous table or counts)
-    cudaFree(b->d_eh_edges);
-    cudaFree(b->d_eh_counts);
-    b->d_eh_edges = nullptr;
-    b->d_eh_counts = nullptr;
-    b->eh_bins = b->eh_quantity = 0;
+    drop_error_hist(b);
     if (!reg) return KFPOS_OK;
-    const size_t hbytes = sizeof(unsigned long long) * (size_t)(n_edges + 1) * (size_t)b->es_rows;
-    cudaError_t e = cudaMalloc((void **)&b->d_eh_edges, sizeof(double) * tbl.size());
-    if (e == cudaSuccess) e = cudaMemcpy(b->d_eh_edges, tbl.data(), sizeof(double) * tbl.size(), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && hbytes) e = cudaMalloc((void **)&b->d_eh_counts, hbytes);
-    if (e == cudaSuccess && hbytes) e = cudaMemset(b->d_eh_counts, 0, hbytes);
+    b->eh_bins = n_edges + 1;
+    cudaError_t e = b->eh_edges.reserve(sizeof(double) * tbl.size());
+    if (e == cudaSuccess) e = cudaMemcpy(b->eh_edges.p, tbl.data(), sizeof(double) * tbl.size(), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = alloc_counts(b, nullptr);
     if (e != cudaSuccess) {
-        cudaFree(b->d_eh_edges);
-        cudaFree(b->d_eh_counts);
-        b->d_eh_edges = nullptr;
-        b->d_eh_counts = nullptr;
+        drop_error_hist(b);
         cudaGetLastError();
         return map_cuda_err(e);
     }
     b->eh_quantity = quantity;
-    b->eh_bins = n_edges + 1;
     return KFPOS_OK;
 }
 
 namespace {
 int eh_ready(const kfpos_batch *b, int64_t n_rows, const uint64_t *counts) {
     if (!b || b->model == KFPOS_MODEL_ML || !counts) return KFPOS_ERR_INVALID;
-    if (!b->d_eh_counts) return KFPOS_ERR_NOT_READY; // no histogram or no truth trajectory
+    if (!b->eh_counts.p) return KFPOS_ERR_NOT_READY; // no histogram or no truth trajectory
     return n_rows == b->es_rows ? KFPOS_OK : KFPOS_ERR_INVALID;
 }
 // [es_rows][eh_bins] of this batch into the device array `d_out`: the rows the cursor has passed, the rest zero
 int enqueue_error_hist(kfpos_batch *b, unsigned long long *d_out, cudaStream_t s) {
-    const int64_t done = b->es_cursor < b->es_rows ? b->es_cursor : b->es_rows;
+    const int64_t done = es_done(b);
     const size_t row_bytes = sizeof(unsigned long long) * (size_t)b->eh_bins;
-    if (done > 0) CK(cudaMemcpyAsync(d_out, b->d_eh_counts, row_bytes * (size_t)done, cudaMemcpyDeviceToDevice, s));
+    if (done > 0) CK(cudaMemcpyAsync(d_out, b->eh_counts.p, row_bytes * (size_t)done, cudaMemcpyDeviceToDevice, s));
     if (done < b->es_rows) CK(cudaMemsetAsync(d_out + done * b->eh_bins, 0, row_bytes * (size_t)(b->es_rows - done), s));
     return KFPOS_OK;
 }
 } // namespace
 
 extern "C" int kfpos_batch_error_hist(kfpos_batch *b, int64_t n_rows, uint64_t *counts, void *stream) {
-    int rc = eh_ready(b, n_rows, counts);
-    if (rc) return rc;
-    DeviceGuard g(b->device);
-    cudaStream_t s = (cudaStream_t)stream;
-    Staging st(b, s);
-    auto *d_out = (unsigned long long *)st.out(counts, sizeof(uint64_t) * (size_t)b->eh_bins * (size_t)n_rows);
-    if (st.rc) return st.rc;
-    if ((rc = enqueue_error_hist(b, d_out, s))) return rc;
-    return st.finish();
+    return kfpos_error_hist_allreduce(b, nullptr, n_rows, counts, stream);
 }
 
 extern "C" int kfpos_error_hist_allreduce(kfpos_batch *b, struct ncclComm *comm, int64_t n_rows, uint64_t *counts,
@@ -1500,19 +1486,16 @@ extern "C" int kfpos_error_hist_allreduce(kfpos_batch *b, struct ncclComm *comm,
     const size_t n = (size_t)b->eh_bins * (size_t)n_rows;
     Staging st(b, s);
     auto *d_out = (unsigned long long *)st.out(counts, sizeof(uint64_t) * n);
-    if (st.rc) return st.rc;
-    if (!comm) {
-        if ((rc = enqueue_error_hist(b, d_out, s))) return rc;
-        return st.finish();
-    }
-    // every rank's counts to every rank ([rank][row][bin]), then the integer sum over the rank index: exact in
-    // any order, so any split of the filters over the ranks gives the single-GPU counts
-    unsigned long long *d_mine = st.buf<unsigned long long>(sizeof(uint64_t) * n);
+    unsigned long long *d_mine = comm ? st.buf<unsigned long long>(sizeof(uint64_t) * n) : d_out; // as for the sums
     if (st.rc) return st.rc;
     if ((rc = enqueue_error_hist(b, d_mine, s))) return rc;
-    int n_ranks = 0;
-    if ((rc = all_gather(comm, d_mine, n, b->eh_gather, &n_ranks, s, NCCL_UINT64))) return rc;
-    CK(launch_sum_ranks_u64(n_ranks, (int64_t)n, (const unsigned long long *)b->eh_gather.p, d_out, s));
+    if (comm) {
+        // every rank's counts to every rank ([rank][row][bin]), then the integer sum over the rank index: exact in
+        // any order, so any split of the filters over the ranks gives the single-GPU counts
+        int n_ranks = 0;
+        if ((rc = all_gather(comm, d_mine, n, b->gather, &n_ranks, s, NCCL_UINT64))) return rc;
+        CK(launch_sum_ranks_u64(n_ranks, (int64_t)n, (const unsigned long long *)b->gather.p, d_out, s));
+    }
     return st.finish();
 }
 
@@ -1731,14 +1714,12 @@ extern "C" int kfpos_batch_crlb(kfpos_batch *b, int set, int n_rows, const doubl
     if (mode != SCORE_NONE && !sel) return KFPOS_ERR_INVALID;
     DeviceGuard g(b->device);
     cudaStream_t s = (cudaStream_t)stream;
-    const int64_t W = (b->N + 31) / 32;
+    const int64_t W = es_warps(b);
     const size_t N = (size_t)b->N, M = (size_t)b->anchors.n, R = (size_t)n_rows;
     const size_t row_bytes = sizeof(double) * CRLB_W * (size_t)W;
-    // the per-warp partials of a batch of rows, folded before the next batch: at most 256 MB of scratch
-    int64_t batch_rows = (int64_t)(((size_t)256 << 20) / row_bytes);
-    if (batch_rows < 1) batch_rows = 1;
-    if (batch_rows > n_rows) batch_rows = n_rows;
-    CK(b->crlb.reserve(row_bytes * (size_t)batch_rows));
+    // the per-warp partials of a batch of rows, folded before the next batch
+    const int64_t batch_rows = fold_rows(row_bytes, n_rows);
+    CK(b->fold.reserve(row_bytes * (size_t)batch_rows));
     Staging st(b, s);
     CrlbParams p;
     p.anchors = b->anchors;
@@ -1749,7 +1730,7 @@ extern "C" int kfpos_batch_crlb(kfpos_batch *b, int set, int n_rows, const doubl
     const uint32_t *d_nlos = set == KFPOS_CRLB_LOS ? st.in(nlos, sizeof(uint32_t) * N * R) : nullptr;
     double *d_out = st.out(out, sizeof(double) * CRLB_W * R);
     if (st.rc) return st.rc;
-    p.partials = (double *)b->crlb.p;
+    p.partials = (double *)b->fold.p;
     p.w_scalar = var ? 0.0 : 1.0 / var_scalar;
     p.N = b->N; p.n_warps = W; p.M = (int)M; p.fmt = fmt; p.set = set; p.sel_mode = mode;
     p.dim = b->model == KFPOS_MODEL_K8 || (ml && b->cfg.use2d) ? 2 : 3;

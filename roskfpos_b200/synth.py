@@ -234,6 +234,7 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
     import ctypes as C
     import torch
     from . import lib as L
+    from .batch import _stream_ptr
     macro = MACRO_FULL if full else MACRO_IMU_MAG
     M, N = len(anchors), int(n_filters)
     rows_of = {EV_IMU: 3, EV_PX4: 5, EV_COMPASS: 1}
@@ -270,7 +271,7 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
     for i, (kind, g, tt, off) in enumerate(sev):
         arr[i].kind, arr[i].global_index, arr[i].t, arr[i].offset = int(kind), int(g), float(tt), int(off)
     anc = np.ascontiguousarray(anchors, dtype=np.float64)
-    sp = None if stream is None else C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
+    sp = _stream_ptr(stream)
     L.check(L.lib().kfpos_synth_k8(dev.index or 0, N, int(first_filter), C.c_uint64(seed), M,
                                    C.c_void_p(anc.ctypes.data), 1.049, float(sigma_r), len(sev),
                                    C.cast(arr, C.c_void_p), float(t), n_rng * M, n_sens,
@@ -311,6 +312,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     import ctypes as C
     import torch
     from . import lib as L
+    from .batch import _stream_ptr
     fmt = L.FMT_I32_MM if fmt is None else int(fmt)
     if fmt not in (L.FMT_I32_MM, L.FMT_U16_MM):
         raise ValueError("toa_montecarlo_chunk: fmt must be FMT_I32_MM or FMT_U16_MM")
@@ -330,7 +332,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     gen = L.KfposSynthToa(seed=int(seed), first_filter=int(first_filter), first_epoch=int(epoch0), tag_z=float(tag_z),
                           sigma_r=float(sigma_r), p_missing=float(p_missing), p_nlos=float(p_nlos),
                           nlos_mean=float(nlos_mean))
-    sp = None if stream is None else C.c_void_p(int(getattr(stream, "cuda_stream", stream)))
+    sp = _stream_ptr(stream)
     args = (dev.index or 0, N, M, C.c_void_p(anc.ctypes.data), n, C.c_void_p(t.ctypes.data), C.byref(gen), fmt,
             C.c_void_p(ranges.data_ptr()))
     nlos = buf("nlos", (n, N), torch.int32) if want_nlos else None  # torch has no general uint32: the mask bits

@@ -9,7 +9,7 @@ from roskfpos_b200 import synth
 
 pytestmark = pytest.mark.gpu
 
-INVALID, NOT_READY = -1, -4
+INVALID, NOMEM, NOT_READY = -1, -3, -4
 
 
 # ---------------------------------------------------------------------------------------------- host emulation
@@ -404,3 +404,34 @@ def test_errors(kflib):
         b.replay_toa(0.1, np.concatenate([r, r[:1]]), err=0.01)
     with Batch(kflib.MODEL_ML, N, anchors=anc) as b:
         assert kflib.lib().kfpos_batch_set_truth_traj(b._h, 6, C.c_void_p(truth.ctypes.data), None) == INVALID
+
+
+def test_failed_registration(kflib):
+    """A truth trajectory whose scratch cannot be allocated (2^40 rows) is refused with NOMEM and leaves nothing
+    registered: epoch_stats is NOT_READY and a histogram still registers.  A registration after it gives the rows
+    and counts of a fresh batch bit for bit."""
+    from roskfpos_b200.batch import Batch
+    import ctypes as C
+    import torch
+    N = 256
+    anc, truth, r = t6_case(N)
+    edges = np.linspace(0.02, 1.0, 12)
+
+    def run(b):
+        b.set_truth_traj(truth[1:])
+        b.set_state(truth[0])
+        b.replay_toa(0.1, r, err=0.01)
+        return b.epoch_stats(), b.error_hist()
+    with Batch(kflib.MODEL_T6, N, anchors=anc, accel_noise=0.5) as b:
+        b.set_error_hist(edges)
+        fresh = run(b)
+    small = torch.zeros((2, 3, N), dtype=torch.float64, device="cuda:0")
+    out = np.zeros((6, 6))
+    with Batch(kflib.MODEL_T6, N, anchors=anc, accel_noise=0.5) as b:
+        rc = kflib.lib().kfpos_batch_set_truth_traj(b._h, C.c_int64(1 << 40), C.c_void_p(small.data_ptr()), None)
+        assert rc == NOMEM
+        assert kflib.lib().kfpos_batch_epoch_stats(b._h, 6, C.c_void_p(out.ctypes.data), None) == NOT_READY
+        b.set_error_hist(edges)
+        again = run(b)
+    assert np.array_equal(again[0], fresh[0]) and np.array_equal(again[1], fresh[1])
+    assert fresh[1].sum() > 0
