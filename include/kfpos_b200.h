@@ -615,6 +615,60 @@ int kfpos_synth_toa_ranges_geo(int device, int64_t n_filters, int n_anchors, con
                                int n_obstacles, const kfpos_obstacle *obstacles, int fmt,
                                void *ranges, uint32_t *nlos, void *stream);
 
+/* Ranging epochs along a caller's trajectory (DESIGN §4.5g): kfpos_synth_toa_ranges_geo with the truth of epoch
+ * g = first_epoch + k read from row k of `truth`, SoA [n_epochs][3][N] (x, y, z per epoch; the layout of
+ * kfpos_batch_set_truth_traj and kfpos_batch_crlb), HOST or device, in place of the Lissajous; gen->tag_z is
+ * ignored (z comes from the array, the slab test uses it too).  Everything else is kfpos_synth_toa_ranges_geo's:
+ * the Philox counters, noise, i.i.d. impairments, boxes, mask, formats and clamp -- so the truth of
+ * kfpos_synth_k8_truth at the same times gives the same bytes as kfpos_synth_toa_ranges / _nlos / _geo.  A NaN
+ * truth value gives absent rangings (0: mm > 0 fails); an infinite one gives the format's largest value (the
+ * clamp).  obstacles may be NULL with n_obstacles == 0,
+ * nlos may be NULL.  A host truth, ranges or nlos is staged and `stream` synchronised before returning; with device
+ * pointers only the call is asynchronous on `stream`.  Errors are kfpos_synth_toa_ranges_geo's; a NULL truth with
+ * n_epochs > 0 is KFPOS_ERR_INVALID.                                                                            */
+int kfpos_synth_toa_ranges_truth(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                 int n_epochs, const double *truth, const kfpos_synth_toa *gen,
+                                 int n_obstacles, const kfpos_obstacle *obstacles, int fmt,
+                                 void *ranges, uint32_t *nlos, void *stream);
+
+/* A random walk of the tag inside a caller's box (DESIGN §4.5g), the truth kfpos_synth_toa_ranges_truth takes:
+ * discrete white-noise acceleration, the F and Q of the T6 prediction, per axis i, kept inside [lo_i, hi_i].
+ * For filter gf = first_filter + f (Philox4x32-10 counter (gf lo, gf hi, event, sample), key (seed lo, seed hi)):
+ *   initial   (init 1) velocity 0; position lo_i + (hi_i - lo_i) u_i with (u_x, u_y) the uniforms of counter
+ *             (gf, 0xFFFFFFFF, 2) and u_z the first of (gf, 0xFFFFFFFF, 3); an axis with accel_sd_i == 0 starts at
+ *             (lo_i + hi_i) / 2 and stays there (a fixed tag height);
+ *   epoch g   (n_x, n_y) = the Box-Muller pair of counter (gf, g, 0x20000000); n_z the first normal of
+ *             (gf, g, 0x20000001), drawn only when accel_sd_z > 0 (else a_z = 0); per axis, with dt = period and
+ *             h = dt dt / 2:  a = accel_sd_i n_i,  p' = (p + v dt) + a h,  v' = v + a dt;
+ *             if p' > hi: p' = (hi + hi) - p', v' = -v'; else if p' < lo: p' = (lo + lo) - p', v' = -v';
+ *             then p' = min(max(p', lo), hi), v' = min(max(v', -v_max), v_max).
+ * Every step is one IEEE operation (no contraction), so a host reproduces a trajectory from its normals, and
+ * each value is a pure function of (seed, gf, g) and the initial state: a run gives the same trajectory however
+ * it is sharded (first_filter) or cut into chunks (first_epoch, with `state` carried).  The walk's samples
+ * (0x20000000, 0x20000001) are not among the ranging generator's (0..15, 0x80000000 | a, 0x40000000 | a), so
+ * the walk and the rangings may share one seed without sharing a draw.
+ * state: SoA [6][N] x, y, z, vx, vy, vz (the T6 state layout): the state at first_epoch on entry (read with
+ * init 0), the state after the last epoch on return.  truth: SoA [n_epochs][3][N], row k the position at time
+ * (first_epoch + k + 1) period (x0 is the state at t = 0).  init 1 with n_epochs == 0 writes the initial state
+ * and returns.  Host or device arrays; a host one is staged and `stream` synchronised before returning, with
+ * device pointers only the call is asynchronous on `stream`.  KFPOS_ERR_INVALID: a bad count, first_filter or
+ * first_epoch < 0, an epoch range that reaches the reserved index, period <= 0 or not finite, accel_sd negative
+ * or not finite, v_max <= 0 or NaN, a non-finite corner or !(lo < hi) on an axis, init not 0 or 1, a NULL state,
+ * a NULL truth with n_epochs > 0.  KFPOS_ERR_CUDA without a device (there is no CPU path).                       */
+struct kfpos_synth_walk { /* a struct tag only, beside the function of the same name (as struct stat / stat()) */
+    uint64_t seed;
+    int64_t first_filter;  /* global index of output filter 0 (sharding)                 */
+    int64_t first_epoch;   /* global index of epoch 0 of this call (chunking)            */
+    double period;         /* s, > 0                                                     */
+    double accel_sd[3];    /* m/s^2 per axis, >= 0, finite                               */
+    double v_max[3];       /* m/s per axis, > 0 (INFINITY: no cap)                       */
+    double lo[3], hi[3];   /* region, m, finite, lo < hi                                 */
+    int32_t init;          /* 1: draw the initial state; 0: continue from `state`        */
+    int32_t reserved;
+};
+int kfpos_synth_walk(int device, int64_t n_filters, int n_epochs, const struct kfpos_synth_walk *walk,
+                     double *state, double *truth, void *stream);
+
 /* NLOS detection scores of a ranging selection (no reference equivalent; DESIGN §4.5d): how the selection of
  * rows [0, n_rows) of a log this batch has just replayed (T6, kfpos_batch_replay_toa) or solved (ML,
  * kfpos_batch_ml_solve) compares with the NLOS truth.  ranges: the log, SoA [n_rows][n_anchors][N] in any fmt; a

@@ -1580,16 +1580,17 @@ extern "C" int kfpos_synth_k8_truth(int device, int64_t n_filters, int64_t first
 }
 
 namespace {
-// kfpos_synth_toa_ranges with an optional NLOS mask output (kfpos_synth_toa_ranges_nlos) and optional obstacles
-// (kfpos_synth_toa_ranges_geo)
+// kfpos_synth_toa_ranges with an optional NLOS mask output (kfpos_synth_toa_ranges_nlos), optional obstacles
+// (kfpos_synth_toa_ranges_geo) and an optional truth array in place of the Lissajous at t
+// (kfpos_synth_toa_ranges_truth)
 int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz, int n_epochs,
                      const double *t, const kfpos_synth_toa *gen, int n_obstacles, const kfpos_obstacle *obstacles,
-                     int fmt, void *ranges, uint32_t *nlos, void *stream) {
+                     int fmt, void *ranges, uint32_t *nlos, void *stream, const double *truth = nullptr) {
     static_assert(sizeof(kfpos_obstacle) == sizeof(SynthObstacle) && KFPOS_MAX_OBSTACLES == SYNTH_TOA_OBSTACLES,
                   "the kernel's obstacle table mirrors kfpos_obstacle");
     const auto prob = [](double q) { return q >= 0.0 && q <= 1.0; }; // false for NaN
     if (n_filters <= 0 || n_anchors <= 0 || n_anchors > KFPOS_MAX_ANCHORS || !anchors_xyz || n_epochs < 0 ||
-        (n_epochs > 0 && (!t || !ranges)) || !gen || (fmt != KFPOS_FMT_I32_MM && fmt != KFPOS_FMT_U16_MM))
+        (n_epochs > 0 && ((!t && !truth) || !ranges)) || !gen || (fmt != KFPOS_FMT_I32_MM && fmt != KFPOS_FMT_U16_MM))
         return KFPOS_ERR_INVALID;
     if (!prob(gen->p_missing) || !prob(gen->p_nlos) || !(gen->sigma_r >= 0.0) ||
         (gen->p_nlos > 0.0 && !(gen->nlos_mean > 0.0)) || gen->first_filter < 0 || gen->first_epoch < 0 ||
@@ -1613,11 +1614,13 @@ int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double 
     const size_t row = fmt_size(fmt) * (size_t)n_anchors * (size_t)n_filters; // bytes of one epoch
     const size_t mask_row = sizeof(uint32_t) * (size_t)n_filters;
     // the epoch times travel in the parameter block, SYNTH_TOA_T per launch: nothing to stage, so device outputs
-    // leave the call asynchronous (the next chunk can be generated while this one is replayed)
+    // (and a device truth) leave the call asynchronous (the next chunk can be generated while this one is replayed)
     SynthToaParams p{};
     int rc = anchor_table(n_anchors, anchors_xyz, &p.anchors);
     if (rc) return rc;
     Staging st(s);
+    const size_t truth_row = 3 * (size_t)n_filters; // doubles of one epoch
+    const double *d_t = st.in(truth, sizeof(double) * truth_row * (size_t)n_epochs);
     char *d_r = st.out((char *)ranges, row * (size_t)n_epochs);
     uint32_t *d_m = st.out(nlos, mask_row * (size_t)n_epochs);
     if (st.rc) return st.rc;
@@ -1629,7 +1632,8 @@ int synth_toa_ranges(int device, int64_t n_filters, int n_anchors, const double 
     for (int k0 = 0; k0 < n_epochs; k0 += SYNTH_TOA_T) {
         p.n_epochs = n_epochs - k0 < SYNTH_TOA_T ? n_epochs - k0 : SYNTH_TOA_T;
         p.epoch0 = (uint32_t)(gen->first_epoch + k0);
-        memcpy(p.t, t + k0, sizeof(double) * (size_t)p.n_epochs);
+        if (d_t) p.truth = d_t + truth_row * (size_t)k0;
+        else memcpy(p.t, t + k0, sizeof(double) * (size_t)p.n_epochs);
         p.ranges = d_r + row * (size_t)k0;
         p.nlos = d_m ? d_m + (size_t)n_filters * (size_t)k0 : nullptr;
         CK(launch_synth_toa(p, fmt == KFPOS_FMT_U16_MM, s));
@@ -1659,6 +1663,50 @@ extern "C" int kfpos_synth_toa_ranges_geo(int device, int64_t n_filters, int n_a
                                           void *stream) {
     return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, t, gen, n_obstacles, obstacles, fmt,
                             ranges, nlos, stream);
+}
+
+extern "C" int kfpos_synth_toa_ranges_truth(int device, int64_t n_filters, int n_anchors, const double *anchors_xyz,
+                                            int n_epochs, const double *truth, const kfpos_synth_toa *gen,
+                                            int n_obstacles, const kfpos_obstacle *obstacles, int fmt, void *ranges,
+                                            uint32_t *nlos, void *stream) {
+    if (n_epochs > 0 && !truth) return KFPOS_ERR_INVALID;
+    return synth_toa_ranges(device, n_filters, n_anchors, anchors_xyz, n_epochs, nullptr, gen, n_obstacles, obstacles,
+                            fmt, ranges, nlos, stream, truth);
+}
+
+extern "C" int kfpos_synth_walk(int device, int64_t n_filters, int n_epochs, const struct kfpos_synth_walk *walk,
+                                double *state, double *truth, void *stream) {
+    if (n_filters <= 0 || n_epochs < 0 || !walk || !state || (n_epochs > 0 && !truth)) return KFPOS_ERR_INVALID;
+    const struct kfpos_synth_walk &w = *walk;
+    if (w.first_filter < 0 || w.first_epoch < 0 ||
+        w.first_epoch + n_epochs > (int64_t)0xFFFFFFFF) // epoch index 0xFFFFFFFF: the per-filter constants
+        return KFPOS_ERR_INVALID;
+    if (!(w.period > 0.0) || !std::isfinite(w.period) || (w.init != 0 && w.init != 1)) return KFPOS_ERR_INVALID;
+    for (int i = 0; i < 3; ++i)
+        if (!(w.accel_sd[i] >= 0.0) || !std::isfinite(w.accel_sd[i]) || !(w.v_max[i] > 0.0) ||
+            !std::isfinite(w.lo[i]) || !std::isfinite(w.hi[i]) || !(w.lo[i] < w.hi[i]))
+            return KFPOS_ERR_INVALID;
+    if (int rc = check_device(device)) return rc;
+    if (n_epochs == 0 && !w.init) return KFPOS_OK;
+    DeviceGuard g(device);
+    if (!g.ok) return KFPOS_ERR_CUDA;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t N = (size_t)n_filters;
+    Staging st(s);
+    SynthWalkParams p;
+    // `state` is read (init 0) and written: a host array is copied in and back
+    p.state = st.out(state, sizeof(double) * 6 * N);
+    if (!w.init && p.state != state) st.copy_in(p.state, state, sizeof(double) * 6 * N);
+    p.truth = st.out(truth, sizeof(double) * 3 * N * (size_t)n_epochs);
+    if (st.rc) return st.rc;
+    p.N = n_filters; p.filter0 = w.first_filter; p.seed = w.seed;
+    p.n_epochs = n_epochs; p.init = w.init; p.epoch0 = (uint32_t)w.first_epoch;
+    p.dt = w.period; p.h = w.period * w.period / 2.0;
+    for (int i = 0; i < 3; ++i) {
+        p.accel_sd[i] = w.accel_sd[i]; p.v_max[i] = w.v_max[i]; p.lo[i] = w.lo[i]; p.hi[i] = w.hi[i];
+    }
+    CK(launch_synth_walk(p, s));
+    return st.finish();
 }
 
 namespace {

@@ -439,8 +439,9 @@ struct SynthTruthParams {
     double *truth;
 };
 cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s);
-// ranging epochs of the same truth for [T][M][N] range logs (kfpos_synth_toa_ranges); a launch covers at most
-// SYNTH_TOA_T epochs, whose times travel in the parameter block (8 KB of the 32 KB it may hold)
+// ranging epochs of the same truth, or of a caller's truth array, for [T][M][N] range logs (kfpos_synth_toa_ranges,
+// kfpos_synth_toa_ranges_truth); a launch covers at most SYNTH_TOA_T epochs, whose times travel in the parameter
+// block (8 KB of the 32 KB it may hold)
 constexpr int SYNTH_TOA_T = 1024;
 constexpr int SYNTH_TOA_OBSTACLES = 32; // KFPOS_MAX_OBSTACLES
 struct SynthObstacle {                  // kfpos_obstacle
@@ -458,8 +459,21 @@ struct SynthToaParams {
     uint32_t *nlos; // SoA [n_epochs][N] NLOS bit masks, or null (last: the offsets of the fields above stay)
     int n_obstacles; // boxes of kfpos_synth_toa_ranges_geo, 0: none (after the fields above, which keep their offsets)
     SynthObstacle obstacles[SYNTH_TOA_OBSTACLES];
+    const double *truth; // SoA [n_epochs][3][N] positions of kfpos_synth_toa_ranges_truth, or null: the Lissajous at t
 };
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s); // u16: uint16 mm, else int32 mm
+// the random walk of kfpos_synth_walk: discrete white-noise acceleration kept inside the box [lo, hi]
+struct SynthWalkParams {
+    int64_t N, filter0;
+    uint64_t seed;
+    int n_epochs, init; // init: draw the initial state, else read it from `state`
+    uint32_t epoch0;    // global index of epoch 0 of this call (RNG counter)
+    double dt, h;       // period and period^2 / 2
+    double accel_sd[3], v_max[3], lo[3], hi[3];
+    double *state; // SoA [6][N]: x, y, z, vx, vy, vz at epoch0 on entry, after the last epoch on return
+    double *truth; // SoA [n_epochs][3][N]
+};
+cudaError_t launch_synth_walk(const SynthWalkParams &p, cudaStream_t s);
 
 // selection scores against the NLOS truth (kfpos_score.cu, kfpos_batch_score_selection): counts [n_rows][8],
 // zeroed by the caller.  How `sel` [n_rows][N] is read: SCORE_NONE not at all (nothing dropped), SCORE_LOO the

@@ -6,7 +6,9 @@
 // would be 280 GB), only the chunk in flight.
 // synth_toa_kernel: ranging epochs for every consumer of a [T][M][N] millimetre range log (T6 / K8 / T9
 // ranging replays, the ML batch), with optional missing rangings and exponential NLOS biases (DESIGN §4.5c), and
-// optional boxes in the room that bias or remove the rangings whose direct path crosses them (DESIGN §4.5f).
+// optional boxes in the room that bias or remove the rangings whose direct path crosses them (DESIGN §4.5f), on
+// the Lissajous below or on a caller's truth array (DESIGN §4.5g).
+// synth_walk_kernel: a random walk of the tag inside a caller's box, the truth array of the above (DESIGN §4.5g).
 //
 // Every value is a pure function of (seed, global filter index, event index, sample index) through
 // the counter-based Philox4x32-10 generator (Salmon et al., SC'11; kfpos_synth.cuh), so a filter's stream
@@ -124,9 +126,11 @@ cudaError_t launch_synth_k8_truth(const SynthTruthParams &p, cudaStream_t s) {
 // GEO: the boxes of kfpos_synth_toa_ranges_geo (DESIGN §4.5f).  The slab test of the segment truth -> anchor uses
 // only single IEEE operations (no contraction), so a host reproduces every decision from the device truth; the
 // Philox draw (gf, g, 0x40000000 | a) of the loss and the exponential bias is made for blocked rangings only.
+// TRUTH: the position of epoch k is row k of the caller's truth array, SoA [k][3][N] (kfpos_synth_toa_ranges_truth,
+// DESIGN §4.5g), three coalesced loads instead of filter_constants / kin_at; the slab test uses its z.
 // The epoch times and the anchors are read from the parameter block: every lane reads the same one at the
 // same time (constant-bank broadcast).  Stores: SoA [k][a][N], filter index fastest -- coalesced.
-template <typename Out, bool IMPAIR, bool MASK = false, bool GEO = false>
+template <typename Out, bool IMPAIR, bool MASK = false, bool GEO = false, bool TRUTH = false>
 __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) {
     const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
     if (f >= p.N) return;
@@ -137,7 +141,14 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
     Out *out = (Out *)p.ranges + f;
     const double lim = sizeof(Out) == 2 ? 65535.0 : 2147483647.0;
     for (int k = 0; k < p.n_epochs; ++k) {
+        // with TRUTH, kn and the constants are unused and eliminated.  The position is chosen at each use: naming it
+        // once here moves the tag_z load and changes the schedule of the existing instantiations
         const Kin kn = kin_at(p.t[k], pa, pb, th0);
+        double tx = 0.0, ty = 0.0, tz = 0.0;
+        if constexpr (TRUTH) {
+            const double *tr = p.truth + (int64_t)k * 3 * N + f;
+            tx = tr[0]; ty = tr[N]; tz = tr[2 * N];
+        }
         const uint32_t g = p.epoch0 + (uint32_t)k;
         uint32_t bits = 0u;
         for (int a = 0; a < p.M; a += 2) {
@@ -145,7 +156,8 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
             normal2(p.seed, gf, g, (uint32_t)(a >> 1), n0, n1);
             for (int q = 0; q < 2 && a + q < p.M; ++q) {
                 const int i = a + q;
-                const double ex = kn.px - p.anchors.x[i], ey = kn.py - p.anchors.y[i], ez = p.tag_z - p.anchors.z[i];
+                const double ex = (TRUTH ? tx : kn.px) - p.anchors.x[i], ey = (TRUTH ? ty : kn.py) - p.anchors.y[i],
+                             ez = (TRUTH ? tz : p.tag_z) - p.anchors.z[i];
                 const double d = sqrt(ex * ex + ey * ey + ez * ez);
                 double r = d + p.sigma_r * (q ? n1 : n0);
                 bool missing = false, biased = false;
@@ -158,9 +170,9 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
                     if (biased) r += -p.nlos_mean * log(v / p.p_nlos);
                 }
                 if (GEO) {
-                    const double tp[3] = {kn.px, kn.py, p.tag_z};
-                    const double dv[3] = {__dsub_rn(p.anchors.x[i], kn.px), __dsub_rn(p.anchors.y[i], kn.py),
-                                          __dsub_rn(p.anchors.z[i], p.tag_z)};
+                    const double tp[3] = {TRUTH ? tx : kn.px, TRUTH ? ty : kn.py, TRUTH ? tz : p.tag_z};
+                    const double dv[3] = {__dsub_rn(p.anchors.x[i], tp[0]), __dsub_rn(p.anchors.y[i], tp[1]),
+                                          __dsub_rn(p.anchors.z[i], tp[2])};
                     double inv[3];
 #pragma unroll
                     for (int j = 0; j < 3; ++j) inv[j] = __ddiv_rn(1.0, dv[j]);
@@ -208,16 +220,22 @@ __global__ void __launch_bounds__(128) synth_toa_kernel(const SynthToaParams p) 
     }
 }
 
-template <typename Out, bool MASK, bool GEO>
+template <typename Out, bool MASK, bool GEO, bool TRUTH>
 static void launch_synth_toa_k(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
-    if (imp) synth_toa_kernel<Out, true, MASK, GEO><<<grid, 128, 0, s>>>(p);
-    else synth_toa_kernel<Out, false, MASK, GEO><<<grid, 128, 0, s>>>(p);
+    if (imp) synth_toa_kernel<Out, true, MASK, GEO, TRUTH><<<grid, 128, 0, s>>>(p);
+    else synth_toa_kernel<Out, false, MASK, GEO, TRUTH><<<grid, 128, 0, s>>>(p);
 }
 
-template <typename Out, bool GEO>
+template <typename Out, bool GEO, bool TRUTH>
 static void launch_synth_toa_m(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
-    if (p.nlos) launch_synth_toa_k<Out, true, GEO>(p, imp, grid, s);
-    else launch_synth_toa_k<Out, false, GEO>(p, imp, grid, s);
+    if (p.nlos) launch_synth_toa_k<Out, true, GEO, TRUTH>(p, imp, grid, s);
+    else launch_synth_toa_k<Out, false, GEO, TRUTH>(p, imp, grid, s);
+}
+
+template <typename Out, bool TRUTH>
+static void launch_synth_toa_g(const SynthToaParams &p, bool imp, unsigned grid, cudaStream_t s) {
+    if (p.n_obstacles > 0) launch_synth_toa_m<Out, true, TRUTH>(p, imp, grid, s);
+    else launch_synth_toa_m<Out, false, TRUTH>(p, imp, grid, s);
 }
 
 cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) {
@@ -225,12 +243,82 @@ cudaError_t launch_synth_toa(const SynthToaParams &p, bool u16, cudaStream_t s) 
     const bool imp = p.p_missing > 0 || p.p_nlos > 0;
     const unsigned grid = (unsigned)((p.N + 127) / 128);
     if (u16) {
-        if (p.n_obstacles > 0) launch_synth_toa_m<uint16_t, true>(p, imp, grid, s);
-        else launch_synth_toa_m<uint16_t, false>(p, imp, grid, s);
+        if (p.truth) launch_synth_toa_g<uint16_t, true>(p, imp, grid, s);
+        else launch_synth_toa_g<uint16_t, false>(p, imp, grid, s);
     } else {
-        if (p.n_obstacles > 0) launch_synth_toa_m<int32_t, true>(p, imp, grid, s);
-        else launch_synth_toa_m<int32_t, false>(p, imp, grid, s);
+        if (p.truth) launch_synth_toa_g<int32_t, true>(p, imp, grid, s);
+        else launch_synth_toa_g<int32_t, false>(p, imp, grid, s);
     }
+    return cudaGetLastError();
+}
+
+// The random walk of kfpos_synth_walk (DESIGN §4.5g), one thread per filter, the state in registers across the
+// epochs.  Discrete white-noise acceleration (the F and Q of t6_predict_cov) per axis i, a_i = accel_sd_i n_i:
+//   p' = (p + v dt) + a h,  v' = v + a dt,  h = dt^2 / 2 (from the host);
+//   a wall crossed reflects the position and reverses the velocity; then p' is clamped to [lo, hi] and v' to
+//   [-v_max, v_max].
+// Every step is one IEEE operation (no contraction), so a host reproduces a trajectory from its normals.
+// Draws: initial position uniforms (gf, 0xFFFFFFFF, 2) (x, y) and (gf, 0xFFFFFFFF, 3) (z); the normals of epoch g
+// (gf, g, 0x20000000) (x, y) and (gf, g, 0x20000001) (z, only when accel_sd_z > 0).  Stores: SoA, coalesced.
+__global__ void __launch_bounds__(128) synth_walk_kernel(const SynthWalkParams p) {
+    const int64_t f = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (f >= p.N) return;
+    const int64_t N = p.N;
+    const uint64_t gf = (uint64_t)(p.filter0 + f);
+    const uint32_t s0 = (uint32_t)p.seed, s1 = (uint32_t)(p.seed >> 32);
+    double x[3], v[3];
+    if (p.init) {
+        double u[4];
+        uniform2(philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 2u, s0, s1), u[0], u[1]);
+        u[2] = 0.5;
+        if (p.accel_sd[2] > 0.0)
+            uniform2(philox4x32_10((uint32_t)gf, (uint32_t)(gf >> 32), 0xFFFFFFFFu, 3u, s0, s1), u[2], u[3]);
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            x[i] = p.accel_sd[i] > 0.0 ? __dadd_rn(p.lo[i], __dmul_rn(__dsub_rn(p.hi[i], p.lo[i]), u[i]))
+                                       : __dmul_rn(__dadd_rn(p.lo[i], p.hi[i]), 0.5);
+            v[i] = 0.0;
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            x[i] = p.state[i * N + f];
+            v[i] = p.state[(3 + i) * N + f];
+        }
+    }
+    for (int k = 0; k < p.n_epochs; ++k) {
+        const uint32_t g = p.epoch0 + (uint32_t)k;
+        double n[3] = {0.0, 0.0, 0.0}, unused;
+        normal2(p.seed, gf, g, 0x20000000u, n[0], n[1]);
+        if (p.accel_sd[2] > 0.0) normal2(p.seed, gf, g, 0x20000001u, n[2], unused);
+        double *o = p.truth + (int64_t)k * 3 * N + f;
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            const double a = __dmul_rn(p.accel_sd[i], n[i]);
+            double xn = __dadd_rn(__dadd_rn(x[i], __dmul_rn(v[i], p.dt)), __dmul_rn(a, p.h));
+            double vn = __dadd_rn(v[i], __dmul_rn(a, p.dt));
+            if (xn > p.hi[i]) {
+                xn = __dsub_rn(__dadd_rn(p.hi[i], p.hi[i]), xn);
+                vn = -vn;
+            } else if (xn < p.lo[i]) {
+                xn = __dsub_rn(__dadd_rn(p.lo[i], p.lo[i]), xn);
+                vn = -vn;
+            }
+            x[i] = fmin(fmax(xn, p.lo[i]), p.hi[i]);
+            v[i] = fmin(fmax(vn, -p.v_max[i]), p.v_max[i]);
+            o[i * N] = x[i];
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        p.state[i * N + f] = x[i];
+        p.state[(3 + i) * N + f] = v[i];
+    }
+}
+
+cudaError_t launch_synth_walk(const SynthWalkParams &p, cudaStream_t s) {
+    if (p.N <= 0) return cudaSuccess;
+    synth_walk_kernel<<<(unsigned)((p.N + 127) / 128), 128, 0, s>>>(p);
     return cudaGetLastError();
 }
 

@@ -1,9 +1,12 @@
 // kfpos_synth.cuh -- the counter-based random numbers and the truth kinematics of the Monte Carlo input
-// generators (kfpos_synth.cu: synth_k8_kernel, synth_k8_truth_kernel and synth_toa_kernel).
+// generators (kfpos_synth.cu: synth_k8_kernel, synth_k8_truth_kernel, synth_toa_kernel and synth_walk_kernel).
 //
 // Every value is a pure function of (seed, global filter index, event index, sample index) through the
 // counter-based Philox4x32-10 generator (Salmon et al., SC'11): counter (filter lo, filter hi, event,
-// sample), key (seed lo, seed hi).  Event index 0xFFFFFFFF is reserved for the per-filter constants.
+// sample), key (seed lo, seed hi).  Event index 0xFFFFFFFF is reserved for the per-filter constants: samples 0
+// and 1 for filter_constants, 2 and 3 for the initial position of the random walk (synth_walk_kernel).  Samples
+// of an epoch: 0..15 the ranging noise, 0x80000000 | a and 0x40000000 | a its impairments, 0x20000000 and
+// 0x20000001 the walk's accelerations -- the walk and the rangings may share one seed without sharing a draw.
 #pragma once
 #include "kfpos_math.cuh"
 

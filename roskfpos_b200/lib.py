@@ -72,6 +72,13 @@ class KfposObstacle(C.Structure):
                 ("p_loss", C.c_double)]
 
 
+class KfposSynthWalk(C.Structure):
+    """struct kfpos_synth_walk: the random walk of kfpos_synth_walk (DESIGN §4.5g)."""
+    _fields_ = [("seed", C.c_uint64), ("first_filter", C.c_int64), ("first_epoch", C.c_int64), ("period", C.c_double),
+                ("accel_sd", C.c_double * 3), ("v_max", C.c_double * 3), ("lo", C.c_double * 3), ("hi", C.c_double * 3),
+                ("init", C.c_int32), ("reserved", C.c_int32)]
+
+
 _LIB = None
 
 # name -> (restype, argtypes); every symbol include/kfpos_b200.h declares
@@ -127,6 +134,9 @@ SIGNATURES = {
     "kfpos_batch_crlb": (_I, [_VP, _I, _I, _VP, _VP, _I, _D, _VP, _VP, _VP, _VP, _VP]),
     "kfpos_synth_toa_ranges_geo": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _I, _VP, _VP,
                                         _VP]),
+    "kfpos_synth_toa_ranges_truth": (_I, [_I, _I64, _I, _VP, _I, _VP, C.POINTER(KfposSynthToa), _I, _VP, _I, _VP, _VP,
+                                          _VP]),
+    "kfpos_synth_walk": (_I, [_I, _I64, _I, C.POINTER(KfposSynthWalk), _VP, _VP, _VP]),
 }
 ASM_FIX_ROW_CLEAR = 1
 

@@ -290,9 +290,65 @@ def k8_montecarlo_chunk(n_filters, macro0, n_macro, anchors, device, seed=SEED, 
     return res
 
 
+def walk_truth_chunk(n_filters, epoch0, n_epochs, device, *, seed, period, accel_sd, v_max, lo, hi, first_filter=0,
+                     state=None, want_x0=False, out=None, stream=None):
+    """Epochs [epoch0, epoch0 + n_epochs) of the random walk of kfpos_synth_walk (DESIGN §4.5g), generated ON THE
+    DEVICE: discrete white-noise acceleration of sd accel_sd (m/s^2, per axis) with speeds capped at v_max (m/s, per
+    axis, inf: no cap), reflected at the walls of the box [lo, hi] (m).  An axis with accel_sd 0 stays at the
+    centre of the box (a fixed tag height).  Each position is a pure function of (seed, first_filter + f, epoch)
+    and the state the chunk starts from, so sharding and chunking change nothing.
+    state: None draws the initial state (zero velocity, uniform in the box); else the [6][N] float64 device tensor
+    (x, y, z, vx, vy, vz, the T6 state layout) at epoch0, which the call advances IN PLACE to the state after the
+    last epoch.  Returns dict(truth [n_epochs][3][N] float64 on `device`, row k the position at time
+    (epoch0 + k + 1) * period, what toa_montecarlo_chunk(truth=...) and Batch.set_truth_traj take; state [6][N];
+    x0 [6][N] the initial state when state is None and want_x0).  `out` may hold the tensors of a previous chunk of
+    the same shape to be reused."""
+    import ctypes as C
+    import torch
+    from . import lib as L
+    from .batch import _stream_ptr
+    N, n = int(n_filters), int(n_epochs)
+    dev = torch.device(device)
+    out = {} if out is None else out
+
+    def buf(name, shape):
+        tns = out.get(name)
+        if tns is None or tuple(tns.shape) != tuple(shape) or tns.dtype != torch.float64:
+            tns = out[name] = torch.empty(shape, device=dev, dtype=torch.float64)
+        return tns
+    vec = lambda v: np.broadcast_to(np.asarray(v, dtype=np.float64), (3,))
+    w = L.KfposSynthWalk(seed=int(seed), first_filter=int(first_filter), first_epoch=int(epoch0), period=float(period))
+    w.accel_sd[:], w.v_max[:], w.lo[:], w.hi[:] = vec(accel_sd), vec(v_max), vec(lo), vec(hi)
+    truth = buf("truth", (n, 3, N))
+    sp = _stream_ptr(stream)
+
+    def call(init, n_ep, st):
+        w.init = init
+        L.check(L.lib().kfpos_synth_walk(dev.index or 0, N, n_ep, C.byref(w), C.c_void_p(st.data_ptr()),
+                                         C.c_void_p(truth.data_ptr()) if n_ep else None, sp), "kfpos_synth_walk")
+    res = dict(truth=truth)
+    if state is None:
+        state = buf("state", (6, N))
+        if want_x0:  # the initial state on its own, then the epochs from it: the same numbers as one init call
+            x0 = buf("x0", (6, N))
+            call(1, 0, x0)
+            state.copy_(x0)
+            res["x0"] = x0
+            call(0, n, state)
+        else:
+            call(1, n, state)
+    else:
+        if tuple(state.shape) != (6, N) or state.dtype != torch.float64 or not state.is_cuda:
+            raise ValueError("walk_truth_chunk: state must be a [6][N] float64 device tensor")
+        call(0, n, state)
+    res["state"] = state
+    return res
+
+
 def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED, period=0.1, sigma_r=0.10,
                          p_missing=0.0, p_nlos=0.0, nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None,
-                         want_x0=False, want_truth=False, out=None, stream=None, want_nlos=False, obstacles=None):
+                         want_x0=False, want_truth=False, out=None, stream=None, want_nlos=False, obstacles=None,
+                         truth=None):
     """Ranging epochs [epoch0, epoch0 + n_epochs) of the T6 Monte Carlo workload, generated ON THE DEVICE by
     kfpos_synth_toa_ranges (Philox4x32-10; a ranging depends only on seed, the global filter index
     first_filter + f, the global epoch index and the anchor, so sharding and chunking change nothing).  Epoch k
@@ -308,7 +364,11 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     reused.  ML batches take `ranges` row by row.
     obstacles: [n][9] boxes (lo x y z, hi x y z, excess_per_m, spread, p_loss; DESIGN §4.5f) whose crossing biases
     or removes a ranging (kfpos_synth_toa_ranges_geo); the nlos mask then also marks the blocked rangings.  None or
-    an empty array: no boxes, the calls above."""
+    an empty array: no boxes, the calls above.
+    truth: a [n_epochs][3][N] float64 device tensor of positions (walk_truth_chunk, or any trajectory; DESIGN §4.5g)
+    in place of the Lissajous: the rangings come from kfpos_synth_toa_ranges_truth (tag_z is ignored), boxes and
+    the mask work as above, want_truth returns this tensor and truth_end is its last row.  want_x0 then has no
+    Lissajous to start from and is refused (walk_truth_chunk gives a walk's x0)."""
     import ctypes as C
     import torch
     from . import lib as L
@@ -318,6 +378,12 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
         raise ValueError("toa_montecarlo_chunk: fmt must be FMT_I32_MM or FMT_U16_MM")
     anc = np.ascontiguousarray(anchors, dtype=np.float64).reshape(-1, 3)
     M, N, n = len(anc), int(n_filters), int(n_epochs)
+    if truth is not None:
+        if tuple(truth.shape) != (n, 3, N) or truth.dtype != torch.float64 or not truth.is_cuda:
+            raise ValueError("toa_montecarlo_chunk: truth must be a [n_epochs][3][N] float64 device tensor")
+        if want_x0:
+            raise ValueError("toa_montecarlo_chunk: want_x0 needs the Lissajous; walk_truth_chunk gives a walk's x0")
+        truth = truth.contiguous()
     # times from the global epoch index, so that they do not depend on where a chunk starts
     t = np.ascontiguousarray(np.arange(epoch0 + 1, epoch0 + n + 1, dtype=np.float64) * period)
     dev = torch.device(device)
@@ -337,12 +403,20 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
             C.c_void_p(ranges.data_ptr()))
     nlos = buf("nlos", (n, N), torch.int32) if want_nlos else None  # torch has no general uint32: the mask bits
     box = np.zeros((0, 9)) if obstacles is None else np.asarray(obstacles, dtype=np.float64).reshape(-1, 9)
+    tbl = None
     if len(box):
         tbl = (L.KfposObstacle * len(box))()
         for o, b in zip(tbl, box):
             o.lo[:], o.hi[:] = b[0:3], b[3:6]
             o.excess_per_m, o.spread, o.p_loss = b[6], b[7], b[8]
-        L.check(L.lib().kfpos_synth_toa_ranges_geo(*args[:7], len(box), C.cast(tbl, C.c_void_p), *args[7:],
+        tbl = C.cast(tbl, C.c_void_p)
+    if truth is not None:
+        targs = args[:5] + (C.c_void_p(truth.data_ptr()),) + args[6:]
+        L.check(L.lib().kfpos_synth_toa_ranges_truth(*targs[:7], len(box), tbl, *targs[7:],
+                                                     None if nlos is None else C.c_void_p(nlos.data_ptr()), sp),
+                "kfpos_synth_toa_ranges_truth")
+    elif len(box):
+        L.check(L.lib().kfpos_synth_toa_ranges_geo(*args[:7], len(box), tbl, *args[7:],
                                                    None if nlos is None else C.c_void_p(nlos.data_ptr()), sp),
                 "kfpos_synth_toa_ranges_geo")
     elif want_nlos:
@@ -361,7 +435,11 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
     res = dict(ranges=ranges, dt=float(period), t=t)
     if want_nlos:
         res["nlos"] = nlos
-    if want_truth:
+    if truth is not None:
+        if want_truth:
+            res["truth"] = truth
+        res["truth_end"] = truth[-1]
+    elif want_truth:
         res["truth"] = truth_at("truth", t)
         res["truth_end"] = res["truth"][-1]
     else:
@@ -376,7 +454,7 @@ def toa_montecarlo_chunk(n_filters, epoch0, n_epochs, anchors, device, seed=SEED
 
 def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma_r=0.10, p_missing=0.0, p_nlos=0.0,
                    nlos_mean=0.8, tag_z=1.0, first_filter=0, fmt=None, err=0.01, epoch0=0, init_state=True,
-                   stream=None, hist=None, score=False, *, crlb=None, obstacles=None):
+                   stream=None, hist=None, score=False, *, crlb=None, obstacles=None, walk=None):
     """A Monte Carlo run of any length on a T6 Batch (anchors set to `anchors`), in chunks of `chunk` epochs:
     for each chunk toa_montecarlo_chunk generates the rangings and the truth, Batch.set_truth_traj registers the
     truth (which resets the row cursor, so the chunk's rows start at 0), Batch.replay_toa runs the chunk and
@@ -395,7 +473,11 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
     floor to whole millimetres); a dict {set: [n_epochs][4]} (batch.crlb_summary) is appended as the last element
     of the return value, a tuple then.
     obstacles: the boxes of toa_montecarlo_chunk (DESIGN §4.5f); score and crlb "los" then use the mask that also
-    marks the rangings they block."""
+    marks the rangings they block.
+    walk=dict(accel_sd=..., v_max=..., lo=..., hi=...): the tag follows the random walk of walk_truth_chunk (DESIGN
+    §4.5g) instead of the Lissajous, with the run's seed, period and first_filter; tag_z is then unused.  The walk
+    starts at epoch0 from its drawn initial state (init_state sets the batch to it, as x0), and its state is carried
+    from chunk to chunk on the device, so any chunk length gives the same run."""
     from . import lib as L
     if batch.model != L.MODEL_T6:
         raise ValueError("toa_montecarlo runs T6 batches; ML batches take toa_montecarlo_chunk output directly")
@@ -407,17 +489,31 @@ def toa_montecarlo(batch, n_epochs, chunk, anchors, seed=SEED, period=0.1, sigma
     bounds = {name: [] for name in crlb}
     want_sel, want_nlos = score or "used" in crlb, score or "los" in crlb
     var = float(sigma_r) ** 2 + 1e-6 / 12.0
-    rows, counts, scores, bufs = [], [], [], {}
-    sel = None
+    rows, counts, scores, bufs, wbufs = [], [], [], {}, {}
+    sel = wstate = None
+    if walk is not None:
+        walk = dict(walk)
+        if set(walk) != {"accel_sd", "v_max", "lo", "hi"}:
+            raise ValueError("toa_montecarlo: walk takes exactly accel_sd, v_max, lo and hi")
     if hist is not None:
         batch.set_error_hist(hist[0], hist[1])
     try:
         for k0 in range(0, int(n_epochs), int(chunk)):
             n = min(int(chunk), int(n_epochs) - k0)
-            w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
-                                     want_x0=init_state and k0 == 0, out=bufs, want_nlos=want_nlos, **kw)
+            x0 = None
+            if walk is None:
+                w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
+                                         want_x0=init_state and k0 == 0, out=bufs, want_nlos=want_nlos, **kw)
+                x0 = w.get("x0")
+            else:
+                wk = walk_truth_chunk(batch.N, epoch0 + k0, n, "cuda:%d" % batch.device, seed=seed, period=period,
+                                      first_filter=first_filter, state=wstate, want_x0=init_state and k0 == 0,
+                                      out=wbufs, stream=stream, **walk)
+                wstate, x0 = wk["state"], wk.get("x0")
+                w = toa_montecarlo_chunk(batch.N, epoch0 + k0, n, anchors, "cuda:%d" % batch.device, want_truth=True,
+                                         out=bufs, want_nlos=want_nlos, truth=wk["truth"], **kw)
             if init_state and k0 == 0:
-                batch.set_state(w["x0"], None, stream=stream)
+                batch.set_state(x0, None, stream=stream)
             batch.set_truth_traj(w["truth"], stream=stream)
             if want_sel and (sel is None or sel.shape[0] != n):
                 import torch
